@@ -2,7 +2,7 @@
 """Headline benchmark: PolynomialBatch commit throughput (iNTT + coset LDE + bit-reversed row-major leaves + Poseidon
 Merkle tree to the cap) on N B200s, in Melem/s (= N_rows * n_cols input elements per second), BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one whole commit of the workload (default 2^20 x 135, rate_bits 3, cap_height 4 = BASELINE.json configs[2],
@@ -36,6 +36,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "oracle")):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True       # the benchmark leaves the tree it runs from as it found it (no __pycache__ of the modules above)
 
 P = 0xFFFF_FFFF_0000_0001
 METRIC = "commit Melem/s (2^20x135 LDE+Poseidon Merkle)"
@@ -63,7 +64,15 @@ def parse():
                          "x 2^16 -> prove_openings -> FRI [4,4,4] -> PoW 16 -> 28 query rounds), second line of BASELINE.json's metric")
     ap.add_argument("--single-process", action="store_true",
                     help="--gpus N from ONE process through gl_commit_multi (the form CircuitData::prove can call), instead of torchrun")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (a fixed, seeded sample of "
+                         "the large arrays, at most 64 MB in all), so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference" and a.workload == "commit":
+        ap.error("--dump-outputs: the reference commit arm times the CPU restatement and keeps no outputs")
+    return a
 
 
 def workload_name(a):
@@ -74,6 +83,72 @@ def perms_per_commit(log_n, cols, r, h):
     R = 1 << (log_n + r)
     per_leaf = (cols + 7) // 8 if cols > 4 else 0
     return R * per_leaf + (R - (1 << h))
+
+
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array of field words as out_dir/<name>.npy: float64 with a trailing axis of two, the low and the high 32 bits of each
+    uint64 word (a whole word does not fit a float64 mantissa; each half does, so the dump is exact)."""
+    import numpy as np
+    out = {}
+    for name, a in arrays.items():
+        w = np.asarray(a, dtype=np.uint64)
+        out[name] = np.stack([w & np.uint64(0xFFFFFFFF), w >> np.uint64(32)], axis=-1).astype(np.float64)
+    total = sum(x.nbytes for x in out.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x)
+
+
+def dump_sample(n, k, seed):
+    """k sorted indices out of range(n), the same for every run and build (all of them when k >= n)"""
+    import numpy as np
+    if k >= n:
+        return np.arange(n, dtype=np.uint64)
+    return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False)).astype(np.uint64)
+
+
+def tree_outputs(cap, trees, batch=None):
+    """What a caller of a commit receives, sized for DUMP_BYTES: the whole cap, seeded samples of the leaf rows with their Merkle paths
+    (which carry digests from every layer of the tree) and, when the batch keeps them, of the coefficients.  `trees` cover equal
+    consecutive leaf ranges (one tree, or the shard trees of gl_commit_multi)."""
+    import numpy as np
+    cap = np.asarray(cap, dtype=np.uint64).reshape(-1, 4)
+    per, cols = trees[0].n_leaves, trees[0].leaf_len
+    depth = per.bit_length() - 1 - trees[0].cap_height
+    row_bytes = 16 * (1 + cols + 4 * depth + (1 + cols if batch is not None else 0))
+    k = min(4096, max(1, (DUMP_BYTES - 16 * cap.size) // row_bytes))
+    idx = dump_sample(per * len(trees), k, seed=1)
+    rows = np.zeros((idx.size, cols), dtype=np.uint64)
+    paths = np.zeros((idx.size, depth, 4), dtype=np.uint64)
+    for q, t in enumerate(trees):
+        sel = (idx // per) == q
+        if sel.any():
+            rows[sel], paths[sel] = t.open_batch(idx[sel] % per)
+    out = {"cap": cap, "leaf_index": idx, "leaves": rows, "merkle_paths": paths}
+    if batch is not None:
+        cidx = dump_sample(1 << batch.degree_log, k, seed=2)
+        out.update({"coeff_index": cidx, "coeffs": batch.polynomials[:, cidx]})
+    return out
+
+
+def proof_outputs(proof):
+    """every field of a wrapper-pipeline proof (tests/wrapper_pipeline.py), one array per field, tree and FRI layer"""
+    out = {"commit_caps": proof["commit_caps"], "commit_phase_caps": proof["commit_phase_caps"], "final_poly": proof["final_poly"],
+           "pow_witness": [proof["pow_witness"]], "query_indices": proof["query_indices"]}
+    rounds = proof["query_rounds"]
+    for k in range(len(rounds[0]["initial"])):
+        out[f"query_rows_tree{k}"] = [rn["initial"][k][0] for rn in rounds]
+        out[f"query_paths_tree{k}"] = [rn["initial"][k][1] for rn in rounds]
+    for j in range(len(rounds[0]["steps"])):
+        out[f"query_evals_layer{j}"] = [rn["steps"][j][0] for rn in rounds]
+        out[f"query_paths_layer{j}"] = [rn["steps"][j][1] for rn in rounds]
+    return out
 
 
 # ------------------------------------------------------------------------------------------------ CPU baseline
@@ -245,6 +320,8 @@ def run_wrapper(a):
         for _ in range(a.steps):
             proof = wp.run_oracle(oc, cols, log_n, timings=tm)
         ms = (time.perf_counter() - t0) / a.steps * 1e3
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, proof_outputs(proof))
         line.update({"impl": "reference", "value": round(ms, 2), "ms_per_step": round(ms, 2), "stage_ms": {k: round(v, 2) for k, v in tm.items()},
                      "cpu_baseline": {"value": round(ms, 2), "unit": "ms", "cores": oc.num_threads(), "kind": "port",
                                       "sample": "the whole pipeline, oracle/gl_oracle.c + Python glue"},
@@ -277,6 +354,8 @@ def run_wrapper(a):
     t1 = time.perf_counter()
     ms = (t1 - t0) / a.steps * 1e3
     clocks = sampler.stop(t0, t1)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, proof_outputs(proof))
     h2d = sum(c.nbytes for c in cols)
     d2h = sum(np.asarray(x).nbytes for rnd in proof["query_rounds"] for pair in rnd["initial"] + rnd["steps"] for x in pair) + \
         sum(np.asarray(c).nbytes for c in proof["commit_caps"] + proof["commit_phase_caps"]) + np.asarray(proof["final_poly"]).nbytes
@@ -413,11 +492,15 @@ def run_single_process(a):
     harr = np.ctypeslib.as_array(ctypes.cast(ptr, ctypes.POINTER(ctypes.c_uint64)), shape=(cols, n))
     harr[:] = splitmix_columns(1, cols, n)
     sampler = ClockSampler(0)
+    kept = []                        # --dump-outputs: the shard trees of the last timed step, released after the dump
 
-    def step():
+    def step(last=False):
         cap, trees = g.commit_multi(ctxs, list(harr), r, h)
-        for t in trees:
-            t.free()
+        if last and a.dump_outputs:
+            kept.extend(trees)
+        else:
+            for t in trees:
+                t.free()
         return cap.hashes
 
     for _ in range(max(a.warmup, 0)):
@@ -425,10 +508,14 @@ def run_single_process(a):
     sampler.start()
     time.sleep(0.2)
     t0 = time.perf_counter()
-    for _ in range(a.steps):
-        cap = step()
+    for i in range(a.steps):
+        cap = step(last=i == a.steps - 1)
     t1 = time.perf_counter()
     clocks = sampler.stop(t0, t1)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, tree_outputs(cap, kept))
+        for t in kept:
+            t.free()
     ms = (t1 - t0) / a.steps * 1e3
     val = cols * n / (ms * 1e-3) / 1e6
     stage = {}
@@ -484,17 +571,21 @@ def main():
     log_n, cols, r, h = a.log_n, a.cols, a.rate_bits, a.cap_height
     n = 1 << log_n
     cap = np.zeros(4 << h, dtype=np.uint64)
+    kept = []                        # --dump-outputs: the batch handle of the last timed step, released after the dump
 
     if world == 1:
         d_cols = synth_columns(torch, dev, cols, n, 1)
         torch.cuda.synchronize()
 
-        def step():
+        def step(last=False):
             hd = ctypes.c_uint64()
             rc = lib.gl_dev_commit(ctx.handle, d_cols.data_ptr(), n, cols, log_n, r, h, 0, cap.ctypes.data, ctypes.byref(hd))
             if rc != 0:
                 raise RuntimeError(lib.gl_ctx_last_error(ctx.handle).decode())
-            lib.gl_tree_free(ctx.handle, hd.value)
+            if last and a.dump_outputs:
+                kept.append(hd.value)
+            else:
+                lib.gl_tree_free(ctx.handle, hd.value)
     else:
         plan = sharded.ShardPlan(cols, log_n, r, h, world)
         c0, c1 = plan.col_range(rank)
@@ -502,7 +593,7 @@ def main():
         state = sharded.ShardedCommit(ctx, plan, rank, dist, torch, exchange=a.exchange)
         torch.cuda.synchronize()
 
-        def step():
+        def step(last=False):
             cap[:] = state.commit(d_cols)
 
     def barrier():
@@ -522,8 +613,8 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.perf_counter()
     e0.record(stream)
-    for _ in range(a.steps):
-        step()
+    for i in range(a.steps):
+        step(last=i == a.steps - 1)
         ms, ln = ctx.stage_times()
         for k, v in ms.items():
             stage_acc[k] = stage_acc.get(k, 0.0) + v
@@ -547,6 +638,13 @@ def main():
     # plain JSON — the oracle itself is not executed here).  A mismatch fails the run: a fast wrong commit is not a result.
     import headline
     parity = headline.parity_block(cap_dev, log_n, cols, r, h, seed=1)
+    if a.dump_outputs and rank == 0:
+        if world == 1:                   # one device: the whole batch stays behind the handle (coefficients, leaves, digests)
+            batch = g.PolynomialBatch(ctx, g.MerkleTree(ctx, kept[0], cap_dev), cols)
+            dump_outputs(a.dump_outputs, tree_outputs(cap_dev, [batch.merkle_tree], batch))
+            batch.merkle_tree.free()
+        else:                            # sharded: a caller of ShardedCommit.commit receives the cap
+            dump_outputs(a.dump_outputs, {"cap": cap_dev.reshape(-1, 4)})
 
     # ---- e2e: the C-ABI call a Rust shim would make, host buffers in, cap out, every step --------------------------
     e2e = None

@@ -19,20 +19,14 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 # ------------------------------------------------------------------------------------------------ CPU: the oracle itself
 def test_poseidon2_constants_match_the_reference_source():
+    """tests/golden/poseidon2_constants.json holds the constants as parsed out of the reference's poseidon2_goldilocks.rs
+    (tools/gen_poseidon2_constants.py); the oracle's and the device's tables must be those numbers."""
     fix = json.load(open(os.path.join(ROOT, "tests", "golden", "poseidon2_constants.json")))
     assert fix["MAT_DIAG_M_1"] == go.MAT_DIAG_M_1 and fix["RC"] == go.RC and fix["RC_MID"] == go.RC_MID
     assert all(0 <= x < P for row in go.RC for x in row) and all(0 <= x < P for x in go.RC_MID)
     cuh = open(os.path.join(ROOT, "plonky2.5_b200", "csrc", "poseidon2_constants.cuh")).read()
     for x in go.RC_MID + go.RC[3] + [d - 1 for d in go.MAT_DIAG_M_1]:
         assert "0x%016xULL" % x in cuh
-    ref = "/root/reference/src/common/poseidon2/poseidon2_goldilocks.rs"
-    if os.path.exists(ref):                              # build container only
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("gen_p2", os.path.join(ROOT, "tools", "gen_poseidon2_constants.py"))
-        gen = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(gen)
-        c = gen.parse(ref)
-        assert c["MAT_DIAG_M_1"] == go.MAT_DIAG_M_1 and c["RC"] == go.RC and c["RC_MID"] == go.RC_MID
 
 
 def test_gate_oracle_consistency():
