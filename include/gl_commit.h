@@ -82,8 +82,8 @@ int gl_commit(gl_ctx* ctx, const uint64_t* const* cols, uint32_t n_cols, uint32_
  * apply to them.  All contexts are locked for the duration of the call; status and message are reported through ctxs[0].
  * With TWO contexts on two devices (and 2 <= 2^rate_bits) the call runs the streamed coset plan (gl_commit_coset_stream below: column
  * groups dealt cyclically, per wave copy -> iNTT -> ticket -> peer pulls -> own cosets -> leaf sponge, no barrier between the first wave
- * and the cap); otherwise the column->row shipment described above.  GL_MULTI_PLAN=stream forces the streamed plan for any n_ctx <=
- * 2^rate_bits with one context per device (slower than the shipment at 8 devices in ONE process, see DESIGN.md §6), =p2p forbids it.
+ * and the cap); otherwise the column->row shipment described above (at 8 devices in ONE process the streamed plan is slower than the
+ * shipment, see DESIGN.md §6).
  * Tested bit-exact against the oracle with several contexts on one device and with one device per context (tests/test_gpu_parity.py
  * spreads the contexts over every visible GPU; bench.py --gpus N --single-process times it).                                      */
 int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* cols, uint32_t n_cols, uint32_t log_n, uint32_t rate_bits,
@@ -242,9 +242,11 @@ int gl_dev_commit(gl_ctx* ctx, const uint64_t* d_cols, uint64_t col_stride, uint
 int gl_dev_lde(gl_ctx* ctx, const uint64_t* d_cols, uint64_t col_stride, uint32_t n_cols, uint32_t log_n,
                uint32_t rate_bits, int input_is_coeffs, uint64_t* d_out_rows, uint32_t out_pitch,
                uint64_t* d_out_coeffs);
-/* stage 1 fused with the column->row exchange (one process per GPU, NVLink peer memory): like gl_dev_lde, but the last
- * NTT pass of every coset stores each leaf-row segment directly into the leaf buffer of the rank that owns that row:
- * global leaf row i lives in peer_leaves[i / (R/n_peers)] at row i % (R/n_peers), columns [col_off, col_off+n_cols) of
+/* stage 1 fused with the column->row exchange (one process per GPU, NVLink peer memory): like gl_dev_lde, but every coset's
+ * rows go to the leaf buffer of the rank that owns them.  A coset whose rows all belong to this rank (its buffer is one
+ * allocated by gl_dev_ipc_alloc on ctx) is stored there by the last NTT pass itself; every other coset is evaluated into a
+ * local buffer and shipped by the copy engines, one strided peer copy per owner, while the next coset's NTT runs.
+ * Global leaf row i lives in peer_leaves[i / (R/n_peers)] at row i % (R/n_peers), columns [col_off, col_off+n_cols) of
  * a [R/n_peers][leaf_pitch] matrix.  peer_leaves: HOST array of n_peers device pointers (own buffer + buffers mapped
  * with gl_dev_ipc_open).  The caller synchronises the ranks (barrier) before hashing.  The 2^rate_bits cosets are
  * processed in the order first_coset, first_coset+1, ... (mod 2^rate_bits): ranks that start at different cosets store

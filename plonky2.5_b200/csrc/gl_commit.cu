@@ -32,6 +32,10 @@
 #include "peer_sync.cuh"
 #include "permutation.cuh"
 
+#ifndef LEAF_BLOCK
+#define LEAF_BLOCK 128   // threads per CTA of the leaf-hash kernels (tests/variants.py builds other sizes)
+#endif
+
 namespace {
 
 struct GlError {
@@ -198,7 +202,6 @@ struct gl_ctx {
     std::map<std::pair<uint64_t, uint32_t>, std::unique_ptr<CosetTable>> coset_cache;   // (shift, log_len) -> g^j: FRI layers / final-poly LDE
     size_t coset_cache_words = 0;
     DevBuf in_stage, vals, scratch, hash_state;
-    bool stream_hash = true;              // GL_STREAM_HASH=0: hash the leaves in one launch after the whole LDE even for host columns
     std::map<gl_handle, std::unique_ptr<Tree>> trees;
     std::map<gl_handle, std::unique_ptr<Fri>> fris;
     std::map<gl_handle, std::unique_ptr<Openings>> openings;
@@ -206,19 +209,9 @@ struct gl_ctx {
     float aux_ms = 0;
     gl_handle next_handle = 1;
     cudaStream_t copy_stream = nullptr;   // host->device column copies of gl_commit, overlapped with the NTTs
-    // multi-GPU exchange mode of gl_*_lde_scatter (GL_SCATTER_MODE overrides; DESIGN.md §6 has the measurements):
-    //   0 = the last NTT pass stores every leaf-row segment into its owner's buffer itself (one kernel; 32/64-byte remote stores)
-    //   1 = the coset result stays local and a copy kernel on the high-priority send_stream ships it behind the next coset's NTT
-    //   2 = as 1 without overlap (measurement aid)
-    //   3 = default: cosets owned by this rank are stored by the NTT itself (no copy); the others stay local and the COPY ENGINES
-    //       ship them (one strided 2-D peer copy per owner segment) while the next coset's NTT runs — no SM time, no NVLink
-    //       stalls inside the NTT
-    int scatter_mode = 3;
-    int ntt_version = 2;                  // GL_NTT_VERSION=1 selects the first-generation pass kernel (ntt.cuh) for A/B measurements
-    int ntt_max_a = 10;                   // GL_NTT_MAX_A=11: 2048-row tiles, two passes instead of three at 2^21 / 2^22 — bit-exact and racecheck-clean,
-                                          // but measured SLOWER on B200 (2^22 x 256: iNTT 23.1 vs 19.8 ms, LDE 44.6 vs 37.5 ms): the 4-column tiles and
-                                          // 86 KB of shared memory cost more than the saved pass, so three (8,7,7) passes stay the default
-    int ntt_g10 = 8;                      // GL_NTT_G10=4: 4-column tiles for the 10-stage passes (smaller CTAs)
+    // multi-GPU exchange of gl_*_lde_scatter (DESIGN.md §6 has the measurements): cosets owned by this rank are stored by the NTT
+    // itself (no copy); the others stay local in send_buf and the COPY ENGINES ship them on send_stream (one strided 2-D peer copy per
+    // owner segment) while the next coset's NTT runs — no SM time, no NVLink stalls inside the NTT
     cudaStream_t send_stream = nullptr;
     cudaStream_t pull_stream = nullptr;   // peer -> local coefficient pulls of the coset-sharded plan.  NOT the copy stream: a stream that has
                                           // carried peer copies keeps its copy-engine binding, and host->device chunks queued behind it then
@@ -330,10 +323,6 @@ void launch_pass_a(gl_ctx* c, const ntt::PassParams& p, uint32_t threads, size_t
     ntt::ntt_pass_kernel<G, A><<<grid, threads, smem, c->stream>>>(p);
 }
 // second-generation pass (ntt2.cuh): two columns per thread, carry-save butterflies, all-shift radix-16 last round
-#ifndef LEAF_BLOCK
-#define LEAF_BLOCK 128
-#endif
-#define LEAF_BLOCK_PRELOAD LEAF_BLOCK
 // once per device: the shared-memory opt-in of a second-generation pass kernel (the attribute belongs to the function on a device)
 template <int G, int A>
 void prepare_pass2() {
@@ -379,7 +368,7 @@ void preload_stream_kernels() {
         load((const void*)ntt::ntt_tiny_kernel);
         load((const void*)peersync::signal_kernel);
         load((const void*)peersync::wait_kernel);
-        load((const void*)merkle::leaf_absorb_kernel<LEAF_BLOCK_PRELOAD>);
+        load((const void*)merkle::leaf_absorb_kernel<LEAF_BLOCK>);
         load((const void*)merkle::tree_level_kernel<128>);
     });
     CUDA_CHECK(e);
@@ -387,7 +376,7 @@ void preload_stream_kernels() {
     preload_pass2<8, 10>();
 }
 template <int G>
-bool launch_pass2(gl_ctx* c, ntt::PassParams p, uint32_t cols_padded, uint32_t* launches) {
+void launch_pass2(gl_ctx* c, ntt::PassParams p, uint32_t cols_padded, uint32_t* launches) {
     p.ncg = cols_padded / G;
     const uint64_t grid = (uint64_t)p.ncg << (p.log_n - p.a);
     if (grid >= (1ULL << 31)) GL_THROW(GL_ERR_UNSUPPORTED, "NTT grid too large");
@@ -400,17 +389,13 @@ bool launch_pass2(gl_ctx* c, ntt::PassParams p, uint32_t cols_padded, uint32_t* 
         case 8: launch_pass2_a<G, 8>(c, p, (uint32_t)grid); break;
         case 9: launch_pass2_a<G, 9>(c, p, (uint32_t)grid); break;
         case 10: launch_pass2_a<G, 10>(c, p, (uint32_t)grid); break;
-        case 11:
-            if (G != 4) return false;                       // 2048-row tiles: 4 columns keep the tile at 68 KB
-            launch_pass2_a<4, 11>(c, p, (uint32_t)grid);
-            break;
-        default: return false;
+        default: GL_THROW(GL_ERR_INVALID, "run_ntt: pass size %u has no second-generation kernel", p.a);
     }
     CUDA_CHECK(cudaGetLastError());
     if (launches) (*launches)++;
-    return true;
 }
 
+// first-generation pass (ntt.cuh): instantiated for what run_ntt launches with it — <2,0>, <4,3..10> and <8,3..9>
 template <int G>
 void launch_pass(gl_ctx* c, ntt::PassParams p, uint32_t cols_padded, uint32_t* launches) {
     p.ncg = cols_padded / G;
@@ -419,7 +404,7 @@ void launch_pass(gl_ctx* c, ntt::PassParams p, uint32_t cols_padded, uint32_t* l
     size_t smem = ((size_t)(T + (T >> 3)) * G + (T - (T >> 3))) * 8;   // padded tile + 7T/8 twiddles
     uint64_t grid = (uint64_t)p.ncg << (p.log_n - p.a);
     if (grid >= (1ULL << 31)) GL_THROW(GL_ERR_UNSUPPORTED, "NTT grid too large");
-    if (G == 2) {
+    if constexpr (G == 2) {
         launch_pass_a<G, 0>(c, p, threads, smem, (uint32_t)grid);      // FRI matrices: generic pass size
     } else {
         switch (p.a) {                                                  // pass size as a compile-time constant
@@ -430,7 +415,9 @@ void launch_pass(gl_ctx* c, ntt::PassParams p, uint32_t cols_padded, uint32_t* l
             case 7: launch_pass_a<G, 7>(c, p, threads, smem, (uint32_t)grid); break;
             case 8: launch_pass_a<G, 8>(c, p, threads, smem, (uint32_t)grid); break;
             case 9: launch_pass_a<G, 9>(c, p, threads, smem, (uint32_t)grid); break;
-            case 10: launch_pass_a<G, 10>(c, p, threads, smem, (uint32_t)grid); break;
+            case 10:
+                if constexpr (G == 4) { launch_pass_a<G, 10>(c, p, threads, smem, (uint32_t)grid); break; }
+                [[fallthrough]];                                        // 8 columns: run_ntt takes 10-stage passes in 4-column tiles
             default: GL_THROW(GL_ERR_INVALID, "bad pass size %u", p.a);
         }
     }
@@ -450,14 +437,11 @@ void run_ntt(gl_ctx* c, uint64_t* src, uint32_t src_pitch, uint64_t* dst, uint32
              const uint64_t* const* src_list = nullptr) {
     // src_list (forward, second-generation kernel only): the cols_padded / G column groups are read from separate [N][G] blocks
     // src_list[cg] (src and src_pitch ignored); the later passes run in place on dst with 8-column tiles when the width allows
-    if (src_list && (ifft || scatter || c->ntt_version < 2 || (G != 4 && G != 8) || log_n < 3 || cols_padded / G > (uint32_t)ntt::MAX_PEERS))
+    if (src_list && (ifft || scatter || (G != 4 && G != 8) || log_n < 3 || cols_padded / G > (uint32_t)ntt::MAX_PEERS))
         GL_THROW(GL_ERR_INVALID, "run_ntt: unsupported multi-source transform");
     const uint64_t* W = get_roots(c, log_n);
     uint64_t n_inv = ifft ? gl::h_inv(((uint64_t)1 << log_n) % gl::P) : 1;
-    // the second-generation kernel has an 11-stage form (2048-row tiles of 4 columns): 2^21 and 2^22 then take two passes instead of three
-    const bool wide = c->ntt_version >= 2 && (G == 8 || G == 4) && c->ntt_max_a >= 11 && cols_padded % 4 == 0 &&
-                      (log_n + 9) / 10 > (log_n + 10) / 11 && !src_list && src_pitch % 2 == 0 && dst_pitch % 2 == 0 && (uintptr_t)src % 16 == 0 && (uintptr_t)dst % 16 == 0;
-    auto passes = plan_passes(log_n, wide ? 11 : 10);
+    auto passes = plan_passes(log_n, 10);
     if (passes.empty()) {
         dim3 grid((cols_padded + 63) / 64, 1u << log_n);
         ntt::ntt_tiny_kernel<<<grid, 64, 0, c->stream>>>(src, dst, src_pitch, dst_pitch, cols_padded, log_n,
@@ -492,8 +476,10 @@ void run_ntt(gl_ctx* c, uint64_t* src, uint32_t src_pitch, uint64_t* dst, uint32
             p.src = first ? src : dst; p.src_pitch = first ? src_pitch : dst_pitch;
             p.dst = dst; p.dst_pitch = dst_pitch;
         }
-        int g = G;
+        // 128-bit accesses need even pitches and 16-byte aligned bases (true for every buffer this library lays out)
+        const bool aligned = p.src_pitch % 2 == 0 && p.dst_pitch % 2 == 0 && ((uintptr_t)p.src % 16 == 0) && ((uintptr_t)p.dst % 16 == 0);
         if (src_list) {
+            int g = G;
             if (first) {
                 p.src_list = 1; p.src = nullptr; p.src_pitch = (uint32_t)G;
                 for (uint32_t k = 0; k < cols_padded / G; k++) {
@@ -504,37 +490,24 @@ void run_ntt(gl_ctx* c, uint64_t* src, uint32_t src_pitch, uint64_t* dst, uint32
                 g = 8;
             }
             if (p.dst_pitch % 2 || (uintptr_t)p.dst % 16) GL_THROW(GL_ERR_INVALID, "run_ntt: misaligned destination");
-            if (p.a == 11) g = 4;
-            const bool ok = g == 8 ? launch_pass2<8>(c, p, cols_padded, launches) : launch_pass2<4>(c, p, cols_padded, launches);
-            if (!ok) GL_THROW(GL_ERR_INVALID, "run_ntt: pass size %u has no second-generation kernel", p.a);
-            log_blk -= passes[i];
-            continue;
-        }
-        if (c->ntt_version >= 2 && (g == 8 || g == 4)) {
-            // 128-bit accesses need even pitches and 16-byte aligned bases (true for every buffer this library lays out)
-            const bool aligned = p.src_pitch % 2 == 0 && p.dst_pitch % 2 == 0 && ((uintptr_t)p.src % 16 == 0) && ((uintptr_t)p.dst % 16 == 0);
-            if (g == 8 && p.a == 10 && c->ntt_g10 == 4) g = 4;
-            if (p.a == 11) g = 4;
-            if (aligned && (g == 8 ? launch_pass2<8>(c, p, cols_padded, launches) : launch_pass2<4>(c, p, cols_padded, launches))) {
-                log_blk -= passes[i];
-                continue;
+            g == 8 ? launch_pass2<8>(c, p, cols_padded, launches) : launch_pass2<4>(c, p, cols_padded, launches);
+        } else if ((G == 8 || G == 4) && aligned) {
+            G == 8 ? launch_pass2<8>(c, p, cols_padded, launches) : launch_pass2<4>(c, p, cols_padded, launches);
+        } else {
+            // first-generation kernel: the 2-column FRI matrices, and column groups whose base or pitch is not 16-byte aligned
+            switch (G) {
+                case 8:   // a 10-stage pass in 4-column tiles keeps 512 threads / 40 KB shared memory per CTA
+                    p.a == 10 ? launch_pass<4>(c, p, cols_padded, launches) : launch_pass<8>(c, p, cols_padded, launches);
+                    break;
+                case 4: launch_pass<4>(c, p, cols_padded, launches); break;
+                case 2: launch_pass<2>(c, p, cols_padded, launches); break;
+                default: GL_THROW(GL_ERR_INVALID, "bad column group");
             }
-            g = G;
-        }
-        if (g == 8 && p.a == 10) g = 4;   // keep 512 threads / 40 KB shared memory per CTA
-        switch (g) {
-            case 8: launch_pass<8>(c, p, cols_padded, launches); break;
-            case 4: launch_pass<4>(c, p, cols_padded, launches); break;
-            case 2: launch_pass<2>(c, p, cols_padded, launches); break;
-            default: GL_THROW(GL_ERR_INVALID, "bad column group");
         }
         log_blk -= passes[i];
     }
 }
 
-#ifndef LEAF_BLOCK
-#define LEAF_BLOCK 128
-#endif
 // the tree above the leaf digests: layers 1..log_sub, one launch per layer
 void merkle_levels(gl_ctx* c, uint64_t n_leaves, uint32_t cap_height, uint64_t* d_digests, uint64_t* d_cap, uint32_t* tree_launches) {
     const uint32_t log_sub = log2_exact(n_leaves) - cap_height;
@@ -599,110 +572,122 @@ Fri* find_fri(gl_ctx* c, gl_handle h) {
 
 void record(gl_ctx* c, int i) { CUDA_CHECK(cudaEventRecord(c->ev[i], c->stream)); }
 
+// Stage clock of one call: stage i runs from event i to event i + 1.  reset_stages zeroes the launch counts and times of the stages
+// [first, end) the call books; read_stages waits for the call's work and reads their times.
+void reset_stages(gl_ctx* c, int first, int end) {
+    for (int i = first; i < end; i++) { c->launches[i] = 0; c->stage_ms[i] = 0; }
+}
+void read_stages(gl_ctx* c, int first, int end) {
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    for (int i = first; i < end; i++) CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
+}
+
+void ensure_events(std::vector<cudaEvent_t>& v, size_t n) {   // at least n events without timing
+    while (v.size() < n) {
+        v.push_back(nullptr);
+        CUDA_CHECK(cudaEventCreateWithFlags(&v.back(), cudaEventDisableTiming));
+    }
+}
+
+// Column groups of 8 words (64 B row segments); a shard whose padding to 8 would waste >= 4 columns runs in groups of 4 (32 B = one
+// sector) instead.  coeff_pitch is the row pitch the shard's coefficients are laid out with.
+int column_group(uint32_t n_cols, uint32_t coeff_pitch) {
+    if (coeff_pitch % 4 || coeff_pitch < n_cols) GL_THROW(GL_ERR_INVALID, "coeff_pitch must be a multiple of 4 and >= n_cols");
+    const int G = (round_up(n_cols, 8) - n_cols >= 4) ? 4 : 8;
+    if (coeff_pitch < round_up(n_cols, (uint32_t)G)) GL_THROW(GL_ERR_INVALID, "coeff_pitch too small for the padded column group");
+    return G;
+}
+
+// Transpose of `n_cols` device columns (column-major, col_stride apart) into columns [0, width) of the row-major [N][pitch] `coeffs`
+// (zero beyond n_cols).  Values (vals != nullptr) go through the [N][pitch] scratch `vals` and an iNTT of groups of G columns.
+// split_events: the call is one stage clock of its own (the transpose ends the transpose stage, the iNTT the iNTT stage).
+void intt_columns(gl_ctx* c, const uint64_t* d_cols, uint64_t col_stride, uint32_t n_cols, uint32_t width, uint32_t log_n,
+                  uint64_t* vals, uint64_t* coeffs, uint32_t pitch, int G, bool split_events) {
+    const uint64_t N = 1ULL << log_n;
+    dim3 tb(32, 8), tg((uint32_t)((N + 31) / 32), (width + 31) / 32);
+    ntt::transpose_in_kernel<<<tg, tb, 0, c->stream>>>(d_cols, col_stride, vals ? vals : coeffs, pitch, width, n_cols, N);
+    CUDA_CHECK(cudaGetLastError());
+    c->launches[GL_STAGE_TRANSPOSE]++;
+    if (split_events) record(c, GL_STAGE_INTT);
+    if (vals) run_ntt(c, vals, pitch, coeffs, pitch, round_up(n_cols, (uint32_t)G), log_n, true, nullptr, G, &c->launches[GL_STAGE_INTT]);
+    if (split_events) record(c, GL_STAGE_LDE);
+}
+
+// One coset of a scattered LDE whose rows belong (partly) to other ranks: the coset is evaluated into send_buf[b] and the copy
+// engines ship it on send_stream, one strided 2-D peer copy per owner segment (no SM time), while the next coset's NTT runs on the
+// compute stream.  The buffer is reused only after its previous shipment has finished.
+void ship_coset(gl_ctx* c, uint64_t* coeffs, uint32_t coeff_pitch, uint32_t cols_padded, uint32_t log_n, const CosetTable* tab, int G,
+                const ntt::Scatter& sc, uint32_t col0, uint32_t row_pitch, int b) {
+    const uint64_t N = 1ULL << log_n;
+    uint64_t* buf = c->send_buf[b].p + col0;
+    if (c->sent_pending[b]) CUDA_CHECK(cudaStreamWaitEvent(c->stream, c->ev_sent[b], 0));
+    auto mark = [&](cudaStream_t st) {
+        if (!c->trace) return;
+        cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); c->trace_ev.push_back(e);
+    };
+    if (c->trace && c->trace_ev.empty()) mark(c->stream);
+    mark(c->stream);
+    run_ntt(c, coeffs, coeff_pitch, buf, row_pitch, cols_padded, log_n, false, tab, G, &c->launches[GL_STAGE_LDE]);
+    mark(c->stream);
+    CUDA_CHECK(cudaEventRecord(c->ev_ntt[b], c->stream));
+    CUDA_CHECK(cudaStreamWaitEvent(c->send_stream, c->ev_ntt[b], 0));
+    mark(c->send_stream);
+    const uint64_t rpp = 1ULL << sc.log_rows_per_peer;
+    for (uint64_t r = 0; r < N;) {
+        const uint64_t grow = sc.row0 + r, owner = grow >> sc.log_rows_per_peer, lrow = grow & (rpp - 1);
+        const uint64_t cnt = std::min<uint64_t>(N - r, rpp - lrow);
+        CUDA_CHECK(cudaMemcpy2DAsync(sc.peer[owner] + lrow * sc.pitch + sc.col0, (size_t)sc.pitch * 8, buf + r * row_pitch,
+                                     (size_t)row_pitch * 8, (size_t)sc.ncols * 8, cnt, cudaMemcpyDefault, c->send_stream));
+        r += cnt;
+    }
+    mark(c->send_stream);
+    c->launches[GL_STAGE_LDE]++;   // the shipment books as one launch of the LDE stage
+    CUDA_CHECK(cudaEventRecord(c->ev_sent[b], c->send_stream));
+    c->sent_pending[b] = true;
+}
 
 // iNTT + coset LDE of `n_cols` device columns (column-major, col_stride apart) into columns [col0, col0 + padded) of the
 // row-major outputs.  Column groups are independent, so a batch can be processed in chunks (pipelined behind the
 // host->device copies in gl_commit).  col0 must be a multiple of 8.
+// scatter != nullptr: every coset's rows go to their owners' leaf buffers (d_rows is then the NTT scratch of one coset): a coset
+// whose rows all belong to this rank is stored there by the NTT itself, every other coset is shipped by ship_coset.
 void lde_columns(gl_ctx* c, const uint64_t* d_cols, uint64_t col_stride, uint32_t col0, uint32_t n_cols, uint32_t width,
                  uint32_t log_n, uint32_t rate_bits, int is_coeffs, uint64_t* d_vals, uint64_t* d_coeffs, uint32_t coeff_pitch,
-                 uint64_t* d_rows, uint32_t row_pitch, int G, bool timed, bool split_events, const ntt::Scatter* scatter = nullptr,
-                 uint32_t first_coset = 0, bool intt_only = false) {
+                 uint64_t* d_rows, uint32_t row_pitch, int G, bool split_events, const ntt::Scatter* scatter = nullptr,
+                 uint32_t first_coset = 0) {
     const uint64_t N = 1ULL << log_n;
     const uint32_t cols_padded = round_up(n_cols, G);
     NvtxRange nv_lde(is_coeffs ? "FFT + blinding (coset LDE, leaves stored bit-reversed: includes 'transpose LDEs')"
                                : "IFFT, FFT + blinding (coset LDE, leaves stored bit-reversed: includes 'transpose LDEs')");
-    dim3 tb(32, 8);
-    dim3 tg((uint32_t)((N + 31) / 32), (width + 31) / 32);
-    uint32_t* l_tr = timed ? &c->launches[GL_STAGE_TRANSPOSE] : nullptr;
-    uint32_t* l_in = timed ? &c->launches[GL_STAGE_INTT] : nullptr;
-    uint32_t* l_ld = timed ? &c->launches[GL_STAGE_LDE] : nullptr;
     uint64_t* coeffs = d_coeffs + col0;
-    if (is_coeffs) {
-        ntt::transpose_in_kernel<<<tg, tb, 0, c->stream>>>(d_cols, col_stride, coeffs, coeff_pitch, width, n_cols, N);
-        CUDA_CHECK(cudaGetLastError());
-        if (l_tr) (*l_tr)++;
-        if (split_events) record(c, GL_STAGE_INTT);
-    } else {
-        ntt::transpose_in_kernel<<<tg, tb, 0, c->stream>>>(d_cols, col_stride, d_vals + col0, coeff_pitch, width, n_cols, N);
-        CUDA_CHECK(cudaGetLastError());
-        if (l_tr) (*l_tr)++;
-        if (split_events) record(c, GL_STAGE_INTT);
-        run_ntt(c, d_vals + col0, coeff_pitch, coeffs, coeff_pitch, cols_padded, log_n, true, nullptr, G, l_in);
-    }
-    if (split_events) record(c, GL_STAGE_LDE);
-    if (intt_only) return;                        // coset-sharded plan: the LDE runs after the coefficient exchange
+    intt_columns(c, d_cols, col_stride, n_cols, width, log_n, is_coeffs ? nullptr : d_vals + col0, coeffs, coeff_pitch, G, split_events);
     const auto& tabs = get_lde_tables(c, log_n, rate_bits);
     for (uint32_t k = 0; k < (1u << rate_bits); k++) {
         const uint32_t s = (k + first_coset) & ((1u << rate_bits) - 1);
-        if (scatter) {   // d_rows is an [N][row_pitch] scratch reused by every coset (stream order)
-            ntt::Scatter sc = *scatter;
-            sc.row0 = (uint64_t)h_bitrev(s, rate_bits) * N;
-            sc.col0 = scatter->col0 + col0;   // this chunk's columns inside the leaf row
-            sc.ncols = n_cols;
-            // rows of this coset that live in this rank's own leaf buffer need no shipment: the NTT stores them itself
-            const bool all_local = scatter->self < ntt::MAX_PEERS && (sc.row0 >> sc.log_rows_per_peer) == scatter->self &&
-                                   ((sc.row0 + N - 1) >> sc.log_rows_per_peer) == scatter->self;
-            if (c->scatter_mode == 0 || (c->scatter_mode == 3 && all_local)) {
-                run_ntt(c, coeffs, coeff_pitch, d_rows + col0, row_pitch, cols_padded, log_n, false, &tabs[s], G, l_ld, &sc);
-            } else {
-                // coset result into one of two local buffers; the copy kernel ships it on send_stream while the next coset's
-                // NTT runs on the compute stream (the buffer is reused only after its previous shipment has finished)
-                const int b = (int)(k & 1);
-                uint64_t* buf = c->send_buf[b].p + col0;
-                if (c->sent_pending[b]) CUDA_CHECK(cudaStreamWaitEvent(c->stream, c->ev_sent[b], 0));
-                auto mark = [&](cudaStream_t st) {
-                    if (!c->trace) return;
-                    cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); c->trace_ev.push_back(e);
-                };
-                if (c->trace && c->trace_ev.empty()) mark(c->stream);
-                mark(c->stream);
-                run_ntt(c, coeffs, coeff_pitch, buf, row_pitch, cols_padded, log_n, false, &tabs[s], G, l_ld);
-                mark(c->stream);
-                CUDA_CHECK(cudaEventRecord(c->ev_ntt[b], c->stream));
-                if (c->scatter_mode != 2) CUDA_CHECK(cudaStreamWaitEvent(c->send_stream, c->ev_ntt[b], 0));
-                cudaStream_t ss = c->scatter_mode == 2 ? c->stream : c->send_stream;   // 2: no overlap (measurement aid)
-                mark(ss);
-                const uint32_t words = round_up(n_cols, 2);                            // a padding column may ride along
-                if (c->scatter_mode == 3) {
-                    // copy engines: one strided 2-D peer copy per owner segment of this coset (no SM time at all)
-                    const uint64_t rpp = 1ULL << sc.log_rows_per_peer;
-                    for (uint64_t r = 0; r < N;) {
-                        const uint64_t grow = sc.row0 + r, owner = grow >> sc.log_rows_per_peer, lrow = grow & (rpp - 1);
-                        const uint64_t cnt = std::min<uint64_t>(N - r, rpp - lrow);
-                        CUDA_CHECK(cudaMemcpy2DAsync(sc.peer[owner] + lrow * sc.pitch + sc.col0, (size_t)sc.pitch * 8, buf + r * row_pitch,
-                                                     (size_t)row_pitch * 8, (size_t)n_cols * 8, cnt, cudaMemcpyDefault, ss));
-                        r += cnt;
-                    }
-                } else if (row_pitch % 2 == 0 && sc.pitch % 2 == 0 && sc.col0 % 2 == 0 && sc.col0 + words <= sc.pitch && words / 2 <= 256 && N < (1ULL << 32)) {
-                    const uint32_t n_vec = words / 2, lane_rows = 256 / n_vec;
-                    const uint32_t blocks = (uint32_t)std::min<uint64_t>((N + lane_rows - 1) / lane_rows, (uint64_t)c->sm_count * 2);
-                    ntt::scatter_copy16_kernel<<<blocks, 256, 0, ss>>>(reinterpret_cast<const ulonglong2*>(buf), row_pitch / 2, n_vec, (uint32_t)N, sc);
-                } else {
-                    const uint64_t total = N * n_cols;
-                    const uint32_t blocks = (uint32_t)std::min<uint64_t>((total + 255) / 256, (uint64_t)c->sm_count * 4);
-                    ntt::scatter_copy_kernel<<<blocks, 256, 0, ss>>>(buf, row_pitch, n_cols, N, sc);
-                }
-                CUDA_CHECK(cudaGetLastError());
-                mark(ss);
-                if (l_ld) (*l_ld)++;
-                CUDA_CHECK(cudaEventRecord(c->ev_sent[b], ss));
-                c->sent_pending[b] = true;
-            }
-        } else {
+        if (!scatter) {
             uint64_t* dst = d_rows + (uint64_t)h_bitrev(s, rate_bits) * N * row_pitch + col0;
-            run_ntt(c, coeffs, coeff_pitch, dst, row_pitch, cols_padded, log_n, false, &tabs[s], G, l_ld);
+            run_ntt(c, coeffs, coeff_pitch, dst, row_pitch, cols_padded, log_n, false, &tabs[s], G, &c->launches[GL_STAGE_LDE]);
+            continue;
         }
+        ntt::Scatter sc = *scatter;
+        sc.row0 = (uint64_t)h_bitrev(s, rate_bits) * N;
+        sc.col0 = scatter->col0 + col0;   // this chunk's columns inside the leaf row
+        sc.ncols = n_cols;
+        const bool all_local = scatter->self < ntt::MAX_PEERS && (sc.row0 >> sc.log_rows_per_peer) == scatter->self &&
+                               ((sc.row0 + N - 1) >> sc.log_rows_per_peer) == scatter->self;
+        if (all_local)
+            run_ntt(c, coeffs, coeff_pitch, d_rows + col0, row_pitch, cols_padded, log_n, false, &tabs[s], G, &c->launches[GL_STAGE_LDE], &sc);
+        else
+            ship_coset(c, coeffs, coeff_pitch, cols_padded, log_n, &tabs[s], G, sc, col0, row_pitch, (int)(k & 1));
     }
 }
 
 void lde_stage(gl_ctx* c, const uint64_t* d_cols, uint64_t col_stride, uint32_t n_cols, uint32_t log_n, uint32_t rate_bits,
-               int is_coeffs, uint64_t* d_coeffs, uint32_t coeff_pitch, uint64_t* d_rows, uint32_t row_pitch, bool timed) {
-    // column groups of 8 words (64 B row segments); a narrow shard whose padding to 8 would waste >= 4 columns runs
-    // in groups of 4 (32 B = one sector) instead
-    const int G = (round_up(n_cols, 8) - n_cols >= 4 && coeff_pitch % 4 == 0 && row_pitch % 4 == 0) ? 4 : 8;
+               int is_coeffs, uint64_t* d_coeffs, uint32_t coeff_pitch, uint64_t* d_rows, uint32_t row_pitch) {
+    const int G = column_group(n_cols, coeff_pitch);
     if (!is_coeffs) c->vals.ensure(((uint64_t)1 << log_n) * coeff_pitch);
     lde_columns(c, d_cols, col_stride, 0, n_cols, coeff_pitch, log_n, rate_bits, is_coeffs, c->vals.p, d_coeffs, coeff_pitch, d_rows,
-                row_pitch, G, timed, timed);
+                row_pitch, G, true);
 }
 
 // Host columns -> c->in_stage in chunks on the copy stream; fn(c0, nc, first) runs on the compute stream once chunk
@@ -719,11 +704,7 @@ void for_each_host_chunk(gl_ctx* c, const uint64_t* const* host_cols, uint32_t n
     // — fewer, larger launches and fewer sponge-state hand-overs
     for (uint32_t c0 = 0, sz = 8; c0 < n_cols; c0 += sz, sz = doubling ? std::min(2 * sz, 64u) : std::min(sz + 8, 24u))
         chunks.push_back({c0, std::min(sz, n_cols - c0)});
-    if (c->chunk_ev.size() < chunks.size()) {
-        size_t old = c->chunk_ev.size();
-        c->chunk_ev.resize(chunks.size(), nullptr);
-        for (size_t i = old; i < chunks.size(); i++) CUDA_CHECK(cudaEventCreateWithFlags(&c->chunk_ev[i], cudaEventDisableTiming));
-    }
+    ensure_events(c->chunk_ev, chunks.size());
     CUDA_CHECK(cudaEventRecord(c->ev_sync, c->stream));              // in_stage may still be read by an earlier call
     CUDA_CHECK(cudaStreamWaitEvent(c->copy_stream, c->ev_sync, 0));
     for (size_t k = 0; k < chunks.size(); k++) {
@@ -756,31 +737,31 @@ int commit_impl(gl_ctx* c, const uint64_t* const* host_cols, const uint64_t* d_c
     t->digests.ensure(n_dig * 4);
     t->d_cap.ensure(4ULL << cap_height);
     t->cap.resize(4ULL << cap_height);
-    memset(c->launches, 0, sizeof c->launches);
+    reset_stages(c, 0, GL_N_STAGES);
 
     record(c, GL_STAGE_H2D);
     // Host columns with more than one chunk: the leaf sponge runs chunk by chunk behind the LDE of each chunk (leaf_absorb_kernel), so the
     // PCIe copy of the later chunks hides behind hashing; the stage clock then books those launches under "lde" (they interleave with it).
-    const bool stream_hash = host_cols && c->stream_hash && n_cols > 8 && n_cols > 4;
+    const bool hash_per_chunk = host_cols && n_cols > 8;
     bool leaves_hashed = false;
     if (host_cols) {
         if (!is_coeffs) c->vals.ensure(N * pitch);
-        if (stream_hash) c->hash_state.ensure(12 * R);
+        if (hash_per_chunk) c->hash_state.ensure(12 * R);
         for_each_host_chunk(c, host_cols, n_cols, N, [&](uint32_t c0, uint32_t nc, bool first) {
             const uint32_t width = std::min(round_up(nc, 8), pitch - c0);
             if (first) { record(c, GL_STAGE_TRANSPOSE); record(c, GL_STAGE_INTT); record(c, GL_STAGE_LDE); }   // h2d = first chunk
             lde_columns(c, c->in_stage.p + (uint64_t)c0 * N, N, c0, nc, width, log_n, rate_bits, is_coeffs, c->vals.p, t->coeffs.p, pitch,
-                        t->leaves.p, pitch, 8, true, false);
-            if (stream_hash) {
+                        t->leaves.p, pitch, 8, false);
+            if (hash_per_chunk) {
                 const bool last = c0 + nc == n_cols;
                 leaf_absorb(c, t->leaves.p, R, n_cols, pitch, cap_height, c0, c0 + nc, c->hash_state.p, t->digests.p, t->d_cap.p, c0 == 0, last,
                             &c->launches[GL_STAGE_LEAF_HASH]);
                 leaves_hashed = leaves_hashed || last;
             }
-        }, stream_hash);
+        }, hash_per_chunk);
     } else {
         record(c, GL_STAGE_TRANSPOSE);
-        lde_stage(c, d_cols_in, col_stride, n_cols, log_n, rate_bits, is_coeffs, t->coeffs.p, pitch, t->leaves.p, pitch, true);
+        lde_stage(c, d_cols_in, col_stride, n_cols, log_n, rate_bits, is_coeffs, t->coeffs.p, pitch, t->leaves.p, pitch);
     }
     // Copy-back of the coefficients and the leaves (a host that materialises PolynomialBatch::polynomials / MerkleTree::leaves) leaves
     // on the copy stream as soon as the LDE is done, i.e. PCIe runs while the tree is hashed; only the digests wait for the hash.
@@ -818,8 +799,7 @@ int commit_impl(gl_ctx* c, const uint64_t* const* host_cols, const uint64_t* d_c
         CUDA_CHECK(cudaMemcpyAsync(out_digests, t->digests.p, n_dig * 32, cudaMemcpyDeviceToHost, c->stream));
     if (early_copyback) CUDA_CHECK(cudaStreamWaitEvent(c->stream, c->ev_copyback, 0));   // the d2h stage ends when everything has landed
     record(c, GL_N_STAGES);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    for (int i = 0; i < GL_N_STAGES; i++) CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
+    read_stages(c, 0, GL_N_STAGES);
     memcpy(out_cap, t->cap.data(), 32ULL << cap_height);
     if (out_batch) *out_batch = put_tree(c, std::move(t));
     return GL_OK;
@@ -888,7 +868,7 @@ int gl_ctx_create(gl_ctx** out, int device) {
     if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
     if (cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
     {
-        int lo = 0, hi = 0;   // the shipment's few CTAs must get SM slots as NTT CTAs retire, not queue behind the whole NTT grid
+        int lo = 0, hi = 0;   // the streamed coset plan's few iNTT CTAs must get SM slots as hashing CTAs retire, not queue behind a whole grid
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
         if (cudaStreamCreateWithPriority(&c->send_stream, cudaStreamNonBlocking, hi) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
     }
@@ -896,12 +876,7 @@ int gl_ctx_create(gl_ctx** out, int device) {
         if (cudaEventCreateWithFlags(&c->ev_ntt[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&c->ev_sent[i], cudaEventDisableTiming) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
     if (cudaStreamCreateWithFlags(&c->pull_stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
-    if (const char* m = getenv("GL_SCATTER_MODE")) c->scatter_mode = atoi(m);
     if (const char* m = getenv("GL_TRACE")) c->trace = atoi(m) != 0;
-    if (const char* m = getenv("GL_STREAM_HASH")) c->stream_hash = atoi(m) != 0;
-    if (const char* m = getenv("GL_NTT_VERSION")) c->ntt_version = atoi(m);
-    if (const char* m = getenv("GL_NTT_G10")) c->ntt_g10 = atoi(m);
-    if (const char* m = getenv("GL_NTT_MAX_A")) c->ntt_max_a = atoi(m);
     if (cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
     if (cudaEventCreateWithFlags(&c->ev_copyback, cudaEventDisableTiming) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
     for (auto& e : c->ev)
@@ -980,13 +955,11 @@ int gl_dev_lde(gl_ctx* c, const uint64_t* d_cols, uint64_t col_stride, uint32_t 
     if (!coeffs) { c->scratch.ensure(((uint64_t)1 << log_n) * out_pitch); coeffs = c->scratch.p; }
     get_roots(c, log_n);
     get_lde_tables(c, log_n, rate_bits);
-    for (int i : {GL_STAGE_H2D, GL_STAGE_TRANSPOSE, GL_STAGE_INTT, GL_STAGE_LDE}) { c->launches[i] = 0; c->stage_ms[i] = 0; }
+    reset_stages(c, GL_STAGE_H2D, GL_STAGE_LEAF_HASH);
     record(c, GL_STAGE_TRANSPOSE);
-    lde_stage(c, d_cols, col_stride, n_cols, log_n, rate_bits, input_is_coeffs, coeffs, out_pitch, d_out_rows, out_pitch, true);
+    lde_stage(c, d_cols, col_stride, n_cols, log_n, rate_bits, input_is_coeffs, coeffs, out_pitch, d_out_rows, out_pitch);
     record(c, GL_STAGE_LEAF_HASH);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    for (int i : {GL_STAGE_TRANSPOSE, GL_STAGE_INTT, GL_STAGE_LDE})
-        CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
+    read_stages(c, GL_STAGE_TRANSPOSE, GL_STAGE_LEAF_HASH);
     return GL_OK;
     GL_API_END(c)
 }
@@ -1000,10 +973,8 @@ static int lde_scatter_impl(gl_ctx* c, const uint64_t* d_cols, const uint64_t* c
     if (n_peers == 0 || (n_peers & (n_peers - 1)) || n_peers > ntt::MAX_PEERS) GL_THROW(GL_ERR_INVALID, "n_peers must be a power of two <= %d", ntt::MAX_PEERS);
     const uint64_t N = 1ULL << log_n, R = N << rate_bits;
     if (R < n_peers) GL_THROW(GL_ERR_INVALID, "fewer leaf rows than peers");
-    if (coeff_pitch % 4 || coeff_pitch < n_cols) GL_THROW(GL_ERR_INVALID, "coeff_pitch must be a multiple of 4 and >= n_cols");
-    const int G = (round_up(n_cols, 8) - n_cols >= 4) ? 4 : 8;
+    const int G = column_group(n_cols, coeff_pitch);
     if (col_off + n_cols > leaf_pitch) GL_THROW(GL_ERR_INVALID, "columns do not fit the leaf pitch");
-    if (coeff_pitch < round_up(n_cols, G)) GL_THROW(GL_ERR_INVALID, "coeff_pitch too small for the padded column group");
     ntt::Scatter sc{};
     for (uint32_t q = 0; q < n_peers; q++) {
         if (!peer_leaves[q]) GL_THROW(GL_ERR_INVALID, "peer_leaves[%u] is NULL", q);
@@ -1021,25 +992,26 @@ static int lde_scatter_impl(gl_ctx* c, const uint64_t* d_cols, const uint64_t* c
     get_lde_tables(c, log_n, rate_bits);
     c->scratch.ensure(N * coeff_pitch);      // pass scratch of one coset
     if (!input_is_coeffs) c->vals.ensure(N * coeff_pitch);
-    if (c->scatter_mode) { c->send_buf[0].ensure(N * coeff_pitch); c->send_buf[1].ensure(N * coeff_pitch); }
-    for (int i : {GL_STAGE_H2D, GL_STAGE_TRANSPOSE, GL_STAGE_INTT, GL_STAGE_LDE}) { c->launches[i] = 0; c->stage_ms[i] = 0; }
+    c->send_buf[0].ensure(N * coeff_pitch);
+    c->send_buf[1].ensure(N * coeff_pitch);
+    reset_stages(c, GL_STAGE_H2D, GL_STAGE_LEAF_HASH);
     if (host_cols) {
         record(c, GL_STAGE_H2D);
         for_each_host_chunk(c, host_cols, n_cols, N, [&](uint32_t c0, uint32_t nc, bool first) {
             const uint32_t width = std::min(round_up(nc, (uint32_t)G), coeff_pitch - c0);
             if (first) { record(c, GL_STAGE_TRANSPOSE); record(c, GL_STAGE_INTT); record(c, GL_STAGE_LDE); }
             lde_columns(c, c->in_stage.p + (uint64_t)c0 * N, N, c0, nc, width, log_n, rate_bits, input_is_coeffs, c->vals.p, d_out_coeffs,
-                        coeff_pitch, c->scratch.p, coeff_pitch, G, true, false, &sc, first_coset);
+                        coeff_pitch, c->scratch.p, coeff_pitch, G, false, &sc, first_coset);
         });
     } else {
         record(c, GL_STAGE_TRANSPOSE);
         lde_columns(c, d_cols, col_stride, 0, n_cols, coeff_pitch, log_n, rate_bits, input_is_coeffs, c->vals.p, d_out_coeffs, coeff_pitch,
-                    c->scratch.p, coeff_pitch, G, true, true, &sc, first_coset);
+                    c->scratch.p, coeff_pitch, G, true, &sc, first_coset);
     }
     for (int b = 0; b < 2; b++)              // join the shipments: the LDE stage ends when the last coset has left
         if (c->sent_pending[b]) { CUDA_CHECK(cudaStreamWaitEvent(c->stream, c->ev_sent[b], 0)); c->sent_pending[b] = false; }
     record(c, GL_STAGE_LEAF_HASH);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    read_stages(c, host_cols ? GL_STAGE_H2D : GL_STAGE_TRANSPOSE, GL_STAGE_LEAF_HASH);
     if (c->trace && c->trace_ev.size() > 1) {
         cudaStreamSynchronize(c->send_stream);
         fprintf(stderr, "[gl trace dev %d] coset: ntt start-end | send start-end (ms)\n", c->device);
@@ -1051,8 +1023,6 @@ static int lde_scatter_impl(gl_ctx* c, const uint64_t* d_cols, const uint64_t* c
         for (auto e : c->trace_ev) cudaEventDestroy(e);
         c->trace_ev.clear();
     }
-    for (int i : {GL_STAGE_H2D, GL_STAGE_TRANSPOSE, GL_STAGE_INTT, GL_STAGE_LDE})
-        if (host_cols || i != GL_STAGE_H2D) CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
     return GL_OK;
 }
 
@@ -1077,63 +1047,46 @@ int gl_lde_scatter(gl_ctx* c, const uint64_t* const* cols, uint32_t n_cols, uint
 }
 
 // ---- coset-sharded commit: exchange coefficients, evaluate only the cosets this rank owns (include/gl_commit.h) ---------------------
+// iNTT of a column shard from device (d_cols) or host columns into the row-major [N][coeff_pitch] coefficients the peers pull
+static int intt_impl(gl_ctx* c, const uint64_t* d_cols, const uint64_t* const* host_cols, uint64_t col_stride, uint32_t n_cols, uint32_t log_n,
+                     int input_is_coeffs, uint64_t* d_out_coeffs, uint32_t coeff_pitch) {
+    check_shape(n_cols, log_n, 0, 0);
+    const int G = column_group(n_cols, coeff_pitch);
+    const uint64_t N = 1ULL << log_n;
+    get_roots(c, log_n);
+    if (!input_is_coeffs) c->vals.ensure(N * coeff_pitch);
+    reset_stages(c, GL_STAGE_H2D, GL_STAGE_LEAF_HASH);
+    if (host_cols) {
+        record(c, GL_STAGE_H2D);
+        // the shard crosses PCIe in chunks; transpose + iNTT of chunk k run while chunk k+1 is on the wire
+        for_each_host_chunk(c, host_cols, n_cols, N, [&](uint32_t c0, uint32_t nc, bool first) {
+            const uint32_t width = std::min(round_up(nc, (uint32_t)G), coeff_pitch - c0);
+            if (first) { record(c, GL_STAGE_TRANSPOSE); record(c, GL_STAGE_INTT); }
+            intt_columns(c, c->in_stage.p + (uint64_t)c0 * N, N, nc, width, log_n, input_is_coeffs ? nullptr : c->vals.p + c0, d_out_coeffs + c0,
+                         coeff_pitch, G, false);
+        });
+        record(c, GL_STAGE_LDE);
+    } else {
+        record(c, GL_STAGE_TRANSPOSE);
+        intt_columns(c, d_cols, col_stride, n_cols, coeff_pitch, log_n, input_is_coeffs ? nullptr : c->vals.p, d_out_coeffs, coeff_pitch, G, true);
+    }
+    read_stages(c, host_cols ? GL_STAGE_H2D : GL_STAGE_TRANSPOSE, GL_STAGE_LDE);
+    return GL_OK;
+}
+
 int gl_dev_intt(gl_ctx* c, const uint64_t* d_cols, uint64_t col_stride, uint32_t n_cols, uint32_t log_n, int input_is_coeffs,
                 uint64_t* d_out_coeffs, uint32_t coeff_pitch) {
     GL_API_BEGIN(c)
-    check_shape(n_cols, log_n, 0, 0);
     if (!d_cols || !d_out_coeffs) GL_THROW(GL_ERR_INVALID, "NULL device pointer");
-    if (coeff_pitch % 4 || coeff_pitch < n_cols) GL_THROW(GL_ERR_INVALID, "coeff_pitch must be a multiple of 4 and >= n_cols");
-    const int G = (round_up(n_cols, 8) - n_cols >= 4) ? 4 : 8;
-    if (coeff_pitch < round_up(n_cols, (uint32_t)G)) GL_THROW(GL_ERR_INVALID, "coeff_pitch too small for the padded column group");
-    const uint64_t N = 1ULL << log_n;
-    get_roots(c, log_n);
-    for (int i : {GL_STAGE_H2D, GL_STAGE_TRANSPOSE, GL_STAGE_INTT, GL_STAGE_LDE}) { c->launches[i] = 0; c->stage_ms[i] = 0; }
-    record(c, GL_STAGE_TRANSPOSE);
-    dim3 tb(32, 8), tg((uint32_t)((N + 31) / 32), (coeff_pitch + 31) / 32);
-    if (input_is_coeffs) {
-        ntt::transpose_in_kernel<<<tg, tb, 0, c->stream>>>(d_cols, col_stride, d_out_coeffs, coeff_pitch, coeff_pitch, n_cols, N);
-        CUDA_CHECK(cudaGetLastError());
-        c->launches[GL_STAGE_TRANSPOSE]++;
-        record(c, GL_STAGE_INTT);
-    } else {
-        c->vals.ensure(N * coeff_pitch);
-        ntt::transpose_in_kernel<<<tg, tb, 0, c->stream>>>(d_cols, col_stride, c->vals.p, coeff_pitch, coeff_pitch, n_cols, N);
-        CUDA_CHECK(cudaGetLastError());
-        c->launches[GL_STAGE_TRANSPOSE]++;
-        record(c, GL_STAGE_INTT);
-        run_ntt(c, c->vals.p, coeff_pitch, d_out_coeffs, coeff_pitch, round_up(n_cols, (uint32_t)G), log_n, true, nullptr, G, &c->launches[GL_STAGE_INTT]);
-    }
-    record(c, GL_STAGE_LDE);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    for (int i : {GL_STAGE_TRANSPOSE, GL_STAGE_INTT}) CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
-    return GL_OK;
+    return intt_impl(c, d_cols, nullptr, col_stride, n_cols, log_n, input_is_coeffs, d_out_coeffs, coeff_pitch);
     GL_API_END(c)
 }
 
 int gl_intt_host(gl_ctx* c, const uint64_t* const* cols, uint32_t n_cols, uint32_t log_n, int input_is_coeffs, uint64_t* d_out_coeffs,
                  uint32_t coeff_pitch) {
     GL_API_BEGIN(c)
-    check_shape(n_cols, log_n, 0, 0);
     if (!cols || !d_out_coeffs) GL_THROW(GL_ERR_INVALID, "NULL pointer");
-    if (coeff_pitch % 4 || coeff_pitch < n_cols) GL_THROW(GL_ERR_INVALID, "coeff_pitch must be a multiple of 4 and >= n_cols");
-    const int G = (round_up(n_cols, 8) - n_cols >= 4) ? 4 : 8;
-    if (coeff_pitch < round_up(n_cols, (uint32_t)G)) GL_THROW(GL_ERR_INVALID, "coeff_pitch too small for the padded column group");
-    const uint64_t N = 1ULL << log_n;
-    get_roots(c, log_n);
-    if (!input_is_coeffs) c->vals.ensure(N * coeff_pitch);
-    for (int i : {GL_STAGE_H2D, GL_STAGE_TRANSPOSE, GL_STAGE_INTT, GL_STAGE_LDE}) { c->launches[i] = 0; c->stage_ms[i] = 0; }
-    record(c, GL_STAGE_H2D);
-    // the shard crosses PCIe in chunks; transpose + iNTT of chunk k run while chunk k+1 is on the wire
-    for_each_host_chunk(c, cols, n_cols, N, [&](uint32_t c0, uint32_t nc, bool first) {
-        const uint32_t width = std::min(round_up(nc, (uint32_t)G), coeff_pitch - c0);
-        if (first) { record(c, GL_STAGE_TRANSPOSE); record(c, GL_STAGE_INTT); }
-        lde_columns(c, c->in_stage.p + (uint64_t)c0 * N, N, c0, nc, width, log_n, 0, input_is_coeffs, c->vals.p, d_out_coeffs, coeff_pitch, nullptr, 0, G,
-                    true, false, nullptr, 0, true);
-    });
-    record(c, GL_STAGE_LDE);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    for (int i : {GL_STAGE_H2D, GL_STAGE_TRANSPOSE, GL_STAGE_INTT}) CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
-    return GL_OK;
+    return intt_impl(c, nullptr, cols, 0, n_cols, log_n, input_is_coeffs, d_out_coeffs, coeff_pitch);
     GL_API_END(c)
 }
 
@@ -1154,12 +1107,8 @@ int gl_dev_lde_own_cosets(gl_ctx* c, uint64_t* const* peer_coeffs, uint64_t* con
     }
     get_roots(c, log_n);
     const auto& tabs = get_lde_tables(c, log_n, rate_bits);
-    if (c->pull_ev.size() < n_peers) {
-        size_t old = c->pull_ev.size();
-        c->pull_ev.resize(n_peers, nullptr);
-        for (size_t i = old; i < n_peers; i++) CUDA_CHECK(cudaEventCreateWithFlags(&c->pull_ev[i], cudaEventDisableTiming));
-    }
-    c->launches[GL_STAGE_LDE] = 0; c->stage_ms[GL_STAGE_LDE] = 0;
+    ensure_events(c->pull_ev, n_peers);
+    reset_stages(c, GL_STAGE_LDE, GL_STAGE_LEAF_HASH);
     record(c, GL_STAGE_LDE);
     // every pull is enqueued up front on the copy stream, nearest neighbour first (rank q pulls from q+1, q+2, ...: at any moment every
     // rank reads from a different peer); the compute stream takes the blocks in the same order, own block first
@@ -1179,8 +1128,7 @@ int gl_dev_lde_own_cosets(gl_ctx* c, uint64_t* const* peer_coeffs, uint64_t* con
         const uint32_t q = (self + k) % n_peers;
         const uint64_t* coeffs = q == self ? peer_coeffs[q] : d_stage[q];
         if (q != self) CUDA_CHECK(cudaStreamWaitEvent(c->stream, c->pull_ev[q], 0));
-        const int G = (round_up(col_counts[q], 8) - col_counts[q] >= 4 || pitches[q] % 8) ? 4 : 8;
-        if (pitches[q] < round_up(col_counts[q], (uint32_t)G)) GL_THROW(GL_ERR_INVALID, "peer %u: pitch too small for the padded column group", q);
+        const int G = (column_group(col_counts[q], pitches[q]) == 4 || pitches[q] % 8) ? 4 : 8;   // 8-column tiles need a pitch of whole groups
         for (uint32_t b = 0; b < blocks_per_rank; b++) {
             const uint32_t s = h_bitrev(first_block + b, rate_bits);       // leaf block b of the batch is LDE coset bitrev_r(b)
             uint64_t* dst = d_leaves + (uint64_t)b * N * leaf_pitch + col_offsets[q];
@@ -1189,8 +1137,7 @@ int gl_dev_lde_own_cosets(gl_ctx* c, uint64_t* const* peer_coeffs, uint64_t* con
         }
     }
     record(c, GL_STAGE_LEAF_HASH);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[GL_STAGE_LDE], c->ev[GL_STAGE_LDE], c->ev[GL_STAGE_LEAF_HASH]));
+    read_stages(c, GL_STAGE_LDE, GL_STAGE_LEAF_HASH);
     if (c->trace) {   // NVLink ingress of this rank: the G-1 coefficient blocks, back to back on the copy engine
         cudaStreamSynchronize(c->pull_stream);
         float ms = 0;
@@ -1276,18 +1223,13 @@ void coset_stream_impl(gl_ctx* c, const gl_stream_plan_t* plan, const uint64_t* 
         c->scratch.ensure(std::max<uint64_t>(4ULL << cap_height, 1));
         d_cap = c->scratch.p;
     }
-    auto grow = [](std::vector<cudaEvent_t>& v, size_t n) {
-        size_t old = v.size();
-        if (old >= n) return;
-        v.resize(n, nullptr);
-        for (size_t i = old; i < n; i++) CUDA_CHECK(cudaEventCreateWithFlags(&v[i], cudaEventDisableTiming));
-    };
-    grow(c->chunk_ev, W); grow(c->own_ev, W); grow(c->pull_ev, (size_t)W * G);
+    ensure_events(c->chunk_ev, W);
+    ensure_events(c->own_ev, W);
+    ensure_events(c->pull_ev, (size_t)W * G);
     uint64_t timeout_ns = 20000ULL * 1000000ULL;
     if (const char* m = getenv("GL_PEER_TIMEOUT_MS")) timeout_ns = strtoull(m, nullptr, 10) * 1000000ULL;
     const uint64_t ticket0 = plan->epoch * W + 1;                        // wave w publishes ticket0 + w
-    memset(c->launches, 0, sizeof c->launches);
-    memset(c->stage_ms, 0, sizeof c->stage_ms);
+    reset_stages(c, 0, GL_N_STAGES);
 
     record(c, GL_STAGE_H2D);
     CUDA_CHECK(cudaMemsetAsync(c->sync_err.p, 0, 8, c->stream));
@@ -1312,12 +1254,8 @@ void coset_stream_impl(gl_ctx* c, const gl_stream_plan_t* plan, const uint64_t* 
             const uint32_t nc = L.cols(self, w);
             if (!nc) continue;
             CUDA_CHECK(cudaStreamWaitEvent(c->stream, c->chunk_ev[w], 0));
-            uint64_t* block = own_buf + w * blk;
-            dim3 tb(32, 8), tg((uint32_t)((N + 31) / 32), (gw + 31) / 32);
-            ntt::transpose_in_kernel<<<tg, tb, 0, c->stream>>>(c->in_stage.p + w * blk, N, input_is_coeffs ? block : c->vals.p + w * blk, gw, gw, nc, N);
-            CUDA_CHECK(cudaGetLastError());
-            c->launches[GL_STAGE_TRANSPOSE]++;
-            if (!input_is_coeffs) run_ntt(c, c->vals.p + w * blk, gw, block, gw, gw, log_n, true, nullptr, (int)gw, &c->launches[GL_STAGE_INTT]);
+            intt_columns(c, c->in_stage.p + w * blk, N, nc, gw, log_n, input_is_coeffs ? nullptr : c->vals.p + w * blk, own_buf + w * blk, gw,
+                         (int)gw, false);
             CUDA_CHECK(cudaEventRecord(c->own_ev[w], c->stream));
             if (G > 1) {
                 peersync::Slots s{};
@@ -1351,7 +1289,7 @@ void coset_stream_impl(gl_ctx* c, const gl_stream_plan_t* plan, const uint64_t* 
     // transforms of 32-byte row segments, 16 small launches per wave at 8 GPUs — measured 0.95 ms per wave against 0.6 for this form.)
     // The FIRST wave keeps per-group launches: its groups arrive one by one behind the slowest rank's copy, and transforming each as it
     // lands hides the NTTs behind the remaining pulls (8 GPUs: first wave done at 3.3 ms instead of 3.9).
-    const bool can_merge = c->ntt_version >= 2 && log_n >= 3 && c->ntt_max_a <= 10;
+    const bool can_merge = log_n >= 3;
     for (uint32_t w = 0; w < W; w++) {
         const bool one_launch = can_merge && w > 0;
         bool first_in_wave = true;
@@ -1392,10 +1330,9 @@ void coset_stream_impl(gl_ctx* c, const gl_stream_plan_t* plan, const uint64_t* 
     CUDA_CHECK(cudaMemcpyAsync(out_cap, d_cap, 32ULL << cap_height, cudaMemcpyDeviceToHost, c->stream));
     CUDA_CHECK(cudaMemcpyAsync(&err, c->sync_err.p, 8, cudaMemcpyDeviceToHost, c->stream));
     record(c, GL_N_STAGES);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    read_stages(c, 0, GL_N_STAGES);
     CUDA_CHECK(cudaStreamSynchronize(c->send_stream));                   // (both idle by dependency; the host buffers are only borrowed)
     CUDA_CHECK(cudaStreamSynchronize(c->pull_stream));
-    for (int i = 0; i < GL_N_STAGES; i++) CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
     if (c->trace) {
         std::string line;
         char buf[96];
@@ -1525,15 +1462,13 @@ int gl_dev_merkle(gl_ctx* c, const uint64_t* d_leaves, uint64_t n_leaves, uint32
     if (pitch % 8 || pitch < leaf_len) GL_THROW(GL_ERR_INVALID, "pitch must be a multiple of 8 and >= leaf_len");
     if (!d_digests && n_leaves > (1ULL << cap_height)) GL_THROW(GL_ERR_INVALID, "d_digests is NULL");
     c->scratch.ensure(4ULL << cap_height);
-    for (int i : {GL_STAGE_LEAF_HASH, GL_STAGE_TREE, GL_STAGE_D2H}) { c->launches[i] = 0; c->stage_ms[i] = 0; }
+    reset_stages(c, GL_STAGE_LEAF_HASH, GL_N_STAGES);
     record(c, GL_STAGE_LEAF_HASH);
     merkle_build(c, d_leaves, n_leaves, leaf_len, pitch, cap_height, d_digests, c->scratch.p, &c->launches[GL_STAGE_LEAF_HASH],
                  &c->launches[GL_STAGE_TREE], c->ev[GL_STAGE_TREE]);
     record(c, GL_STAGE_D2H);
     CUDA_CHECK(cudaMemcpyAsync(out_cap, c->scratch.p, 32ULL << cap_height, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    for (int i : {GL_STAGE_LEAF_HASH, GL_STAGE_TREE})
-        CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
+    read_stages(c, GL_STAGE_LEAF_HASH, GL_STAGE_D2H);
     return GL_OK;
     GL_API_END(c)
 }
@@ -1646,7 +1581,6 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
     // Host columns, as many cosets as contexts or more: the STREAMED coset plan (coset_stream_impl) — per wave every context copies and
     // inverse-transforms its column group, the others pull it behind a ticket, each evaluates its own cosets and absorbs the wave into the
     // leaf sponge; the workers never meet between the first and the last barrier.
-    const char* plan_env = getenv("GL_MULTI_PLAN");
     // One context per DEVICE only: a ticket wait parks the items queued behind it, and streams of different contexts on one device can share
     // a hardware queue — the peer's signal could sit behind the very wait it is meant to release.  (With one context per device every
     // device's queues only ever hold that context's own work, enqueued copy -> iNTT + signal -> waits -> compute, so nothing a peer depends on
@@ -1656,10 +1590,8 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
         for (uint32_t q = 0; q < g; q++) distinct_devices = distinct_devices && ctxs[q]->device != ctxs[g]->device;
     // Measured (host columns, 2^20 x 135): 2 devices 2 350 Melem/s streamed against 2 245 with the shipment plan; 8 devices 6 108 against
     // 6 575 — the streamed plan enqueues ~250 launches / copies / events per context and call, and eight worker threads of ONE process push
-    // them through the same driver locks (one process per GPU does not pay that: 7 491).  So it is the default for two contexts only;
-    // GL_MULTI_PLAN=stream forces it, GL_MULTI_PLAN=p2p forbids it.
-    const bool want_stream = plan_env ? !strcmp(plan_env, "stream") : n_ctx <= 2;
-    const bool streamed = G <= (1u << rate_bits) && n_cols > 4 && distinct_devices && want_stream;
+    // them through the same driver locks (one process per GPU does not pay that: 7 491).  So it is the plan for two contexts only.
+    const bool streamed = G <= (1u << rate_bits) && n_cols > 4 && distinct_devices && n_ctx <= 2;
     gl_stream_plan_t sp{};
     sp.n_cols = n_cols; sp.log_n = log_n; sp.rate_bits = rate_bits; sp.cap_height = local_cap_height; sp.n_peers = G;
     sp.group_width = (n_cols >= 4 * 8 * G || G == 1) ? 8 : 4; sp.leaf_pitch = leaf_pitch; sp.epoch = 0;
@@ -1756,14 +1688,13 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
             phase([&] {   // C: hash the own leaf range down to this rank's slice of the cap
                 CUDA_CHECK(cudaSetDevice(c->device));
                 Tree* t = trees[g].get();
-                for (int i : {GL_STAGE_LEAF_HASH, GL_STAGE_TREE, GL_STAGE_D2H}) { c->launches[i] = 0; c->stage_ms[i] = 0; }
+                reset_stages(c, GL_STAGE_LEAF_HASH, GL_N_STAGES);
                 record(c, GL_STAGE_LEAF_HASH);
                 merkle_build(c, t->leaves.p, rows_per_rank, n_cols, leaf_pitch, local_cap_height, t->digests.p, t->d_cap.p,
                              &c->launches[GL_STAGE_LEAF_HASH], &c->launches[GL_STAGE_TREE], c->ev[GL_STAGE_TREE]);
                 record(c, GL_STAGE_D2H);
                 CUDA_CHECK(cudaMemcpyAsync(t->cap.data(), t->d_cap.p, 32ULL << local_cap_height, cudaMemcpyDeviceToHost, c->stream));
-                CUDA_CHECK(cudaStreamSynchronize(c->stream));
-                for (int i : {GL_STAGE_LEAF_HASH, GL_STAGE_TREE}) CUDA_CHECK(cudaEventElapsedTime(&c->stage_ms[i], c->ev[i], c->ev[i + 1]));
+                read_stages(c, GL_STAGE_LEAF_HASH, GL_STAGE_D2H);
             });
         barrier.arrive_and_wait();               // nobody releases a leaf buffer a peer may still be copying into
     };

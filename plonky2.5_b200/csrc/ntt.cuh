@@ -248,45 +248,6 @@ __global__ void ntt_tiny_kernel(const uint64_t* __restrict__ src, uint64_t* __re
     dst[(uint64_t)drow * dst_pitch + col] = acc;
 }
 
-// Multi-GPU exchange as a copy that runs BEHIND the next coset's NTT (separate stream): rows [0, n_rows) of a local
-// [n_rows][src_pitch] coset result go to the owners' leaf buffers (see PassParams::peer); consecutive threads move
-// consecutive words of a row, so every row is one contiguous run of n_cols*8 bytes on the wire.
-__global__ void scatter_copy_kernel(const uint64_t* __restrict__ src, uint32_t src_pitch, uint32_t n_cols, uint64_t n_rows,
-                                    const Scatter sc) {
-    const uint64_t total = n_rows * n_cols;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x) {
-        const uint64_t r = i / n_cols;
-        const uint32_t col = (uint32_t)(i - r * n_cols);
-        const uint64_t grow = sc.row0 + r;
-        uint64_t* base = sc.peer[grow >> sc.log_rows_per_peer];
-        base[(grow & ((1ULL << sc.log_rows_per_peer) - 1)) * sc.pitch + sc.col0 + col] = src[r * src_pitch + col];
-    }
-}
-// 16-byte version (n_vec = words/2 per row; source and destination rows 16-byte aligned), four rows in flight per thread
-__global__ void scatter_copy16_kernel(const ulonglong2* __restrict__ src, uint32_t src_pitch_v, uint32_t n_vec, uint32_t n_rows,
-                                      const Scatter sc) {
-    const uint32_t lane_rows = blockDim.x / n_vec;              // rows covered by one CTA per step (blockDim.x >= n_vec)
-    const uint32_t v = threadIdx.x % n_vec, lr = threadIdx.x / n_vec;
-    if (lr >= lane_rows) return;
-    const uint32_t step = gridDim.x * lane_rows;
-    for (uint32_t r0 = blockIdx.x * lane_rows + lr; r0 < n_rows; r0 += 4 * step) {
-        ulonglong2 x[4];
-#pragma unroll
-        for (int u = 0; u < 4; u++) {
-            const uint32_t r = r0 + u * step;
-            if (r < n_rows) x[u] = src[(size_t)r * src_pitch_v + v];
-        }
-#pragma unroll
-        for (int u = 0; u < 4; u++) {
-            const uint32_t r = r0 + u * step;
-            if (r >= n_rows) continue;
-            const uint64_t grow = sc.row0 + r;
-            ulonglong2* base = reinterpret_cast<ulonglong2*>(sc.peer[grow >> sc.log_rows_per_peer]);
-            base[((grow & ((1ULL << sc.log_rows_per_peer) - 1)) * sc.pitch + sc.col0) / 2 + v] = x[u];
-        }
-    }
-}
-
 // out[j] = g^j (canonical), j < n <= 2^32, from the table g2k[k] = g^(2^k)
 struct PowTable { uint64_t g2k[32]; };
 __global__ void powers_kernel(uint64_t* __restrict__ out, uint64_t n, const PowTable pt) {

@@ -177,7 +177,7 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 // ---- pass structure ------------------------------------------------------------------------------------------------------------------------
 // rounds of a 2^A-point pass: non-final rounds are radix-8 (radix-16 for A = 8) followed by a table twiddle; the final round is the
 // all-shift radix-16 where the stage count allows it
-__host__ __device__ constexpr int plan_n(int A) { return A >= 9 ? 3 : (A >= 5 ? 2 : 1); }   // A = 11: radix-8, then two radix-16 rounds
+__host__ __device__ constexpr int plan_n(int A) { return A >= 9 ? 3 : (A >= 5 ? 2 : 1); }
 __host__ __device__ constexpr int plan_k(int A, int r) {
     switch (A) {
         case 3: return r == 0 ? 3 : 0;
@@ -188,7 +188,6 @@ __host__ __device__ constexpr int plan_k(int A, int r) {
         case 8: return r < 2 ? 4 : 0;
         case 9: return r < 3 ? 3 : 0;
         case 10: return r < 2 ? 3 : (r == 2 ? 4 : 0);
-        case 11: return r == 0 ? 3 : (r < 3 ? 4 : 0);
         default: return 0;
     }
 }

@@ -122,8 +122,8 @@ class ShardedCommit:
 
     exchange="p2p" (default when the ranks can map each other's memory): steps 1 and 2 are one call — gl_dev_lde_scatter /
     gl_lde_scatter deliver every coset's rows into the owners' leaf buffers over NVLink (buffers exported/mapped with CUDA IPC)
-    while the next coset's NTT runs (DESIGN.md §6: copy engines by default, NTT-side remote stores or a copy kernel with
-    GL_SCATTER_MODE), so there is no all-to-all, no receive buffer and no repacking; the ranks only meet at a stream-ordered
+    while the next coset's NTT runs (DESIGN.md §6: the rank's own cosets are stored by the NTT, the others shipped by the copy
+    engines), so there is no all-to-all, no receive buffer and no repacking; the ranks only meet at a stream-ordered
     1-element all-reduce before hashing.  exchange="nccl": gl_dev_lde + all_to_all_single + gl_dev_repack (the baseline the
     fused path is measured against, and the collective fallback when peer mapping is unavailable).
     exchange="coset" (what "auto" picks for device-resident columns when world <= 2^rate_bits): the ranks exchange COEFFICIENT blocks and
