@@ -152,6 +152,14 @@ int gl_openings_add_batch(gl_ctx* ctx, gl_handle openings, const gl_handle* batc
 int gl_openings_final_poly(gl_ctx* ctx, gl_handle openings, uint64_t* out_coeffs_ext /* N*2 words */);
 int gl_openings_lde(gl_ctx* ctx, gl_handle openings, uint32_t rate_bits, uint32_t cap_height, gl_handle* out_fri);
 int gl_openings_end(gl_ctx* ctx, gl_handle openings);
+
+/* ---- OpeningSet::new  (plonky2 plonk/proof.rs; the eval_commitment closure) ----------------------------------
+ * Evaluates every polynomial of a committed batch at n_points extension points [a0, a1] (inputs may be non-canonical):
+ * out_values = [n_points][leaf_len][2] words, canonical; out[p][j] = sum_k coeffs_j[k] * points[p]^k.
+ * 1 <= n_points <= 2 (zeta; zeta and g*zeta for the Z commit).  The coefficient matrix never leaves the device.
+ * A tree without coefficients (gl_merkle_new trees, gl_commit_multi shard trees) is refused with GL_ERR_INVALID.     */
+int gl_batch_eval(gl_ctx* ctx, gl_handle batch, const uint64_t* points_ext, uint32_t n_points, uint64_t* out_values_ext);
+
 /* read the current coefficients (len extension elements) / bit-reversed values of a gl_fri state (tests, debugging) */
 int gl_fri_read(gl_ctx* ctx, gl_handle fri, uint64_t* out_coeffs_ext, uint64_t* out_values_bitrev_ext, uint64_t* out_len);
 

@@ -13,7 +13,8 @@
  *     plonky2 fri/prover.rs          fri_proof, fri_committed_trees, fri_proof_of_work, fri_prover_query_rounds
  *     plonky2 fri/{mod,structure,proof}.rs   FriConfig, FriParams, FriInstanceInfo, FriBatchInfo, FriPolynomialInfo,
  *                                    FriProof, FriQueryRound, FriInitialTreeProof, FriQueryStep
- *     plonky2 iop/challenger.rs      Challenger<GoldilocksField, PoseidonHash>
+ *     plonky2 iop/challenger.rs      Challenger<GoldilocksField, PoseidonHash>, observe_openings
+ *     plonky2 plonk/proof.rs         OpeningSet::{new, to_fri_openings};  fri/structure.rs  FriOpenings, FriOpeningBatch
  *
  * (`new` is a C++ keyword: MerkleTree::new_.)  Upstream functions are infallible and `assert!`-panic on misuse; here a
  * violated upstream assert throws plonky2::Panic carrying the upstream message, any other failure (no CUDA device,
@@ -81,6 +82,10 @@ struct MerkleCap {
 };
 
 struct MerkleProof { std::vector<HashOut> siblings; size_t len() const { return siblings.size(); } };
+
+/* plonky2 fri/structure.rs · FriOpeningBatch { values }, FriOpenings { batches } */
+struct FriOpeningBatch { std::vector<Ext> values; };
+struct FriOpenings { std::vector<FriOpeningBatch> batches; };
 
 /* ------------------------------------------------------------------------------------------------ Context */
 /* One CUDA device + stream + cached twiddle tables (gl_ctx).  Calls on one Context are serialised by the library;
@@ -280,6 +285,11 @@ public:
     void observe_cap(const MerkleCap& cap) { for (const auto& h : cap.hashes) observe_hash(h); }
     void observe_extension_element(const Ext& e) { observe_elements(e.data(), 2); }
     void observe_extension_elements(const std::vector<Ext>& es) { for (const auto& e : es) observe_extension_element(e); }
+    /* every batch's values, in order (upstream: challenger.observe_openings(&openings.to_fri_openings())) */
+    void observe_openings(const FriOpenings& openings) {
+        for (const auto& b : openings.batches)
+            if (!b.values.empty()) observe_elements(b.values[0].data(), 2 * b.values.size());
+    }
 
     F get_challenge() {
         if (!input_buffer.empty() || output_buffer.empty()) duplexing();
@@ -671,6 +681,56 @@ public:
     }
 };
 
+/* ------------------------------------------------------------------------------------------------ OpeningSet */
+/* OpeningSet::new's eval_commitment closure on the device (gl_batch_eval): every polynomial of `batch` at each of 1 or 2 extension
+ * points; out[p][j] = polynomials[j].to_extension().eval(points[p]).  The coefficients stay in HBM. */
+inline std::vector<std::vector<Ext>> eval_commitment(const PolynomialBatch& batch, const std::vector<Ext>& points) {
+    Context& c = batch.merkle_tree.context();
+    const size_t n = batch.num_polys();
+    std::vector<Ext> flat(points.size() * n);
+    c.check(gl_batch_eval(c.raw(), batch.merkle_tree.handle(), points.empty() ? nullptr : points[0].data(), uint32_t(points.size()),
+                          flat.empty() ? nullptr : flat[0].data()));
+    std::vector<std::vector<Ext>> out(points.size());
+    for (size_t p = 0; p < points.size(); p++) out[p].assign(flat.begin() + p * n, flat.begin() + (p + 1) * n);
+    return out;
+}
+
+/* plonky2 plonk/proof.rs · OpeningSet, without lookups (the reference's circuits use none) */
+struct OpeningSet {
+    std::vector<Ext> constants, plonk_sigmas, wires, plonk_zs, plonk_zs_next, partial_products, quotient_polys;
+
+    /* OpeningSet::new(zeta, g, constants_sigmas, wires, zs_partial_products, quotient, common_data): four device calls, the Z commit at
+     * zeta and g * zeta in one.  Commit #0 holds the constants first; commit #2 the Z polynomial of every challenge first
+     * (gl_partial_products' order), then the partial products. */
+    static OpeningSet new_(const Ext& zeta, const Ext& g, const PolynomialBatch& constants_sigmas, const PolynomialBatch& wires,
+                           const PolynomialBatch& zs_partial_products, const PolynomialBatch& quotient, size_t num_constants,
+                           size_t num_challenges) {
+        if (num_constants > constants_sigmas.num_polys() || num_challenges > zs_partial_products.num_polys())
+            throw Panic("OpeningSet::new: num_constants / num_challenges exceed the width of their commit");
+        auto mul = [](uint64_t a, uint64_t b) { return uint64_t((unsigned __int128)(a % ORDER) * (b % ORDER) % ORDER); };
+        auto add = [](uint64_t a, uint64_t b) { return uint64_t(((unsigned __int128)a + b) % ORDER); };
+        const Ext gz = {add(mul(g[0], zeta[0]), mul(7, mul(g[1], zeta[1]))), add(mul(g[0], zeta[1]), mul(g[1], zeta[0]))};
+        const auto cs = eval_commitment(constants_sigmas, {zeta})[0];
+        const auto zs = eval_commitment(zs_partial_products, {zeta, gz});
+        OpeningSet o;
+        o.constants.assign(cs.begin(), cs.begin() + num_constants);
+        o.plonk_sigmas.assign(cs.begin() + num_constants, cs.end());
+        o.wires = eval_commitment(wires, {zeta})[0];
+        o.plonk_zs.assign(zs[0].begin(), zs[0].begin() + num_challenges);
+        o.plonk_zs_next.assign(zs[1].begin(), zs[1].begin() + num_challenges);
+        o.partial_products.assign(zs[0].begin() + num_challenges, zs[0].end());
+        o.quotient_polys = eval_commitment(quotient, {zeta})[0];
+        return o;
+    }
+
+    /* the zeta batch (constants, sigmas, wires, zs, partial products, quotient) and the g * zeta batch (zs_next) */
+    FriOpenings to_fri_openings() const {
+        FriOpeningBatch at_zeta;
+        for (const auto* v : {&constants, &plonk_sigmas, &wires, &plonk_zs, &partial_products, &quotient_polys})
+            at_zeta.values.insert(at_zeta.values.end(), v->begin(), v->end());
+        return FriOpenings{{std::move(at_zeta), FriOpeningBatch{plonk_zs_next}}};
+    }
+};
 
 /* ------------------------------------------------------------------------------------------------ quotient / permutation / witness */
 /* SURVEY §8(f) ranks 3-4.  Gate kinds are include/gl_commit.h's GL_GATE_* (the reference's own gates: Poseidon2Gate and the eight

@@ -7,12 +7,12 @@ repository root) or via importlib.
 """
 from . import _lib  # noqa: F401
 from . import sharded  # noqa: F401
-from .api import (Challenger, Context, FriBatchInfo, FriParams, FriProofHead, GlError, MerkleCap, MerkleTree,  # noqa: F401
-                  PolynomialBatch, commit_multi, default_context, fri_committed_trees, fri_proof_of_work, fri_prover_query_rounds, prove_openings, reduction_arity_bits)
+from .api import (Challenger, Context, FriBatchInfo, FriOpeningBatch, FriOpenings, FriParams, FriProofHead, GlError, MerkleCap,  # noqa: F401
+                  MerkleTree, OpeningSet, PolynomialBatch, commit_multi, eval_commitment, default_context, fri_committed_trees, fri_proof_of_work, fri_prover_query_rounds, prove_openings, reduction_arity_bits)
 from .api import (GATE_COMPARISON, GATE_POSEIDON2, GATE_U32_ADD_MANY, GATE_U32_ARITHMETIC, GATE_U32_INTERLEAVE, GATE_U32_RANGE_CHECK,  # noqa: F401
                   GATE_U32_SUBTRACTION, GATE_UNINTERLEAVE_TO_B32, GATE_UNINTERLEAVE_TO_U32, Quotient, evaluate_gate_constraints, gate_shape,
                   partial_products_and_zs, poseidon2_gate_witness)
 from .build import build  # noqa: F401
 
-__all__ = ["Challenger", "Context", "FriBatchInfo", "FriParams", "FriProofHead", "GlError", "MerkleCap", "MerkleTree",
-           "PolynomialBatch", "commit_multi", "default_context", "fri_committed_trees", "fri_proof_of_work", "fri_prover_query_rounds", "prove_openings", "reduction_arity_bits", "build"]
+__all__ = ["Challenger", "Context", "FriBatchInfo", "FriOpeningBatch", "FriOpenings", "FriParams", "FriProofHead", "GlError", "MerkleCap",
+           "MerkleTree", "OpeningSet", "PolynomialBatch", "commit_multi", "eval_commitment", "default_context", "fri_committed_trees", "fri_proof_of_work", "fri_prover_query_rounds", "prove_openings", "reduction_arity_bits", "build"]

@@ -61,6 +61,7 @@ SIGNATURES = {
     "gl_openings_final_poly": (c_int, [c_void_p, c_uint64, c_void_p]),
     "gl_openings_lde": (c_int, [c_void_p, c_uint64, c_uint32, c_uint32, POINTER(c_uint64)]),
     "gl_openings_end": (c_int, [c_void_p, c_uint64]),
+    "gl_batch_eval": (c_int, [c_void_p, c_uint64, c_void_p, c_uint32, c_void_p]),
     "gl_fri_read": (c_int, [c_void_p, c_uint64, c_void_p, c_void_p, POINTER(c_uint64)]),
     "gl_gate_num_wires": (c_int, [c_int, c_uint32]),
     "gl_gate_num_constraints": (c_int, [c_int, c_uint32]),

@@ -343,6 +343,11 @@ class Challenger:
     def observe_extension_elements(self, es):
         self.observe_elements(es)
 
+    def observe_openings(self, fri_openings: "FriOpenings"):
+        """every batch's values, in order, as extension elements (upstream: observe_openings(&openings.to_fri_openings()))"""
+        for batch in fri_openings.batches:
+            self.observe_extension_elements(batch.values)
+
     def get_challenge(self) -> int:
         if self.input_buffer or not self.output_buffer:
             self._duplexing()
@@ -453,6 +458,62 @@ class FriBatchInfo:
     def __init__(self, point: Tuple[int, int], polynomials: Sequence[Tuple[int, int]]):
         self.point = (int(point[0]), int(point[1]))
         self.polynomials = [(int(o), int(i)) for (o, i) in polynomials]
+
+
+def eval_commitment(batch: "PolynomialBatch", points) -> np.ndarray:
+    """OpeningSet::new's eval_commitment closure: every polynomial of `batch` at each of 1 or 2 extension points (a0, a1), on the
+    device (gl_batch_eval); the coefficients stay in HBM.  Returns [n_points][num_polys][2] canonical words."""
+    pts = np.array([[int(p[0]), int(p[1])] for p in points], dtype=np.uint64)
+    t = batch.merkle_tree
+    out = np.zeros((len(pts), t.leaf_len, 2), dtype=np.uint64)
+    _check(batch.ctx, batch.ctx.lib.gl_batch_eval(batch.ctx.handle, t._h, _ptr(pts) if pts.size else None, len(pts), _ptr(out)))
+    return out
+
+
+class FriOpeningBatch:
+    """plonky2 fri/structure.rs · FriOpeningBatch { values: Vec<F::Extension> } — [n][2] words"""
+
+    def __init__(self, values):
+        self.values = np.ascontiguousarray(values, dtype=np.uint64).reshape(-1, 2)
+
+
+class FriOpenings:
+    """plonky2 fri/structure.rs · FriOpenings { batches: Vec<FriOpeningBatch> }"""
+
+    def __init__(self, batches: Sequence[FriOpeningBatch]):
+        self.batches = list(batches)
+
+
+class OpeningSet:
+    """plonky2 plonk/proof.rs · OpeningSet without lookups (the reference's circuits use none); every field is [n][2] words."""
+
+    def __init__(self, constants, plonk_sigmas, wires, plonk_zs, plonk_zs_next, partial_products, quotient_polys):
+        self.constants, self.plonk_sigmas, self.wires = constants, plonk_sigmas, wires
+        self.plonk_zs, self.plonk_zs_next, self.partial_products = plonk_zs, plonk_zs_next, partial_products
+        self.quotient_polys = quotient_polys
+
+    @classmethod
+    def new(cls, zeta, g, constants_sigmas: "PolynomialBatch", wires: "PolynomialBatch", zs_partial_products: "PolynomialBatch",
+            quotient: "PolynomialBatch", num_constants: int, num_challenges: int) -> "OpeningSet":
+        """OpeningSet::new: the four commits at zeta, the Z/partial-products commit also at g * zeta (one device call for both points).
+        Commit #0 holds the constants first, then the sigmas; commit #2 the Z polynomial of every challenge first (gl_partial_products'
+        order), then the partial products.  g: the subgroup generator, a base element or an extension element (a0, a1)."""
+        z = (int(zeta[0]) % P, int(zeta[1]) % P)
+        g0, g1 = (int(g), 0) if np.isscalar(g) else (int(g[0]), int(g[1]))
+        gz = ((g0 * z[0] + 7 * g1 * z[1]) % P, (g0 * z[1] + g1 * z[0]) % P)
+        if num_constants > constants_sigmas.merkle_tree.leaf_len or num_challenges > zs_partial_products.merkle_tree.leaf_len:
+            raise ValueError("num_constants / num_challenges exceed the width of their commit")
+        cs = eval_commitment(constants_sigmas, [z])[0]
+        zs = eval_commitment(zs_partial_products, [z, gz])
+        return cls(constants=cs[:num_constants], plonk_sigmas=cs[num_constants:], wires=eval_commitment(wires, [z])[0],
+                   plonk_zs=zs[0][:num_challenges], plonk_zs_next=zs[1][:num_challenges], partial_products=zs[0][num_challenges:],
+                   quotient_polys=eval_commitment(quotient, [z])[0])
+
+    def to_fri_openings(self) -> FriOpenings:
+        """the zeta batch (constants, sigmas, wires, zs, partial products, quotient) and the g * zeta batch (zs_next)"""
+        zeta_batch = np.concatenate([self.constants, self.plonk_sigmas, self.wires, self.plonk_zs, self.partial_products,
+                                     self.quotient_polys])
+        return FriOpenings([FriOpeningBatch(zeta_batch), FriOpeningBatch(self.plonk_zs_next)])
 
 
 class FriProofHead:

@@ -2109,6 +2109,51 @@ int gl_openings_end(gl_ctx* c, gl_handle oh) {
     GL_API_END(c)
 }
 
+// ------------------------------------------------------------------------------------------------ OpeningSet::new
+int gl_batch_eval(gl_ctx* c, gl_handle batch, const uint64_t* points_ext, uint32_t n_points, uint64_t* out_values_ext) {
+    GL_API_BEGIN(c)
+    Tree* t = find_tree(c, batch);
+    if (!t->has_coeffs) GL_THROW(GL_ERR_INVALID, "tree has no coefficients");
+    if (!points_ext || !out_values_ext) GL_THROW(GL_ERR_INVALID, "NULL pointer");
+    if (n_points == 0) GL_THROW(GL_ERR_INVALID, "n_points must be at least 1");
+    if (n_points > 2) GL_THROW(GL_ERR_UNSUPPORTED, "n_points = %u > 2", n_points);
+    openings::EvalPoints pts{};
+    for (uint32_t p = 0; p < n_points; p++) {
+        HExt z = {gl::canon(points_ext[2 * p]), gl::canon(points_ext[2 * p + 1])};
+        for (uint32_t b = 0; b < 32; b++) {
+            pts.z2k[p][b][0] = z.a0; pts.z2k[p][b][1] = z.a1;
+            z = h_ext_mul(z, z);
+        }
+    }
+    const uint64_t N = 1ULL << t->degree_log;
+    const uint32_t sub_rows = (uint32_t)std::min<uint64_t>(N, openings::EVAL_SUB);
+    const uint32_t col_tiles = (t->leaf_len + openings::EVAL_THREADS - 1) / openings::EVAL_THREADS;
+    const uint32_t wc = (t->leaf_len + col_tiles - 1) / col_tiles;
+    const uint32_t lanes = std::min(openings::EVAL_THREADS / wc, sub_rows);
+    const uint32_t threads = round_up(lanes * wc, 32);
+    uint32_t n_parts = (uint32_t)(N / sub_rows);   // row CTAs: a power of two, at most EVAL_MAX_PARTS / col_tiles
+    while (n_parts > 1 && n_parts * col_tiles > openings::EVAL_MAX_PARTS) n_parts >>= 1;
+    const uint32_t subs = (uint32_t)(N / sub_rows / n_parts);
+    const uint32_t n_out = n_points * t->leaf_len;
+    c->scratch.ensure(2 * (size_t)n_out * (n_parts + 1));
+    ulonglong2* partial = reinterpret_cast<ulonglong2*>(c->scratch.p);
+    ulonglong2* d_out = partial + (size_t)n_out * n_parts;
+    const dim3 grid(n_parts, col_tiles);
+    if (n_points == 1)
+        openings::batch_eval_partial_kernel<1><<<grid, threads, 0, c->stream>>>(t->coeffs.p, t->pitch, t->leaf_len, wc, lanes, sub_rows, subs,
+                                                                                 pts, partial);
+    else
+        openings::batch_eval_partial_kernel<2><<<grid, threads, 0, c->stream>>>(t->coeffs.p, t->pitch, t->leaf_len, wc, lanes, sub_rows, subs,
+                                                                                 pts, partial);
+    CUDA_CHECK(cudaGetLastError());
+    openings::batch_eval_reduce_kernel<<<(n_out + 31) / 32, dim3(32, 32), 0, c->stream>>>(partial, n_parts, n_out, d_out);
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaMemcpyAsync(out_values_ext, d_out, 16 * (size_t)n_out, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    return GL_OK;
+    GL_API_END(c)
+}
+
 int gl_fri_read(gl_ctx* c, gl_handle fh, uint64_t* out_coeffs, uint64_t* out_values, uint64_t* out_len) {
     GL_API_BEGIN(c)
     Fri* f = find_fri(c, fh);

@@ -374,6 +374,16 @@ impl<'c> DeviceTree<'c> {
     pub fn digests(&self) -> Result<Vec<u64>, Error> {
         self.read(ffi::GL_PART_DIGESTS, 8 * (self.info.n_leaves as usize - (1usize << self.info.cap_height)))
     }
+    /// `OpeningSet::new`'s `eval_commitment`: every polynomial of the batch at each of 1 or 2 extension points,
+    /// `out[p][j] = polynomials[j].to_extension().eval(points[p])`; the coefficients stay on the device
+    pub fn eval_at(&self, points: &[Ext]) -> Result<Vec<Vec<Ext>>, Error> {
+        let ll = self.info.leaf_len as usize;
+        let mut out = vec![[0u64; 2]; points.len() * ll];
+        let pp = if points.is_empty() { ptr::null() } else { points.as_ptr() as *const u64 };
+        let op = if out.is_empty() { ptr::null_mut() } else { out.as_mut_ptr() as *mut u64 };
+        self.ctx.check(unsafe { ffi::gl_batch_eval(self.ctx.raw, self.handle, pp, points.len() as u32, op) })?;
+        Ok(out.chunks(ll.max(1)).map(|c| c.to_vec()).collect())
+    }
 }
 
 impl Drop for DeviceTree<'_> {
