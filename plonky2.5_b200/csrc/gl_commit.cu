@@ -167,6 +167,14 @@ struct Tree {
     DevBuf leaves, digests, coeffs, d_cap;
     bool has_coeffs = false;
     std::vector<uint64_t> cap;
+    // leaves [n_leaves][pitch], digests, cap on the device and on the host; the coefficients are the caller's
+    Tree(uint64_t n_leaves_, uint32_t leaf_len_, uint32_t pitch_, uint32_t cap_height_)
+        : n_leaves(n_leaves_), leaf_len(leaf_len_), pitch(pitch_), cap_height(cap_height_), cap(4ULL << cap_height_) {
+        leaves.ensure(n_leaves * pitch);
+        digests.ensure(n_digests() * 4);
+        d_cap.ensure(4ULL << cap_height);
+    }
+    uint64_t n_digests() const { return 2 * (n_leaves - (1ULL << cap_height)); }
 };
 
 struct Fri {
@@ -175,6 +183,9 @@ struct Fri {
     uint64_t shift = gl::COSET_SHIFT;
     uint32_t last_arity_bits = 0;
     DevBuf coeffs, values, tmp;   // values are kept in bit-reversed order (what the next layer's leaves need)
+    Fri(uint64_t len_, uint32_t rate_bits_, uint32_t cap_height_) : len(len_), rate_bits(rate_bits_), cap_height(cap_height_) {
+        coeffs.ensure(2 * len); values.ensure(2 * len); tmp.ensure(2 * len);
+    }
 };
 
 struct Quotient {
@@ -187,6 +198,17 @@ struct Quotient {
 struct Openings {
     uint32_t log_n = 0;
     DevBuf final_poly, comp, refs, pw;   // final_poly / composition: N extension elements each
+};
+
+// The objects of one kind a context hands out.  All kinds draw their handles from the context's one counter, so a handle of one kind is
+// never valid as another.
+template <class T>
+struct Handles {
+    const char* kind;   // in "unknown <kind> handle"
+    std::map<gl_handle, std::unique_ptr<T>> live;
+    gl_handle put(gl_ctx* c, std::unique_ptr<T> obj);
+    T* get(gl_handle h) const;
+    void drop(gl_ctx* c, gl_handle h);   // waits for the context's stream: enqueued work may still use the object's buffers
 };
 
 }  // namespace
@@ -202,10 +224,10 @@ struct gl_ctx {
     std::map<std::pair<uint64_t, uint32_t>, std::unique_ptr<CosetTable>> coset_cache;   // (shift, log_len) -> g^j: FRI layers / final-poly LDE
     size_t coset_cache_words = 0;
     DevBuf in_stage, vals, scratch, hash_state;
-    std::map<gl_handle, std::unique_ptr<Tree>> trees;
-    std::map<gl_handle, std::unique_ptr<Fri>> fris;
-    std::map<gl_handle, std::unique_ptr<Openings>> openings;
-    std::map<gl_handle, std::unique_ptr<Quotient>> quotients;
+    Handles<Tree> trees{"tree"};
+    Handles<Fri> fris{"fri"};
+    Handles<Openings> openings{"openings"};
+    Handles<Quotient> quotients{"quotient"};
     float aux_ms = 0;
     gl_handle next_handle = 1;
     cudaStream_t copy_stream = nullptr;   // host->device column copies of gl_commit, overlapped with the NTTs
@@ -232,6 +254,25 @@ struct gl_ctx {
 };
 
 namespace {
+
+template <class T>
+gl_handle Handles<T>::put(gl_ctx* c, std::unique_ptr<T> obj) {
+    const gl_handle h = c->next_handle++;
+    live[h] = std::move(obj);
+    return h;
+}
+template <class T>
+T* Handles<T>::get(gl_handle h) const {
+    auto it = live.find(h);
+    if (it == live.end()) GL_THROW(GL_ERR_HANDLE, "unknown %s handle %llu", kind, (unsigned long long)h);
+    return it->second.get();
+}
+template <class T>
+void Handles<T>::drop(gl_ctx* c, gl_handle h) {
+    get(h);
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    live.erase(h);
+}
 
 const uint64_t* get_roots(gl_ctx* c, uint32_t log_n) {
     auto it = c->roots.find(log_n);
@@ -554,20 +595,19 @@ void check_shape(uint32_t n_cols, uint32_t log_n, uint32_t rate_bits, uint32_t c
                  cap_height, log_n + rate_bits);
 }
 
-gl_handle put_tree(gl_ctx* c, std::unique_ptr<Tree> t) {
-    gl_handle h = c->next_handle++;
-    c->trees[h] = std::move(t);
-    return h;
+// The end of a tree built on the compute stream: digests (if asked for) and cap to the host, and a handle (if asked for)
+void finish_tree(gl_ctx* c, std::unique_ptr<Tree> t, uint64_t* out_digests, uint64_t* out_cap, gl_handle* out_tree) {
+    CUDA_CHECK(cudaMemcpyAsync(t->cap.data(), t->d_cap.p, t->cap.size() * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (out_digests && t->n_digests())
+        CUDA_CHECK(cudaMemcpyAsync(out_digests, t->digests.p, t->n_digests() * 32, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    memcpy(out_cap, t->cap.data(), t->cap.size() * 8);
+    if (out_tree) *out_tree = c->trees.put(c, std::move(t));
 }
-Tree* find_tree(gl_ctx* c, gl_handle h) {
-    auto it = c->trees.find(h);
-    if (it == c->trees.end()) GL_THROW(GL_ERR_HANDLE, "unknown tree handle %llu", (unsigned long long)h);
-    return it->second.get();
-}
-Fri* find_fri(gl_ctx* c, gl_handle h) {
-    auto it = c->fris.find(h);
-    if (it == c->fris.end()) GL_THROW(GL_ERR_HANDLE, "unknown fri handle %llu", (unsigned long long)h);
-    return it->second.get();
+
+void copy_row(gl_ctx* c, const Tree* t, uint64_t row, uint64_t* out_row) {
+    CUDA_CHECK(cudaMemcpyAsync(out_row, t->leaves.p + row * t->pitch, (size_t)t->leaf_len * 8, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));
 }
 
 void record(gl_ctx* c, int i) { CUDA_CHECK(cudaEventRecord(c->ev[i], c->stream)); }
@@ -725,18 +765,12 @@ int commit_impl(gl_ctx* c, const uint64_t* const* host_cols, const uint64_t* d_c
     if (!out_cap) GL_THROW(GL_ERR_INVALID, "out_cap is NULL");
     const uint64_t N = 1ULL << log_n, R = N << rate_bits;
     const uint32_t pitch = round_up(n_cols, 8);
-    const uint64_t n_dig = 2 * (R - (1ULL << cap_height));
     // warm the tables before the timed region starts
     get_roots(c, log_n);
     get_lde_tables(c, log_n, rate_bits);
-    auto t = std::make_unique<Tree>();
-    t->n_leaves = R; t->leaf_len = n_cols; t->pitch = pitch; t->cap_height = cap_height;
+    auto t = std::make_unique<Tree>(R, n_cols, pitch, cap_height);
     t->degree_log = log_n; t->rate_bits = rate_bits; t->has_coeffs = true;
     t->coeffs.ensure(N * pitch);
-    t->leaves.ensure(R * pitch);
-    t->digests.ensure(n_dig * 4);
-    t->d_cap.ensure(4ULL << cap_height);
-    t->cap.resize(4ULL << cap_height);
     reset_stages(c, 0, GL_N_STAGES);
 
     record(c, GL_STAGE_H2D);
@@ -795,14 +829,37 @@ int commit_impl(gl_ctx* c, const uint64_t* const* host_cols, const uint64_t* d_c
         CUDA_CHECK(cudaEventRecord(c->ev_copyback, c->copy_stream));
     }
     CUDA_CHECK(cudaMemcpyAsync(t->cap.data(), t->d_cap.p, (32ULL << cap_height), cudaMemcpyDeviceToHost, c->stream));
-    if (out_digests && n_dig)
-        CUDA_CHECK(cudaMemcpyAsync(out_digests, t->digests.p, n_dig * 32, cudaMemcpyDeviceToHost, c->stream));
+    if (out_digests && t->n_digests())
+        CUDA_CHECK(cudaMemcpyAsync(out_digests, t->digests.p, t->n_digests() * 32, cudaMemcpyDeviceToHost, c->stream));
     if (early_copyback) CUDA_CHECK(cudaStreamWaitEvent(c->stream, c->ev_copyback, 0));   // the d2h stage ends when everything has landed
     record(c, GL_N_STAGES);
     read_stages(c, 0, GL_N_STAGES);
     memcpy(out_cap, t->cap.data(), 32ULL << cap_height);
-    if (out_batch) *out_batch = put_tree(c, std::move(t));
+    if (out_batch) *out_batch = c->trees.put(c, std::move(t));
     return GL_OK;
+}
+
+// why the last failed call on `c` failed, for gl_ctx_last_error
+int set_error(gl_ctx* c, int code, const std::string& msg) {
+    c->err = msg;
+    return code;
+}
+
+// Turns the exception being handled into the return code of a call on `c`.  Call it only from a catch block, with c->mu held.
+int fail(gl_ctx* c) {
+    try {
+        throw;
+    } catch (const GlError& e) {
+        cudaGetLastError();
+        // host buffers are only borrowed: nothing may read or write them after the call returns
+        for (cudaStream_t s : {c->stream, c->copy_stream, c->send_stream, c->pull_stream})
+            if (s) cudaStreamSynchronize(s);
+        return set_error(c, e.code, e.msg);
+    } catch (const std::bad_alloc&) {
+        return set_error(c, GL_ERR_OOM, "host allocation failed");
+    } catch (...) {
+        return set_error(c, GL_ERR_CUDA, "unknown error");
+    }
 }
 
 }  // namespace
@@ -815,22 +872,8 @@ int commit_impl(gl_ctx* c, const uint64_t* const* host_cols, const uint64_t* d_c
         CUDA_CHECK(cudaSetDevice((ctx)->device));
 #define GL_API_END(ctx)                          \
     }                                            \
-    catch (const GlError& e) {                   \
-        (ctx)->err = e.msg;                      \
-        cudaGetLastError();                      \
-        if ((ctx)->stream) cudaStreamSynchronize((ctx)->stream);           /* host buffers are only borrowed: nothing may */ \
-        if ((ctx)->copy_stream) cudaStreamSynchronize((ctx)->copy_stream); /* read or write them after the call returns  */ \
-        if ((ctx)->send_stream) cudaStreamSynchronize((ctx)->send_stream);                                      \
-        if ((ctx)->pull_stream) cudaStreamSynchronize((ctx)->pull_stream);                                      \
-        return e.code;                           \
-    }                                            \
-    catch (const std::bad_alloc&) {              \
-        (ctx)->err = "host allocation failed";   \
-        return GL_ERR_OOM;                       \
-    }                                            \
     catch (...) {                                \
-        (ctx)->err = "unknown error";            \
-        return GL_ERR_CUDA;                      \
+        return fail(ctx);                        \
     }
 
 extern "C" {
@@ -865,22 +908,23 @@ int gl_ctx_create(gl_ctx** out, int device) {
     gl_ctx* c = new (std::nothrow) gl_ctx;
     if (!c) return GL_ERR_OOM;
     c->device = device;
-    if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
-    if (cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
+    auto cuda_failed = [c] { delete c; return GL_ERR_CUDA; };
+    if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) return cuda_failed();
+    if (cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) != cudaSuccess) return cuda_failed();
     {
         int lo = 0, hi = 0;   // the streamed coset plan's few iNTT CTAs must get SM slots as hashing CTAs retire, not queue behind a whole grid
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        if (cudaStreamCreateWithPriority(&c->send_stream, cudaStreamNonBlocking, hi) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
+        if (cudaStreamCreateWithPriority(&c->send_stream, cudaStreamNonBlocking, hi) != cudaSuccess) return cuda_failed();
     }
     for (int i = 0; i < 2; i++)
         if (cudaEventCreateWithFlags(&c->ev_ntt[i], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&c->ev_sent[i], cudaEventDisableTiming) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
-    if (cudaStreamCreateWithFlags(&c->pull_stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
+            cudaEventCreateWithFlags(&c->ev_sent[i], cudaEventDisableTiming) != cudaSuccess) return cuda_failed();
+    if (cudaStreamCreateWithFlags(&c->pull_stream, cudaStreamNonBlocking) != cudaSuccess) return cuda_failed();
     if (const char* m = getenv("GL_TRACE")) c->trace = atoi(m) != 0;
-    if (cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
-    if (cudaEventCreateWithFlags(&c->ev_copyback, cudaEventDisableTiming) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
+    if (cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming) != cudaSuccess) return cuda_failed();
+    if (cudaEventCreateWithFlags(&c->ev_copyback, cudaEventDisableTiming) != cudaSuccess) return cuda_failed();
     for (auto& e : c->ev)
-        if (cudaEventCreate(&e) != cudaSuccess) { delete c; return GL_ERR_CUDA; }
+        if (cudaEventCreate(&e) != cudaSuccess) return cuda_failed();
     cudaDeviceGetAttribute(&c->sm_count, cudaDevAttrMultiProcessorCount, device);
     *out = c;
     return GL_OK;
@@ -890,10 +934,10 @@ void gl_ctx_destroy(gl_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    c->trees.clear();
-    c->fris.clear();
-    c->openings.clear();
-    c->quotients.clear();
+    c->trees.live.clear();
+    c->fris.live.clear();
+    c->openings.live.clear();
+    c->quotients.live.clear();
     c->roots.clear();
     c->pass_roots.clear();
     c->lde_tables.clear();
@@ -1482,14 +1526,8 @@ int gl_merkle_new(gl_ctx* c, const uint64_t* leaves, uint64_t n_leaves, uint32_t
     if ((1ULL << cap_height) > n_leaves)
         GL_THROW(GL_ERR_INVALID, "cap_height should be at most log2(leaves.len()) (cap_height=%u, leaves=%llu)", cap_height,
                  (unsigned long long)n_leaves);
-    auto t = std::make_unique<Tree>();
     const uint32_t pitch = round_up(leaf_len ? leaf_len : 1, 8);
-    const uint64_t n_dig = 2 * (n_leaves - (1ULL << cap_height));
-    t->n_leaves = n_leaves; t->leaf_len = leaf_len; t->pitch = pitch; t->cap_height = cap_height;
-    t->leaves.ensure(n_leaves * pitch);
-    t->digests.ensure(n_dig * 4);
-    t->d_cap.ensure(4ULL << cap_height);
-    t->cap.resize(4ULL << cap_height);
+    auto t = std::make_unique<Tree>(n_leaves, leaf_len, pitch, cap_height);
     if (leaf_len) {
         // packed host rows -> staging -> [n_leaves][pitch] with every word canonicalised (inputs may be any 64-bit representative;
         // everything gl_tree_get / open_batch / read hands back is canonical, like every other ingest path)
@@ -1501,12 +1539,7 @@ int gl_merkle_new(gl_ctx* c, const uint64_t* leaves, uint64_t n_leaves, uint32_t
         CUDA_CHECK(cudaGetLastError());
     }
     merkle_build(c, t->leaves.p, n_leaves, leaf_len, pitch, cap_height, t->digests.p, t->d_cap.p, nullptr, nullptr, nullptr);
-    CUDA_CHECK(cudaMemcpyAsync(t->cap.data(), t->d_cap.p, 32ULL << cap_height, cudaMemcpyDeviceToHost, c->stream));
-    if (out_digests && n_dig)
-        CUDA_CHECK(cudaMemcpyAsync(out_digests, t->digests.p, n_dig * 32, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    memcpy(out_cap, t->cap.data(), 32ULL << cap_height);
-    if (out_tree) *out_tree = put_tree(c, std::move(t));
+    finish_tree(c, std::move(t), out_digests, out_cap, out_tree);
     return GL_OK;
     GL_API_END(c)
 }
@@ -1559,7 +1592,7 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
                     uint32_t cap_height, int input_is_coeffs, uint64_t* out_cap, gl_handle* out_trees) {
     if (!ctxs || n_ctx == 0 || !ctxs[0]) return GL_ERR_INVALID;
     gl_ctx* c0 = ctxs[0];
-    auto fail0 = [&](int code, const char* msg) { std::lock_guard<std::mutex> lk(c0->mu); c0->err = msg; return code; };
+    auto fail0 = [&](int code, const std::string& msg) { std::lock_guard<std::mutex> lk(c0->mu); return set_error(c0, code, msg); };
     if ((n_ctx & (n_ctx - 1)) || n_ctx > (uint32_t)ntt::MAX_PEERS) return fail0(GL_ERR_INVALID, "n_ctx must be a power of two <= 16");
     for (uint32_t g = 0; g < n_ctx; g++) {
         if (!ctxs[g]) return fail0(GL_ERR_INVALID, "NULL context");
@@ -1612,26 +1645,13 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
             if (rcs[g] != GL_OK) return;
             try {
                 body();
-            } catch (const GlError& e) {
-                c->err = e.msg;
-                cudaGetLastError();
-                if (c->stream) cudaStreamSynchronize(c->stream);
-                if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
-                if (c->send_stream) cudaStreamSynchronize(c->send_stream);
-                rcs[g] = e.code;
-            } catch (const std::bad_alloc&) {
-                c->err = "host allocation failed";
-                rcs[g] = GL_ERR_OOM;
+            } catch (...) {
+                rcs[g] = fail(c);
             }
         };
         phase([&] {   // A: this rank's leaf range, digests and sub-cap; peers become addressable
             CUDA_CHECK(cudaSetDevice(c->device));
-            auto t = std::make_unique<Tree>();
-            t->n_leaves = rows_per_rank; t->leaf_len = n_cols; t->pitch = leaf_pitch; t->cap_height = local_cap_height;
-            t->leaves.ensure(rows_per_rank * leaf_pitch);
-            t->digests.ensure(2 * (rows_per_rank - (1ULL << local_cap_height)) * 4);
-            t->d_cap.ensure(4ULL << local_cap_height);
-            t->cap.resize(4ULL << local_cap_height);
+            auto t = std::make_unique<Tree>(rows_per_rank, n_cols, leaf_pitch, local_cap_height);
             if (streamed) {
                 preload_stream_kernels();            // before the barrier: no context may load a kernel once any device parks a ticket wait
                 get_roots(c, log_n);
@@ -1737,7 +1757,7 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
         }
         if (rcs[0] == GL_OK) {   // report through the first context what a peer said
             for (uint32_t g = 1; g < G; g++)
-                if (rcs[g] != GL_OK) { std::string m; { std::lock_guard<std::mutex> lk(ctxs[g]->mu); m = ctxs[g]->err; } fail0(rcs[g], m.c_str()); break; }
+                if (rcs[g] != GL_OK) { std::string m; { std::lock_guard<std::mutex> lk(ctxs[g]->mu); m = ctxs[g]->err; } fail0(rcs[g], m); break; }
         }
         return rc;
     }
@@ -1745,7 +1765,7 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
     for (uint32_t g = 0; g < G; g++) {
         memcpy(out_cap + (size_t)g * (4ULL << local_cap_height), trees[g]->cap.data(), 32ULL << local_cap_height);
         std::lock_guard<std::mutex> lk(ctxs[g]->mu);
-        out_trees[g] = put_tree(ctxs[g], std::move(trees[g]));
+        out_trees[g] = ctxs[g]->trees.put(ctxs[g], std::move(trees[g]));
     }
     return GL_OK;
 }
@@ -1753,7 +1773,7 @@ int gl_commit_multi(gl_ctx* const* ctxs, uint32_t n_ctx, const uint64_t* const* 
 int gl_tree_info(gl_ctx* c, gl_handle h, gl_tree_info_t* out) {
     GL_API_BEGIN(c)
     if (!out) GL_THROW(GL_ERR_INVALID, "out is NULL");
-    Tree* t = find_tree(c, h);
+    Tree* t = c->trees.get(h);
     out->n_leaves = t->n_leaves; out->leaf_len = t->leaf_len; out->cap_height = t->cap_height;
     out->degree_log = t->degree_log; out->rate_bits = t->rate_bits; out->has_coeffs = t->has_coeffs; out->pitch = t->pitch;
     return GL_OK;
@@ -1762,23 +1782,20 @@ int gl_tree_info(gl_ctx* c, gl_handle h, gl_tree_info_t* out) {
 
 int gl_tree_get(gl_ctx* c, gl_handle h, uint64_t leaf_index, uint64_t* out_row) {
     GL_API_BEGIN(c)
-    Tree* t = find_tree(c, h);
+    Tree* t = c->trees.get(h);
     if (leaf_index >= t->n_leaves || !out_row) GL_THROW(GL_ERR_INVALID, "leaf index out of range");
-    CUDA_CHECK(cudaMemcpyAsync(out_row, t->leaves.p + leaf_index * t->pitch, (size_t)t->leaf_len * 8, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    copy_row(c, t, leaf_index, out_row);
     return GL_OK;
     GL_API_END(c)
 }
 
 int gl_tree_get_lde_values(gl_ctx* c, gl_handle h, uint64_t index, uint64_t step, uint64_t* out_row) {
     GL_API_BEGIN(c)
-    Tree* t = find_tree(c, h);
+    Tree* t = c->trees.get(h);
     if (!out_row) GL_THROW(GL_ERR_INVALID, "out_row is NULL");
     if (step != 0 && index > (t->n_leaves - 1) / step) GL_THROW(GL_ERR_INVALID, "index * step out of range");   // also rules out a wrapped product
     uint64_t i = index * step;
-    uint64_t row = h_bitrev((uint32_t)i, log2_exact(t->n_leaves));
-    CUDA_CHECK(cudaMemcpyAsync(out_row, t->leaves.p + row * t->pitch, (size_t)t->leaf_len * 8, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    copy_row(c, t, h_bitrev((uint32_t)i, log2_exact(t->n_leaves)), out_row);
     return GL_OK;
     GL_API_END(c)
 }
@@ -1811,7 +1828,7 @@ void open_batch_impl(gl_ctx* c, Tree* t, const uint64_t* leaf_indices, uint32_t 
 
 int gl_tree_prove(gl_ctx* c, gl_handle h, uint64_t leaf_index, uint64_t* out_siblings) {
     GL_API_BEGIN(c)
-    Tree* t = find_tree(c, h);
+    Tree* t = c->trees.get(h);
     if (leaf_index >= t->n_leaves) GL_THROW(GL_ERR_INVALID, "leaf index out of range");
     uint32_t log_sub = log2_exact(t->n_leaves) - t->cap_height;
     if (!out_siblings && log_sub) GL_THROW(GL_ERR_INVALID, "out_siblings is NULL");   /* an empty proof needs no buffer */
@@ -1822,7 +1839,7 @@ int gl_tree_prove(gl_ctx* c, gl_handle h, uint64_t leaf_index, uint64_t* out_sib
 
 int gl_tree_open_batch(gl_ctx* c, gl_handle h, const uint64_t* leaf_indices, uint32_t n, uint64_t* out_rows, uint64_t* out_siblings) {
     GL_API_BEGIN(c)
-    Tree* t = find_tree(c, h);
+    Tree* t = c->trees.get(h);
     open_batch_impl(c, t, leaf_indices, n, out_rows, out_siblings);
     return GL_OK;
     GL_API_END(c)
@@ -1830,7 +1847,7 @@ int gl_tree_open_batch(gl_ctx* c, gl_handle h, const uint64_t* leaf_indices, uin
 
 int gl_tree_read(gl_ctx* c, gl_handle h, int part, uint64_t* out) {
     GL_API_BEGIN(c)
-    Tree* t = find_tree(c, h);
+    Tree* t = c->trees.get(h);
     if (!out) GL_THROW(GL_ERR_INVALID, "out is NULL");
     switch (part) {
         case GL_PART_COEFFS: {
@@ -1848,11 +1865,9 @@ int gl_tree_read(gl_ctx* c, gl_handle h, int part, uint64_t* out) {
                 CUDA_CHECK(cudaMemcpy2DAsync(out, (size_t)t->leaf_len * 8, t->leaves.p, (size_t)t->pitch * 8, (size_t)t->leaf_len * 8,
                                              t->n_leaves, cudaMemcpyDeviceToHost, c->stream));
             break;
-        case GL_PART_DIGESTS: {
-            uint64_t n_dig = 2 * (t->n_leaves - (1ULL << t->cap_height));
-            if (n_dig) CUDA_CHECK(cudaMemcpyAsync(out, t->digests.p, n_dig * 32, cudaMemcpyDeviceToHost, c->stream));
+        case GL_PART_DIGESTS:
+            if (t->n_digests()) CUDA_CHECK(cudaMemcpyAsync(out, t->digests.p, t->n_digests() * 32, cudaMemcpyDeviceToHost, c->stream));
             break;
-        }
         case GL_PART_CAP: memcpy(out, t->cap.data(), t->cap.size() * 8); break;
         default: GL_THROW(GL_ERR_INVALID, "unknown part %d", part);
     }
@@ -1863,9 +1878,7 @@ int gl_tree_read(gl_ctx* c, gl_handle h, int part, uint64_t* out) {
 
 int gl_tree_free(gl_ctx* c, gl_handle h) {
     GL_API_BEGIN(c)
-    find_tree(c, h);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    c->trees.erase(h);
+    c->trees.drop(c, h);
     return GL_OK;
     GL_API_END(c)
 }
@@ -1876,9 +1889,7 @@ int gl_fri_begin(gl_ctx* c, const uint64_t* coeffs_ext, const uint64_t* values_e
     GL_API_BEGIN(c)
     if (!coeffs_ext || !values_ext || !out_fri) GL_THROW(GL_ERR_INVALID, "NULL pointer");
     if (len == 0 || (len & (len - 1)) || len > (1ULL << 31)) GL_THROW(GL_ERR_INVALID, "len must be a power of two");
-    auto f = std::make_unique<Fri>();
-    f->len = len; f->rate_bits = rate_bits; f->cap_height = cap_height;
-    f->coeffs.ensure(2 * len); f->values.ensure(2 * len); f->tmp.ensure(2 * len);
+    auto f = std::make_unique<Fri>(len, rate_bits, cap_height);
     CUDA_CHECK(cudaMemcpyAsync(f->coeffs.p, coeffs_ext, 16 * len, cudaMemcpyHostToDevice, c->stream));
     CUDA_CHECK(cudaMemcpyAsync(f->tmp.p, values_ext, 16 * len, cudaMemcpyHostToDevice, c->stream));
     fri::canon_kernel<<<(uint32_t)((2 * len + 255) / 256), 256, 0, c->stream>>>(f->coeffs.p, 2 * len);
@@ -1888,9 +1899,7 @@ int gl_fri_begin(gl_ctx* c, const uint64_t* coeffs_ext, const uint64_t* values_e
         reinterpret_cast<const ulonglong2*>(f->tmp.p), reinterpret_cast<ulonglong2*>(f->values.p), bits);
     CUDA_CHECK(cudaGetLastError());
     CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    gl_handle h = c->next_handle++;
-    c->fris[h] = std::move(f);
-    *out_fri = h;
+    *out_fri = c->fris.put(c, std::move(f));
     return GL_OK;
     GL_API_END(c)
 }
@@ -1898,21 +1907,15 @@ int gl_fri_begin(gl_ctx* c, const uint64_t* coeffs_ext, const uint64_t* values_e
 int gl_fri_commit_layer(gl_ctx* c, gl_handle fh, uint32_t arity_bits, uint64_t* out_leaves, uint64_t* out_digests, uint64_t* out_cap,
                         gl_handle* out_tree) {
     GL_API_BEGIN(c)
-    Fri* f = find_fri(c, fh);
+    Fri* f = c->fris.get(fh);
     if (!out_cap) GL_THROW(GL_ERR_INVALID, "out_cap is NULL");
     uint64_t arity = 1ULL << arity_bits;
     if (arity > f->len) GL_THROW(GL_ERR_INVALID, "arity larger than the codeword");
     uint64_t n_leaves = f->len >> arity_bits;
     uint32_t leaf_len = (uint32_t)(2 * arity);
     if ((1ULL << f->cap_height) > n_leaves) GL_THROW(GL_ERR_INVALID, "cap_height should be at most log2(leaves.len())");
-    auto t = std::make_unique<Tree>();
     const uint32_t pitch = round_up(leaf_len, 8);
-    const uint64_t n_dig = 2 * (n_leaves - (1ULL << f->cap_height));
-    t->n_leaves = n_leaves; t->leaf_len = leaf_len; t->pitch = pitch; t->cap_height = f->cap_height;
-    t->leaves.ensure(n_leaves * pitch);
-    t->digests.ensure(n_dig * 4);
-    t->d_cap.ensure(4ULL << f->cap_height);
-    t->cap.resize(4ULL << f->cap_height);
+    auto t = std::make_unique<Tree>(n_leaves, leaf_len, pitch, f->cap_height);
     // bit-reversed values chunked by arity ARE the leaves (flatten = the [a0,a1] interleaving already in memory)
     if (pitch == leaf_len) {
         CUDA_CHECK(cudaMemcpyAsync(t->leaves.p, f->values.p, 16 * f->len, cudaMemcpyDeviceToDevice, c->stream));
@@ -1921,15 +1924,10 @@ int gl_fri_commit_layer(gl_ctx* c, gl_handle fh, uint32_t arity_bits, uint64_t* 
                                      cudaMemcpyDeviceToDevice, c->stream));
     }
     merkle_build(c, t->leaves.p, n_leaves, leaf_len, pitch, f->cap_height, t->digests.p, t->d_cap.p, nullptr, nullptr, nullptr);
-    CUDA_CHECK(cudaMemcpyAsync(t->cap.data(), t->d_cap.p, 32ULL << f->cap_height, cudaMemcpyDeviceToHost, c->stream));
     if (out_leaves)
         CUDA_CHECK(cudaMemcpy2DAsync(out_leaves, (size_t)leaf_len * 8, t->leaves.p, (size_t)pitch * 8, (size_t)leaf_len * 8, n_leaves,
                                      cudaMemcpyDeviceToHost, c->stream));
-    if (out_digests && n_dig)
-        CUDA_CHECK(cudaMemcpyAsync(out_digests, t->digests.p, n_dig * 32, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    memcpy(out_cap, t->cap.data(), 32ULL << f->cap_height);
-    if (out_tree) *out_tree = put_tree(c, std::move(t));
+    finish_tree(c, std::move(t), out_digests, out_cap, out_tree);
     f->last_arity_bits = arity_bits;
     return GL_OK;
     GL_API_END(c)
@@ -1937,7 +1935,7 @@ int gl_fri_commit_layer(gl_ctx* c, gl_handle fh, uint32_t arity_bits, uint64_t* 
 
 int gl_fri_fold(gl_ctx* c, gl_handle fh, const uint64_t beta[2]) {
     GL_API_BEGIN(c)
-    Fri* f = find_fri(c, fh);
+    Fri* f = c->fris.get(fh);
     if (!beta) GL_THROW(GL_ERR_INVALID, "beta is NULL");
     if (f->last_arity_bits == 0) GL_THROW(GL_ERR_INVALID, "gl_fri_fold without a preceding gl_fri_commit_layer");
     NvtxRange nv("fold codewords in the commitment phase");
@@ -1964,7 +1962,7 @@ int gl_fri_fold(gl_ctx* c, gl_handle fh, const uint64_t beta[2]) {
 
 int gl_fri_final_poly(gl_ctx* c, gl_handle fh, uint64_t* out, uint64_t* out_len) {
     GL_API_BEGIN(c)
-    Fri* f = find_fri(c, fh);
+    Fri* f = c->fris.get(fh);
     uint64_t n = f->len >> f->rate_bits;
     if (out_len) *out_len = n;
     if (out && n) CUDA_CHECK(cudaMemcpyAsync(out, f->coeffs.p, 16 * n, cudaMemcpyDeviceToHost, c->stream));
@@ -1975,20 +1973,13 @@ int gl_fri_final_poly(gl_ctx* c, gl_handle fh, uint64_t* out, uint64_t* out_len)
 
 int gl_fri_end(gl_ctx* c, gl_handle fh) {
     GL_API_BEGIN(c)
-    find_fri(c, fh);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    c->fris.erase(fh);
+    c->fris.drop(c, fh);
     return GL_OK;
     GL_API_END(c)
 }
 
 // ------------------------------------------------------------------------------------------------ prove_openings (front half)
 namespace {
-Openings* find_openings(gl_ctx* c, gl_handle h) {
-    auto it = c->openings.find(h);
-    if (it == c->openings.end()) GL_THROW(GL_ERR_HANDLE, "unknown openings handle %llu", (unsigned long long)h);
-    return it->second.get();
-}
 struct HExt { uint64_t a0, a1; };
 HExt h_ext_mul(HExt a, HExt b) {   // F_p[X]/(X^2 - 7)
     uint64_t m11 = gl::h_mul(a.a1, b.a1);
@@ -2010,9 +2001,7 @@ int gl_openings_begin(gl_ctx* c, uint32_t log_n, gl_handle* out) {
     o->comp.ensure(2 * n);
     CUDA_CHECK(cudaMemsetAsync(o->final_poly.p, 0, 16 * n, c->stream));
     CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    gl_handle h = c->next_handle++;
-    c->openings[h] = std::move(o);
-    *out = h;
+    *out = c->openings.put(c, std::move(o));
     return GL_OK;
     GL_API_END(c)
 }
@@ -2020,7 +2009,7 @@ int gl_openings_begin(gl_ctx* c, uint32_t log_n, gl_handle* out) {
 int gl_openings_add_batch(gl_ctx* c, gl_handle oh, const gl_handle* batches, const uint32_t* columns, uint32_t n_polys,
                           const uint64_t alpha[2], const uint64_t point[2], uint64_t* out_quotient) {
     GL_API_BEGIN(c)
-    Openings* o = find_openings(c, oh);
+    Openings* o = c->openings.get(oh);
     if (!alpha || !point || (n_polys && (!batches || !columns))) GL_THROW(GL_ERR_INVALID, "NULL pointer");
     const uint32_t n = 1u << o->log_n;
     std::vector<openings::PolyRef> refs(n_polys);
@@ -2028,7 +2017,7 @@ int gl_openings_add_batch(gl_ctx* c, gl_handle oh, const gl_handle* batches, con
     const HExt al = {gl::canon(alpha[0]), gl::canon(alpha[1])};
     HExt cur = {1, 0};
     for (uint32_t j = 0; j < n_polys; j++) {
-        Tree* t = find_tree(c, batches[j]);
+        Tree* t = c->trees.get(batches[j]);
         if (!t->has_coeffs) GL_THROW(GL_ERR_INVALID, "polynomial %u: the tree has no coefficients", j);
         if (t->degree_log != o->log_n) GL_THROW(GL_ERR_INVALID, "Polynomial degrees inconsistent (polynomial %u has degree_log %u, expected %u)",
                                                 j, t->degree_log, o->log_n);
@@ -2066,7 +2055,7 @@ int gl_openings_add_batch(gl_ctx* c, gl_handle oh, const gl_handle* batches, con
 
 int gl_openings_final_poly(gl_ctx* c, gl_handle oh, uint64_t* out) {
     GL_API_BEGIN(c)
-    Openings* o = find_openings(c, oh);
+    Openings* o = c->openings.get(oh);
     if (!out) GL_THROW(GL_ERR_INVALID, "out is NULL");
     CUDA_CHECK(cudaMemcpyAsync(out, o->final_poly.p, 16ULL << o->log_n, cudaMemcpyDeviceToHost, c->stream));
     CUDA_CHECK(cudaStreamSynchronize(c->stream));
@@ -2076,13 +2065,11 @@ int gl_openings_final_poly(gl_ctx* c, gl_handle oh, uint64_t* out) {
 
 int gl_openings_lde(gl_ctx* c, gl_handle oh, uint32_t rate_bits, uint32_t cap_height, gl_handle* out_fri) {
     GL_API_BEGIN(c)
-    Openings* o = find_openings(c, oh);
+    Openings* o = c->openings.get(oh);
     if (!out_fri) GL_THROW(GL_ERR_INVALID, "out_fri is NULL");
     if (o->log_n + rate_bits > 31) GL_THROW(GL_ERR_UNSUPPORTED, "log_n + rate_bits = %u > 31", o->log_n + rate_bits);
     const uint64_t n = 1ULL << o->log_n, len = n << rate_bits;
-    auto f = std::make_unique<Fri>();
-    f->len = len; f->rate_bits = rate_bits; f->cap_height = cap_height;
-    f->coeffs.ensure(2 * len); f->values.ensure(2 * len); f->tmp.ensure(2 * len);
+    auto f = std::make_unique<Fri>(len, rate_bits, cap_height);
     // final_poly.lde(rate_bits): zero-padded coefficients; values = coset_fft(shift 7), kept bit-reversed (in-place DIF order)
     CUDA_CHECK(cudaMemsetAsync(f->coeffs.p, 0, 16 * len, c->stream));
     CUDA_CHECK(cudaMemcpyAsync(f->coeffs.p, o->final_poly.p, 16 * n, cudaMemcpyDeviceToDevice, c->stream));
@@ -2093,18 +2080,14 @@ int gl_openings_lde(gl_ctx* c, gl_handle oh, uint32_t rate_bits, uint32_t cap_he
         run_ntt(c, f->coeffs.p, 2, f->values.p, 2, 2, log_len, false, get_coset_table(c, gl::COSET_SHIFT, log_len), 2, nullptr);
     }
     CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    gl_handle h = c->next_handle++;
-    c->fris[h] = std::move(f);
-    *out_fri = h;
+    *out_fri = c->fris.put(c, std::move(f));
     return GL_OK;
     GL_API_END(c)
 }
 
 int gl_openings_end(gl_ctx* c, gl_handle oh) {
     GL_API_BEGIN(c)
-    find_openings(c, oh);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    c->openings.erase(oh);
+    c->openings.drop(c, oh);
     return GL_OK;
     GL_API_END(c)
 }
@@ -2112,7 +2095,7 @@ int gl_openings_end(gl_ctx* c, gl_handle oh) {
 // ------------------------------------------------------------------------------------------------ OpeningSet::new
 int gl_batch_eval(gl_ctx* c, gl_handle batch, const uint64_t* points_ext, uint32_t n_points, uint64_t* out_values_ext) {
     GL_API_BEGIN(c)
-    Tree* t = find_tree(c, batch);
+    Tree* t = c->trees.get(batch);
     if (!t->has_coeffs) GL_THROW(GL_ERR_INVALID, "tree has no coefficients");
     if (!points_ext || !out_values_ext) GL_THROW(GL_ERR_INVALID, "NULL pointer");
     if (n_points == 0) GL_THROW(GL_ERR_INVALID, "n_points must be at least 1");
@@ -2156,7 +2139,7 @@ int gl_batch_eval(gl_ctx* c, gl_handle batch, const uint64_t* points_ext, uint32
 
 int gl_fri_read(gl_ctx* c, gl_handle fh, uint64_t* out_coeffs, uint64_t* out_values, uint64_t* out_len) {
     GL_API_BEGIN(c)
-    Fri* f = find_fri(c, fh);
+    Fri* f = c->fris.get(fh);
     if (out_len) *out_len = f->len;
     if (out_coeffs) CUDA_CHECK(cudaMemcpyAsync(out_coeffs, f->coeffs.p, 16 * f->len, cudaMemcpyDeviceToHost, c->stream));
     if (out_values) CUDA_CHECK(cudaMemcpyAsync(out_values, f->values.p, 16 * f->len, cudaMemcpyDeviceToHost, c->stream));
@@ -2206,11 +2189,6 @@ void check_gate(int kind, uint32_t param) {
     if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_COMPARISON) GL_THROW(GL_ERR_INVALID, "unknown gate kind %d", kind);
     if (gate_wires(kind, param) < 0) GL_THROW(GL_ERR_INVALID, "gate kind %d: parameter %u out of range (see include/gl_commit.h)", kind, param);
 }
-Quotient* find_quotient(gl_ctx* c, gl_handle h) {
-    auto it = c->quotients.find(h);
-    if (it == c->quotients.end()) GL_THROW(GL_ERR_HANDLE, "unknown quotient handle %llu", (unsigned long long)h);
-    return it->second.get();
-}
 }  // namespace
 
 int gl_gate_num_wires(int kind, uint32_t param) { return gate_wires(kind, param); }
@@ -2238,16 +2216,14 @@ int gl_quotient_begin(gl_ctx* c, gl_handle wires_batch, uint32_t n_challenges, g
     GL_API_BEGIN(c)
     if (!out_q) GL_THROW(GL_ERR_INVALID, "out_quotient is NULL");
     if (n_challenges == 0 || n_challenges > (uint32_t)gates::MAX_CHALLENGES) GL_THROW(GL_ERR_INVALID, "n_challenges must be 1..%d", gates::MAX_CHALLENGES);
-    Tree* t = find_tree(c, wires_batch);
+    Tree* t = c->trees.get(wires_batch);
     auto q = std::make_unique<Quotient>();
     q->wires = wires_batch; q->n_rows = t->n_leaves; q->n_challenges = n_challenges;
     q->acc.ensure(q->n_rows * n_challenges);
     q->powers.ensure((size_t)gates::MAX_CHALLENGES * gates::MAX_CONSTRAINTS);
     CUDA_CHECK(cudaMemsetAsync(q->acc.p, 0, q->n_rows * n_challenges * 8, c->stream));
     CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    gl_handle h = c->next_handle++;
-    c->quotients[h] = std::move(q);
-    *out_q = h;
+    *out_q = c->quotients.put(c, std::move(q));
     return GL_OK;
     GL_API_END(c)
 }
@@ -2255,10 +2231,10 @@ int gl_quotient_begin(gl_ctx* c, gl_handle wires_batch, uint32_t n_challenges, g
 int gl_quotient_add_gate(gl_ctx* c, gl_handle qh, int kind, uint32_t param, const uint64_t* alphas, uint32_t constraint_offset,
                          gl_handle filter_batch, uint32_t filter_col) {
     GL_API_BEGIN(c)
-    Quotient* q = find_quotient(c, qh);
+    Quotient* q = c->quotients.get(qh);
     check_gate(kind, param);
     if (!alphas) GL_THROW(GL_ERR_INVALID, "alphas is NULL");
-    Tree* t = find_tree(c, q->wires);
+    Tree* t = c->trees.get(q->wires);
     const uint32_t nw = (uint32_t)gate_wires(kind, param), nc = (uint32_t)gate_constraints(kind, param);
     if (t->leaf_len < nw) GL_THROW(GL_ERR_INVALID, "the wires batch has %u columns, the gate needs %u", t->leaf_len, nw);
     if (nc > (uint32_t)gates::MAX_CONSTRAINTS) GL_THROW(GL_ERR_UNSUPPORTED, "too many constraints");
@@ -2266,7 +2242,7 @@ int gl_quotient_add_gate(gl_ctx* c, gl_handle qh, int kind, uint32_t param, cons
     a.rows = t->leaves.p; a.pitch = t->pitch; a.n_rows = q->n_rows; a.acc = q->acc.p; a.powers = q->powers.p;
     a.n_constraints = nc; a.n_challenges = q->n_challenges; a.kind = (uint32_t)kind; a.param = param;
     if (filter_batch) {
-        Tree* f = find_tree(c, filter_batch);
+        Tree* f = c->trees.get(filter_batch);
         if (f->n_leaves != q->n_rows) GL_THROW(GL_ERR_INVALID, "filter batch has %llu rows, the wires batch %llu", (unsigned long long)f->n_leaves, (unsigned long long)q->n_rows);
         if (filter_col >= f->leaf_len) GL_THROW(GL_ERR_INVALID, "filter column %u out of range", filter_col);
         a.filter = f->leaves.p; a.filter_pitch = f->pitch; a.filter_col = filter_col;
@@ -2299,12 +2275,12 @@ int gl_quotient_add_gate(gl_ctx* c, gl_handle qh, int kind, uint32_t param, cons
 int gl_quotient_add_permutation(gl_ctx* c, gl_handle qh, gl_handle sigmas_batch, uint32_t sigma_col0, gl_handle zs_batch, uint32_t n_routed,
                                 uint32_t degree, const uint64_t* k_is, const uint64_t* betas, const uint64_t* gammas, const uint64_t* alphas) {
     GL_API_BEGIN(c)
-    Quotient* q = find_quotient(c, qh);
+    Quotient* q = c->quotients.get(qh);
     if (!k_is || !betas || !gammas || !alphas) GL_THROW(GL_ERR_INVALID, "NULL pointer");
     if (n_routed == 0 || degree == 0) GL_THROW(GL_ERR_INVALID, "n_routed and degree must be positive");
-    Tree* tw = find_tree(c, q->wires);
-    Tree* ts = find_tree(c, sigmas_batch);
-    Tree* tz = find_tree(c, zs_batch);
+    Tree* tw = c->trees.get(q->wires);
+    Tree* ts = c->trees.get(sigmas_batch);
+    Tree* tz = c->trees.get(zs_batch);
     const uint32_t n_ch = q->n_challenges, n_chunks = (n_routed + degree - 1) / degree, n_terms = n_ch * (1 + n_chunks);
     if (!tw->has_coeffs || tw->rate_bits > 6) GL_THROW(GL_ERR_UNSUPPORTED, "the wires batch must be a PolynomialBatch commit with rate_bits <= 6");
     for (Tree* t : {ts, tz})
@@ -2359,7 +2335,7 @@ int gl_quotient_add_permutation(gl_ctx* c, gl_handle qh, gl_handle sigmas_batch,
 
 int gl_quotient_read(gl_ctx* c, gl_handle qh, uint64_t* out) {
     GL_API_BEGIN(c)
-    Quotient* q = find_quotient(c, qh);
+    Quotient* q = c->quotients.get(qh);
     if (!out) GL_THROW(GL_ERR_INVALID, "out is NULL");
     CUDA_CHECK(cudaMemcpyAsync(out, q->acc.p, q->n_rows * q->n_challenges * 8, cudaMemcpyDeviceToHost, c->stream));
     CUDA_CHECK(cudaStreamSynchronize(c->stream));
@@ -2369,8 +2345,8 @@ int gl_quotient_read(gl_ctx* c, gl_handle qh, uint64_t* out) {
 
 int gl_quotient_commit(gl_ctx* c, gl_handle qh, uint32_t cap_height, uint64_t* out_cap, gl_handle* out_batch) {
     GL_API_BEGIN(c)
-    Quotient* q = find_quotient(c, qh);
-    Tree* t = find_tree(c, q->wires);
+    Quotient* q = c->quotients.get(qh);
+    Tree* t = c->trees.get(q->wires);
     if (!out_cap) GL_THROW(GL_ERR_INVALID, "out_cap is NULL");
     const uint32_t log_n = t->degree_log, r = t->rate_bits, bits = log_n + r, n_ch = q->n_challenges;
     if (!t->has_coeffs) GL_THROW(GL_ERR_INVALID, "the wires batch is not a PolynomialBatch commit");
@@ -2405,9 +2381,7 @@ int gl_quotient_commit(gl_ctx* c, gl_handle qh, uint32_t cap_height, uint64_t* o
 
 int gl_quotient_end(gl_ctx* c, gl_handle qh) {
     GL_API_BEGIN(c)
-    find_quotient(c, qh);
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    c->quotients.erase(qh);
+    c->quotients.drop(c, qh);
     return GL_OK;
     GL_API_END(c)
 }
