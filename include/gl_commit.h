@@ -177,18 +177,45 @@ int gl_fri_read(gl_ctx* ctx, gl_handle fri, uint64_t* out_coeffs_ext, uint64_t* 
  *   GL_GATE_U32_INTERLEAVE  .../interleave_u32.rs:104-140      param = num_ops (<= 3)                   34*num_ops wires and constraints
  *   GL_GATE_UNINTERLEAVE_TO_U32 / _TO_B32  .../uninterleave_to_u32.rs:91-134, uninterleave_to_b32.rs:115-168   param = num_ops (<= 2)   67*num_ops each
  *   GL_GATE_COMPARISON      .../comparison.rs:112-190          param = num_bits | num_chunks << 8      5*num_chunks + chunk_bits + 5 wires, + 6 constraints
+ * and plonky2's core gates (plonky2 @ 3de92d9 gates/{noop,constant,public_input,arithmetic_base,base_sum}.rs; upstream source not in
+ * the reference tree: restated, parity unpinned):
+ *   GL_GATE_NOOP            NoopGate                           param 0                                  0 wires, 0 constraints, 0 constants
+ *   GL_GATE_CONSTANT        ConstantGate                       param = num_consts (1..8)                n wires, n constraints, n constants
+ *   GL_GATE_PUBLIC_INPUT    PublicInputGate                    param 0                                  4 wires, 4 constraints, 0 constants
+ *   GL_GATE_ARITHMETIC      ArithmeticGate (base)              param = num_ops (1..33; 20 at 80 routed)  4*n wires, n constraints, 2 constants
+ *   GL_GATE_BASE_SUM        BaseSumGate<B>                     param = num_limbs | B << 8 (B 2..16)      1+n wires, 1+n constraints, 0 constants
  * gl_quotient_add_gate:  acc[k][row] += filter(row) * sum_i alphas[k]^(constraint_offset + i) * constraint_i(wires(row)),  k < n_challenges
- * (alphas are BASE-field challenges, as upstream; filter(row) = column filter_col of the batch filter_batch at the same row — the LDE of the
- * gate's selector filter — or 1 when filter_batch == 0).  gl_quotient_read: [n_challenges][R] words, row order = the leaves' (bit-reversed). */
+ * (alphas are BASE-field challenges, as upstream; filter(row) = column filter_col of the batch filter_batch at the same row, or 1 when
+ * filter_batch == 0).  gl_quotient_read: [n_challenges][R] words, row order = the leaves' (bit-reversed).
+ * gl_gate_eval_rows and gl_quotient_add_gate refuse the gates that read gate constants or the public-inputs hash (CONSTANT, ARITHMETIC,
+ * PUBLIC_INPUT): those go through gl_gate_eval_rows_with_constants and gl_quotient_add_gates.                                             */
 enum { GL_GATE_POSEIDON2 = 0, GL_GATE_U32_ARITHMETIC = 1, GL_GATE_U32_ADD_MANY = 2, GL_GATE_U32_SUBTRACTION = 3, GL_GATE_U32_RANGE_CHECK = 4,
-       GL_GATE_U32_INTERLEAVE = 5, GL_GATE_UNINTERLEAVE_TO_U32 = 6, GL_GATE_UNINTERLEAVE_TO_B32 = 7, GL_GATE_COMPARISON = 8 };
+       GL_GATE_U32_INTERLEAVE = 5, GL_GATE_UNINTERLEAVE_TO_U32 = 6, GL_GATE_UNINTERLEAVE_TO_B32 = 7, GL_GATE_COMPARISON = 8, GL_GATE_NOOP = 9,
+       GL_GATE_CONSTANT = 10, GL_GATE_PUBLIC_INPUT = 11, GL_GATE_ARITHMETIC = 12, GL_GATE_BASE_SUM = 13 };
 int gl_gate_num_wires(int kind, uint32_t param);
 int gl_gate_num_constraints(int kind, uint32_t param);
+/* Gate::num_constants: the gate constants a gate reads (-1 for a bad kind or parameter) */
+int gl_gate_num_constants(int kind, uint32_t param);
 /* every constraint value of every row, uncombined (host rows [n_rows][num_wires] -> out [n_rows][num_constraints]); tests, debugging */
 int gl_gate_eval_rows(gl_ctx* ctx, int kind, uint32_t param, const uint64_t* rows, uint64_t n_rows, uint64_t* out);
+/* gl_gate_eval_rows for every kind, with the gate constants of each row: consts [n_rows][gl_gate_num_constants] (NULL if that is 0) */
+int gl_gate_eval_rows_with_constants(gl_ctx* ctx, int kind, uint32_t param, const uint64_t* rows, const uint64_t* consts,
+                                     const uint64_t public_inputs_hash[4], uint64_t n_rows, uint64_t* out);
 int gl_quotient_begin(gl_ctx* ctx, gl_handle wires_batch, uint32_t n_challenges, gl_handle* out_quotient);
 int gl_quotient_add_gate(gl_ctx* ctx, gl_handle quotient, int kind, uint32_t param, const uint64_t* alphas, uint32_t constraint_offset,
                          gl_handle filter_batch, uint32_t filter_col);
+/* plonky2 plonk/vanishing_poly.rs · evaluate_gate_constraints_base_batch over the resident LDE rows (restated, parity unpinned).
+ * Gate i of CommonCircuitData::gates is (kinds[i], params[i]); SelectorsInfo is selector_indices[n_gates] and groups[2 * num_selectors]
+ * ([start, end) pairs).  constants_sigmas: commit #0 — selectors, lookup selectors and gate constants in columns [0, num_constants), the
+ * sigmas after; it shares the wires batch's rows, degree and rate_bits.  For every gate with constraints, one launch:
+ *     s = constants_sigmas[row][selector_indices[i]],  f_i = prod_{j in group, j != i} (j - s) * (num_selectors > 1 ? 2^32 - 1 - s : 1)
+ *     acc[k][row] += f_i * sum_c alphas[k]^(constraint_offset + c) * c_i,c(row)
+ * with gate constant j = constants_sigmas[row][num_selectors + num_lookup_selectors + j] (gates/gate.rs · compute_filter,
+ * eval_filtered_base_batch).  Every gate is validated before the first launch; a refused call leaves the accumulator unchanged. */
+int gl_quotient_add_gates(gl_ctx* ctx, gl_handle quotient, const int* kinds, const uint32_t* params, uint32_t n_gates,
+                          const uint32_t* selector_indices, const uint32_t* groups, uint32_t num_selectors, uint32_t num_lookup_selectors,
+                          gl_handle constants_sigmas, uint32_t num_constants, const uint64_t public_inputs_hash[4], const uint64_t* alphas,
+                          uint32_t constraint_offset);
 /* the permutation-argument terms of eval_vanishing_poly_base_batch (plonk/vanishing_poly.rs; restated, parity unpinned): for every challenge i
  * L_0(x)(Z_i(x) - 1), then check_partial_products of every challenge — vanishing_terms[0 .. n_ch*(1 + n_chunks)), each alpha_k reducing the
  * whole list; gate constraints follow from constraint_offset = n_ch * (1 + n_chunks).  sigmas_batch: the constants+sigmas commit, the sigma
@@ -205,7 +232,8 @@ int gl_quotient_read(gl_ctx* ctx, gl_handle quotient, uint64_t* out);
  * out_batch: the committed batch (coefficients, leaves, digests resident), as from gl_commit.  Restated from upstream (parity unpinned).  */
 int gl_quotient_commit(gl_ctx* ctx, gl_handle quotient, uint32_t cap_height, uint64_t* out_cap, gl_handle* out_batch);
 int gl_quotient_end(gl_ctx* ctx, gl_handle quotient);
-/* CUDA-event milliseconds of the last gl_quotient_add_gate / gl_poseidon2_gate_witness kernel on this context */
+/* CUDA-event milliseconds of the last gl_quotient_add_gate / gl_poseidon2_gate_witness kernel on this context (gl_quotient_add_gates:
+ * from its first launch to its last; 0 when it launched nothing) */
 int gl_ctx_aux_ms(gl_ctx* ctx, float* out_ms);
 /* witness generation for Poseidon2Gate rows (poseidon2_gate.rs:447-523 · Poseidon2Generator::run_once): inputs [n][13] = the 12 state
  * inputs + the swap flag of each row -> out_rows [n][135], every wire of the row (deltas, S-box inputs of all rounds, outputs)        */

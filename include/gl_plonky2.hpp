@@ -748,6 +748,14 @@ inline std::vector<F> evaluate_gate_constraints(int kind, uint32_t param, const 
     return out;
 }
 
+/* plonky2 gates/selectors.rs · SelectorsInfo: gate i is filtered by selector column selector_indices[i], whose gate range is
+ * groups[selector_indices[i]] = [first, second) */
+struct SelectorsInfo {
+    std::vector<size_t> selector_indices;
+    std::vector<std::pair<size_t, size_t>> groups;
+    size_t num_selectors() const { return groups.size(); }
+};
+
 /* the gate part of plonky2 plonk/prover.rs · compute_quotient_polys over the resident LDE rows of the wires commit, and its tail
  * (divide by Z_H on the coset, coset_ifft, chunks(degree), PolynomialBatch::from_coeffs) */
 class QuotientAccumulator {
@@ -759,6 +767,12 @@ public:
     /* acc[k][row] += filter(row) * sum_i alphas[k]^(constraint_offset + i) * constraint_i(row) */
     void add_gate(int kind, uint32_t param, const std::vector<F>& alphas, size_t constraint_offset = 0, const PolynomialBatch* filter_batch = nullptr,
                   size_t filter_col = 0);
+    /* plonk/vanishing_poly.rs · evaluate_gate_constraints_base_batch: gates[i] = (kind, param) of CommonCircuitData::gates; each gate's
+     * constraints times compute_filter(i, group, s(x), num_selectors > 1), s its selector column of constants_sigmas (commit #0), gate
+     * constants from the columns after the selectors; constraint c weighted by alphas[k]^(constraint_offset + c) */
+    void add_gates(const std::vector<std::pair<int, uint32_t>>& gates, const SelectorsInfo& selectors_info, size_t num_lookup_selectors,
+                   const PolynomialBatch& constants_sigmas, size_t num_constants, const HashOut& public_inputs_hash, const std::vector<F>& alphas,
+                   size_t constraint_offset);
     /* the permutation-argument terms of eval_vanishing_poly_base_batch (vanishing_terms[0 .. n_ch * (1 + n_chunks))) */
     void add_permutation(const PolynomialBatch& sigmas, size_t sigma_col0, const PolynomialBatch& zs_partial_products, size_t n_routed, size_t degree,
                          const std::vector<F>& k_is, const std::vector<F>& betas, const std::vector<F>& gammas, const std::vector<F>& alphas) {
@@ -827,6 +841,20 @@ inline void QuotientAccumulator::add_gate(int kind, uint32_t param, const std::v
     if (alphas.size() != n_challenges_) throw Panic("QuotientAccumulator::add_gate: one alpha per challenge expected");
     ctx_->check(gl_quotient_add_gate(ctx_->raw(), h_, kind, param, alphas.data(), uint32_t(constraint_offset),
                                      filter_batch ? filter_batch->merkle_tree.handle() : 0, uint32_t(filter_col)));
+}
+inline void QuotientAccumulator::add_gates(const std::vector<std::pair<int, uint32_t>>& gates, const SelectorsInfo& selectors_info,
+                                           size_t num_lookup_selectors, const PolynomialBatch& constants_sigmas, size_t num_constants,
+                                           const HashOut& public_inputs_hash, const std::vector<F>& alphas, size_t constraint_offset) {
+    if (alphas.size() != n_challenges_) throw Panic("QuotientAccumulator::add_gates: one alpha per challenge expected");
+    if (selectors_info.selector_indices.size() != gates.size()) throw Panic("QuotientAccumulator::add_gates: one selector index per gate expected");
+    std::vector<int> kinds;
+    std::vector<uint32_t> params, sel, groups;
+    for (const auto& g : gates) { kinds.push_back(g.first); params.push_back(g.second); }
+    for (size_t i : selectors_info.selector_indices) sel.push_back(uint32_t(i));
+    for (const auto& r : selectors_info.groups) { groups.push_back(uint32_t(r.first)); groups.push_back(uint32_t(r.second)); }
+    ctx_->check(gl_quotient_add_gates(ctx_->raw(), h_, kinds.data(), params.data(), uint32_t(kinds.size()), sel.data(), groups.data(),
+                                      uint32_t(selectors_info.num_selectors()), uint32_t(num_lookup_selectors), constants_sigmas.merkle_tree.handle(),
+                                      uint32_t(num_constants), public_inputs_hash.elements.data(), alphas.data(), uint32_t(constraint_offset)));
 }
 inline PolynomialBatch QuotientAccumulator::commit(size_t cap_height) {
     if (cap_height > degree_log_ + rate_bits_) throw Panic("cap_height=" + std::to_string(cap_height) + " should be at most log2(leaves.len())");

@@ -12,6 +12,7 @@ from .api import (Challenger, Context, FriBatchInfo, FriOpeningBatch, FriOpening
 from .api import (GATE_COMPARISON, GATE_POSEIDON2, GATE_U32_ADD_MANY, GATE_U32_ARITHMETIC, GATE_U32_INTERLEAVE, GATE_U32_RANGE_CHECK,  # noqa: F401
                   GATE_U32_SUBTRACTION, GATE_UNINTERLEAVE_TO_B32, GATE_UNINTERLEAVE_TO_U32, Quotient, evaluate_gate_constraints, gate_shape,
                   partial_products_and_zs, poseidon2_gate_witness)
+from .api import GATE_ARITHMETIC, GATE_BASE_SUM, GATE_CONSTANT, GATE_NOOP, GATE_PUBLIC_INPUT, SelectorsInfo  # noqa: F401
 from .build import build  # noqa: F401
 
 __all__ = ["Challenger", "Context", "FriBatchInfo", "FriOpeningBatch", "FriOpenings", "FriParams", "FriProofHead", "GlError", "MerkleCap",

@@ -65,9 +65,13 @@ SIGNATURES = {
     "gl_fri_read": (c_int, [c_void_p, c_uint64, c_void_p, c_void_p, POINTER(c_uint64)]),
     "gl_gate_num_wires": (c_int, [c_int, c_uint32]),
     "gl_gate_num_constraints": (c_int, [c_int, c_uint32]),
+    "gl_gate_num_constants": (c_int, [c_int, c_uint32]),
     "gl_gate_eval_rows": (c_int, [c_void_p, c_int, c_uint32, c_void_p, c_uint64, c_void_p]),
+    "gl_gate_eval_rows_with_constants": (c_int, [c_void_p, c_int, c_uint32, c_void_p, c_void_p, c_void_p, c_uint64, c_void_p]),
     "gl_quotient_begin": (c_int, [c_void_p, c_uint64, c_uint32, POINTER(c_uint64)]),
     "gl_quotient_add_gate": (c_int, [c_void_p, c_uint64, c_int, c_uint32, c_void_p, c_uint32, c_uint64, c_uint32]),
+    "gl_quotient_add_gates": (c_int, [c_void_p, c_uint64, c_void_p, c_void_p, c_uint32, c_void_p, c_void_p, c_uint32, c_uint32, c_uint64, c_uint32,
+                                      c_void_p, c_void_p, c_uint32]),
     "gl_quotient_add_permutation": (c_int, [c_void_p, c_uint64, c_uint64, c_uint32, c_uint64, c_uint32, c_uint32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gl_quotient_read": (c_int, [c_void_p, c_uint64, c_void_p]),
     "gl_quotient_commit": (c_int, [c_void_p, c_uint64, c_uint32, c_void_p, POINTER(c_uint64)]),

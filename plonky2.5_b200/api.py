@@ -606,6 +606,8 @@ def fri_prover_query_rounds(initial_merkle_trees: Sequence[MerkleTree], trees: S
 # ---- SURVEY §8(f) ranks 3-4: gate constraints over the resident LDE rows, partial products / Z, witness rows -------------------------
 GATE_POSEIDON2, GATE_U32_ARITHMETIC, GATE_U32_ADD_MANY, GATE_U32_SUBTRACTION, GATE_U32_RANGE_CHECK = 0, 1, 2, 3, 4
 GATE_U32_INTERLEAVE, GATE_UNINTERLEAVE_TO_U32, GATE_UNINTERLEAVE_TO_B32, GATE_COMPARISON = 5, 6, 7, 8
+# plonky2's core gates: NoopGate, ConstantGate { num_consts }, PublicInputGate, ArithmeticGate { num_ops }, BaseSumGate<B> (num_limbs | B << 8)
+GATE_NOOP, GATE_CONSTANT, GATE_PUBLIC_INPUT, GATE_ARITHMETIC, GATE_BASE_SUM = 9, 10, 11, 12, 13
 
 
 def gate_shape(kind: int, param: int = 0) -> Tuple[int, int]:
@@ -617,16 +619,42 @@ def gate_shape(kind: int, param: int = 0) -> Tuple[int, int]:
     return nw, nc
 
 
-def evaluate_gate_constraints(kind: int, param: int, rows, ctx: Optional[Context] = None) -> np.ndarray:
-    """Gate::eval_unfiltered_base_batch for host rows [n][num_wires]: every constraint value, uncombined ([n][num_constraints])"""
+def evaluate_gate_constraints(kind: int, param: int, rows, ctx: Optional[Context] = None, constants=None,
+                              public_inputs_hash=None) -> np.ndarray:
+    """Gate::eval_unfiltered_base_batch for host rows [n][num_wires]: every constraint value, uncombined ([n][num_constraints]).
+    Gates that read gate constants or the public-inputs hash (GATE_CONSTANT, GATE_ARITHMETIC, GATE_PUBLIC_INPUT) take `constants`
+    ([n][num_constants], the row's local constants after the selectors) and `public_inputs_hash` (4 words)."""
     ctx = ctx or default_context()
     nw, nc = gate_shape(kind, param)
     r = np.ascontiguousarray(rows, dtype=np.uint64)
     if r.ndim != 2 or r.shape[1] != nw:
         raise ValueError(f"rows must be [n][{nw}]")
     out = np.zeros((r.shape[0], nc), dtype=np.uint64)
-    _check(ctx, ctx.lib.gl_gate_eval_rows(ctx.handle, kind, param, _ptr(r), r.shape[0], _ptr(out)))
+    if constants is None and public_inputs_hash is None:
+        _check(ctx, ctx.lib.gl_gate_eval_rows(ctx.handle, kind, param, _ptr(r), r.shape[0], _ptr(out)))
+        return out
+    nk = ctx.lib.gl_gate_num_constants(kind, param)
+    k = np.ascontiguousarray(np.zeros((r.shape[0], 0)) if constants is None else constants, dtype=np.uint64)
+    if k.shape != (r.shape[0], nk):
+        raise ValueError(f"constants must be [n][{nk}]")
+    pi = np.ascontiguousarray(np.zeros(4) if public_inputs_hash is None else public_inputs_hash, dtype=np.uint64).reshape(-1)
+    if pi.size != 4:
+        raise ValueError("public_inputs_hash must be 4 words")
+    _check(ctx, ctx.lib.gl_gate_eval_rows_with_constants(ctx.handle, kind, param, _ptr(r), _ptr(k) if nk else None, _ptr(pi), r.shape[0],
+                                                         _ptr(out)))
     return out
+
+
+class SelectorsInfo:
+    """plonky2 gates/selectors.rs · SelectorsInfo { selector_indices, groups }: gate i is filtered by selector column
+    selector_indices[i], whose group is the gate range groups[selector_indices[i]] = (start, end)."""
+
+    def __init__(self, selector_indices: Sequence[int], groups: Sequence[Tuple[int, int]]):
+        self.selector_indices = [int(i) for i in selector_indices]
+        self.groups = [(int(a), int(b)) for a, b in groups]
+
+    def num_selectors(self) -> int:
+        return len(self.groups)
 
 
 class Quotient:
@@ -648,6 +676,31 @@ class Quotient:
             raise ValueError("one alpha per challenge expected")
         fb, fc = (filter[0].merkle_tree._h, int(filter[1])) if filter is not None else (0, 0)
         _check(self.ctx, self.ctx.lib.gl_quotient_add_gate(self.ctx.handle, self._h, kind, param, _ptr(a), constraint_offset, fb, fc))
+        ms = ctypes.c_float()
+        self.ctx.lib.gl_ctx_aux_ms(self.ctx.handle, byref(ms))
+        return float(ms.value)
+
+    def add_gates(self, gates: Sequence[Tuple[int, int]], selectors_info: SelectorsInfo, constants_sigmas: "PolynomialBatch", num_constants: int,
+                  public_inputs_hash, alphas, constraint_offset: int = 0, num_lookup_selectors: int = 0) -> float:
+        """plonk/vanishing_poly.rs · evaluate_gate_constraints_base_batch over the LDE rows: gates = CommonCircuitData::gates as
+        (kind, param) pairs; every gate's constraints times compute_filter(i, group, s(x), num_selectors > 1), with s the gate's selector
+        column of `constants_sigmas` (commit #0) and the gate constants its columns after the selectors.  Every gate's constraint c is
+        weighted by alpha_k^(constraint_offset + c).  Returns the kernel time in ms (CUDA events, first launch to last)."""
+        a = np.ascontiguousarray(alphas, dtype=np.uint64).reshape(-1)
+        if a.size != self.n_challenges:
+            raise ValueError("one alpha per challenge expected")
+        pi = np.ascontiguousarray(public_inputs_hash, dtype=np.uint64).reshape(-1)
+        if pi.size != 4:
+            raise ValueError("public_inputs_hash must be 4 words")
+        kinds = np.array([int(g[0]) for g in gates], dtype=np.int32)
+        params = np.array([int(g[1]) for g in gates], dtype=np.uint32)
+        sel = np.array(selectors_info.selector_indices, dtype=np.uint32)
+        if sel.size != kinds.size:
+            raise ValueError("SelectorsInfo must have one selector index per gate")
+        grp = np.array(selectors_info.groups, dtype=np.uint32).reshape(-1)
+        _check(self.ctx, self.ctx.lib.gl_quotient_add_gates(self.ctx.handle, self._h, _ptr(kinds), _ptr(params), kinds.size, _ptr(sel), _ptr(grp),
+                                                            selectors_info.num_selectors(), num_lookup_selectors, constants_sigmas.merkle_tree._h,
+                                                            num_constants, _ptr(pi), _ptr(a), constraint_offset))
         ms = ctypes.c_float()
         self.ctx.lib.gl_ctx_aux_ms(self.ctx.handle, byref(ms))
         return float(ms.value)

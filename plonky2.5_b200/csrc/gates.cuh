@@ -22,6 +22,8 @@ constexpr int P2_NUM_CONSTRAINTS = 12 * 7 + 22 + 12 + 1 + 4;           // 123
 constexpr int U32_LIMBS = 32, U32_ROUTED = 6;
 constexpr int MAX_CONSTRAINTS = 160, MAX_CHALLENGES = 4;
 
+struct PiHash { uint64_t w[4]; };   // the public-inputs hash (canonical), passed by value in the kernel arguments
+
 __device__ __forceinline__ uint64_t dbl(uint64_t x) { return gl::add(x, x); }
 
 __device__ __forceinline__ uint64_t sbox7(uint64_t x) {
@@ -266,11 +268,53 @@ __device__ __forceinline__ void comparison_gate(Wires&& w, Emit&& emit, uint32_t
     emit(gl::sub(w(2), w(4 + 5 * nc + chunk_bits)));
 }
 
-enum { GATE_POSEIDON2 = 0, GATE_U32_ARITHMETIC = 1, GATE_U32_ADD_MANY = 2, GATE_U32_SUBTRACTION = 3, GATE_U32_RANGE_CHECK = 4,
-       GATE_U32_INTERLEAVE = 5, GATE_UNINTERLEAVE_TO_U32 = 6, GATE_UNINTERLEAVE_TO_B32 = 7, GATE_COMPARISON = 8 };
+// ---- plonky2's core gates (plonky2 @ 3de92d9 gates/{noop,constant,public_input,arithmetic_base,base_sum}.rs · eval_unfiltered, same
+// constraint order).  Upstream source is not in this tree: restated, parity unpinned (oracle/plonky2_gates_oracle.py restates the same
+// items independently).  `k(j)` reads gate constant j (local_constants after remove_prefix), `pi` is the 4-word public-inputs hash.
+// NoopGate has no constraints and is never evaluated.
 
+// ConstantGate: param = num_consts; k(i) - w(i)
+template <class Wires, class Consts, class Emit>
+__device__ __forceinline__ void constant_gate(Wires&& w, Consts&& k, Emit&& emit, uint32_t n) {
+    for (uint32_t i = 0; i < n; i++) emit(gl::sub(k(i), w(i)));
+}
+// PublicInputGate: w(i) - public_inputs_hash[i]
 template <class Wires, class Emit>
-__device__ __forceinline__ void eval_gate(int kind, uint32_t param, Wires&& w, Emit&& emit) {
+__device__ __forceinline__ void public_input_gate(Wires&& w, const uint64_t (&pi)[4], Emit&& emit) {
+#pragma unroll
+    for (int i = 0; i < 4; i++) emit(gl::sub(w(i), pi[i]));
+}
+// ArithmeticGate (base field): param = num_ops; output - (k(0) m0 m1 + k(1) addend), wires [m0, m1, addend, output] per op
+template <class Wires, class Consts, class Emit>
+__device__ __forceinline__ void arithmetic_gate(Wires&& w, Consts&& k, Emit&& emit, uint32_t num_ops) {
+    const uint64_t c0 = k(0), c1 = k(1);
+    for (uint32_t i = 0; i < num_ops; i++) {
+        const uint64_t computed = gl::add(gl::mulc(gl::mulc(w(4 * i), w(4 * i + 1)), c0), gl::mulc(w(4 * i + 2), c1));
+        emit(gl::sub(w(4 * i + 3), computed));
+    }
+}
+// BaseSumGate<B>: param = num_limbs | B << 8; reduce_with_powers(limbs, B) - sum, then prod_{v < B} (limb - v) per limb
+template <class Wires, class Emit>
+__device__ __forceinline__ void base_sum_gate(Wires&& w, Emit&& emit, uint32_t param) {
+    const uint32_t n = param & 0xFF, base = param >> 8;
+    uint64_t sum = 0;
+    for (int j = (int)n - 1; j >= 0; j--) sum = gl::add(gl::mulc(sum, base), w(1 + j));
+    emit(gl::sub(sum, w(0)));
+#pragma unroll 1
+    for (uint32_t j = 0; j < n; j++) {
+        const uint64_t limb = w(1 + j);
+        uint64_t prod = limb;
+        for (uint32_t v = 1; v < base; v++) prod = gl::mulc(prod, gl::sub(limb, v));
+        emit(prod);
+    }
+}
+
+enum { GATE_POSEIDON2 = 0, GATE_U32_ARITHMETIC = 1, GATE_U32_ADD_MANY = 2, GATE_U32_SUBTRACTION = 3, GATE_U32_RANGE_CHECK = 4,
+       GATE_U32_INTERLEAVE = 5, GATE_UNINTERLEAVE_TO_U32 = 6, GATE_UNINTERLEAVE_TO_B32 = 7, GATE_COMPARISON = 8, GATE_NOOP = 9,
+       GATE_CONSTANT = 10, GATE_PUBLIC_INPUT = 11, GATE_ARITHMETIC = 12, GATE_BASE_SUM = 13 };
+
+template <class Wires, class Consts, class Emit>
+__device__ __forceinline__ void eval_gate(int kind, uint32_t param, Wires&& w, Consts&& k, const uint64_t (&pi)[4], Emit&& emit) {
     switch (kind) {
         case GATE_POSEIDON2: poseidon2_gate(w, emit); break;
         case GATE_U32_ARITHMETIC: u32_arithmetic_gate(w, emit, param); break;
@@ -280,28 +324,55 @@ __device__ __forceinline__ void eval_gate(int kind, uint32_t param, Wires&& w, E
         case GATE_U32_INTERLEAVE: interleave_gate(w, emit, param); break;
         case GATE_UNINTERLEAVE_TO_U32: uninterleave_gate<false>(w, emit, param); break;
         case GATE_UNINTERLEAVE_TO_B32: uninterleave_gate<true>(w, emit, param); break;
+        case GATE_CONSTANT: constant_gate(w, k, emit, param); break;
+        case GATE_PUBLIC_INPUT: public_input_gate(w, pi, emit); break;
+        case GATE_ARITHMETIC: arithmetic_gate(w, k, emit, param); break;
+        case GATE_BASE_SUM: base_sum_gate(w, emit, param); break;
+        case GATE_NOOP: break;
         default: comparison_gate(w, emit, param); break;
     }
 }
 
-// every constraint of every row, uncombined (tests): out[row][i]
+// plonky2 gates/selectors.rs · UNUSED_SELECTOR (u32::MAX)
+constexpr uint64_t UNUSED_SELECTOR = 0xFFFFFFFFULL;
+
+// plonky2 gates/gate.rs · compute_filter(i, group, s, many_selectors): prod_{j in [start, end), j != i} (j - s) * (UNUSED_SELECTOR - s if many)
+__device__ __forceinline__ uint64_t selector_filter(uint64_t s, uint32_t i, uint32_t start, uint32_t end, uint32_t many) {
+    uint64_t f = many ? gl::sub(UNUSED_SELECTOR, s) : 1;
+#pragma unroll 1
+    for (uint32_t j = start; j < end; j++)
+        if (j != i) f = gl::mulc(f, gl::sub(j, s));
+    return f;
+}
+
+// every constraint of every row, uncombined (tests): out[row][i]; consts [n_rows][n_consts] (nullptr when the gate reads none)
 __global__ void gate_constraints_kernel(int kind, uint32_t param, const uint64_t* __restrict__ rows, uint32_t pitch, uint64_t n_rows,
-                                        uint32_t n_constraints, uint64_t* __restrict__ out) {
+                                        uint32_t n_constraints, const uint64_t* __restrict__ consts, uint32_t n_consts, const PiHash pi,
+                                        uint64_t* __restrict__ out) {
     const uint64_t row = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (row >= n_rows) return;
     const uint64_t* r = rows + row * pitch;
+    const uint64_t* c = consts + row * n_consts;
     uint64_t* o = out + row * n_constraints;
     uint32_t k = 0;
-    eval_gate(kind, param, [&](int i) { return gl::canon(__ldg(r + i)); }, [&](uint64_t v) { o[k++] = v; });
+    eval_gate(kind, param, [&](int i) { return gl::canon(__ldg(r + i)); }, [&](int i) { return gl::canon(__ldg(c + i)); }, pi.w,
+              [&](uint64_t v) { o[k++] = v; });
 }
+
+enum { FILTER_NONE = 0, FILTER_COLUMN = 1, FILTER_SELECTOR = 2 };
 
 struct QuotientArgs {
     const uint64_t* rows;          // wires: [n_rows][pitch] (the leaf matrix of the wires commit)
-    const uint64_t* filter;        // optional per-row multiplier (column `filter_col` of a [n_rows][filter_pitch] matrix), or nullptr
+    const uint64_t* filter;        // [n_rows][filter_pitch] matrix the filter is read from (FILTER_COLUMN / FILTER_SELECTOR), else nullptr
     uint64_t* acc;                 // [n_challenges][n_rows], += in place
     const uint64_t* powers;        // [n_challenges][n_constraints]: alpha_k^(offset + i), canonical
     uint64_t n_rows;
     uint32_t pitch, filter_pitch, filter_col, n_constraints, n_challenges, kind, param;
+    // FILTER_COLUMN: filter(row) = column filter_col.  FILTER_SELECTOR: `filter` is the constants/sigmas leaf matrix, column filter_col the
+    // gate's selector s, and filter(row) = selector_filter(s, gate_index, group_start, group_end, many_selectors); the gate constants are
+    // its columns [const_col0, ...)
+    uint32_t filter_mode, gate_index, group_start, group_end, many_selectors, const_col0;
+    PiHash pi;
 };
 
 // acc[k][row] += filter(row) * sum_i powers[k][i] * constraint_i(row)
@@ -318,16 +389,20 @@ __global__ void __launch_bounds__(128) gate_quotient_kernel(const QuotientArgs a
     for (int k = 0; k < NCH; k++) acc[k] = 0;
     uint32_t i = 0;
     eval_gate((int)a.kind, a.param, [&](int j) { return gl::canon(__ldg(r + j)); },
+              [&](int j) { return gl::canon(__ldg(a.filter + row * a.filter_pitch + a.const_col0 + j)); }, a.pi.w,
               [&](uint64_t v) {
 #pragma unroll
                   for (int k = 0; k < NCH; k++) acc[k] = gl::add(acc[k], gl::mulc(v, pw[k * a.n_constraints + i]));
                   i++;
               });
     uint64_t f = 1;
-    if (a.filter) f = gl::canon(__ldg(a.filter + row * a.filter_pitch + a.filter_col));
+    if (a.filter_mode != FILTER_NONE) {
+        f = gl::canon(__ldg(a.filter + row * a.filter_pitch + a.filter_col));
+        if (a.filter_mode == FILTER_SELECTOR) f = selector_filter(f, a.gate_index, a.group_start, a.group_end, a.many_selectors);
+    }
 #pragma unroll
     for (int k = 0; k < NCH; k++) {
-        uint64_t v = a.filter ? gl::mulc(acc[k], f) : acc[k];
+        uint64_t v = a.filter_mode != FILTER_NONE ? gl::mulc(acc[k], f) : acc[k];
         uint64_t* dst = a.acc + (uint64_t)k * a.n_rows + row;
         *dst = gl::add(*dst, v);
     }

@@ -2167,6 +2167,11 @@ int gate_wires(int kind, uint32_t param) {
             const uint32_t cb = (lo + hi - 1) / hi;
             return cb <= 6 && 4 + 5 * hi + cb + 1 <= 135 ? (int)(4 + 5 * hi + cb + 1) : -1;
         }
+        case GL_GATE_NOOP: return param == 0 ? 0 : -1;
+        case GL_GATE_CONSTANT: return param >= 1 && param <= 8 ? (int)param : -1;
+        case GL_GATE_PUBLIC_INPUT: return param == 0 ? 4 : -1;
+        case GL_GATE_ARITHMETIC: return param >= 1 && param <= 33 ? (int)(4 * param) : -1;
+        case GL_GATE_BASE_SUM: return lo >= 1 && 1 + lo <= 135 && hi >= 2 && hi <= 16 ? (int)(1 + lo) : -1;
         default: return -1;
     }
 }
@@ -2182,32 +2187,95 @@ int gate_constraints(int kind, uint32_t param) {
         case GL_GATE_U32_INTERLEAVE: return (int)(34 * param);
         case GL_GATE_UNINTERLEAVE_TO_U32:
         case GL_GATE_UNINTERLEAVE_TO_B32: return (int)(67 * param);
-        default: return (int)(2 + 5 * hi + 1 + ((lo + hi - 1) / hi + 1) + 2);
+        case GL_GATE_COMPARISON: return (int)(2 + 5 * hi + 1 + ((lo + hi - 1) / hi + 1) + 2);
+        case GL_GATE_NOOP: return 0;
+        case GL_GATE_CONSTANT: return (int)param;
+        case GL_GATE_PUBLIC_INPUT: return 4;
+        case GL_GATE_ARITHMETIC: return (int)param;
+        default: return (int)(1 + lo);   // GL_GATE_BASE_SUM
+    }
+}
+int gate_constants(int kind, uint32_t param) {
+    if (gate_wires(kind, param) < 0) return -1;
+    switch (kind) {
+        case GL_GATE_CONSTANT: return (int)param;
+        case GL_GATE_ARITHMETIC: return 2;
+        default: return 0;
     }
 }
 void check_gate(int kind, uint32_t param) {
-    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_COMPARISON) GL_THROW(GL_ERR_INVALID, "unknown gate kind %d", kind);
+    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_BASE_SUM) GL_THROW(GL_ERR_INVALID, "unknown gate kind %d", kind);
     if (gate_wires(kind, param) < 0) GL_THROW(GL_ERR_INVALID, "gate kind %d: parameter %u out of range (see include/gl_commit.h)", kind, param);
+}
+// the entry points without gate constants / public-inputs hash refuse the gates that read them
+void check_gate_without_constants(int kind, uint32_t param, const char* entry) {
+    check_gate(kind, param);
+    if (gate_constants(kind, param) > 0 || kind == GL_GATE_PUBLIC_INPUT)
+        GL_THROW(GL_ERR_INVALID, "gate kind %d reads gate constants or the public-inputs hash: use %s", kind, entry);
+}
+
+// gate constraints of host rows on the device: out [n_rows][num_constraints]; consts [n_rows][gate_constants] or NULL when that is 0
+void eval_rows(gl_ctx* c, int kind, uint32_t param, const uint64_t* rows, const uint64_t* consts, const uint64_t* pi_hash, uint64_t n_rows,
+               uint64_t* out) {
+    const uint32_t nw = (uint32_t)gate_wires(kind, param), nc = (uint32_t)gate_constraints(kind, param), nk = (uint32_t)gate_constants(kind, param);
+    if (n_rows == 0 || nc == 0) return;
+    c->scratch.ensure(n_rows * (nw + nk + nc));
+    uint64_t* d_rows = c->scratch.p;
+    uint64_t* d_consts = d_rows + n_rows * nw;
+    uint64_t* d_out = d_consts + n_rows * nk;
+    gates::PiHash pi{};
+    for (int i = 0; i < 4 && pi_hash; i++) pi.w[i] = gl::canon(pi_hash[i]);
+    CUDA_CHECK(cudaMemcpyAsync(d_rows, rows, n_rows * nw * 8, cudaMemcpyHostToDevice, c->stream));
+    if (nk) CUDA_CHECK(cudaMemcpyAsync(d_consts, consts, n_rows * nk * 8, cudaMemcpyHostToDevice, c->stream));
+    gates::gate_constraints_kernel<<<(uint32_t)((n_rows + 127) / 128), 128, 0, c->stream>>>(kind, param, d_rows, nw, n_rows, nc, d_consts, nk, pi,
+                                                                                             d_out);
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaMemcpyAsync(out, d_out, n_rows * nc * 8, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+}
+
+// alpha_k^(offset + i), i < nc, for every challenge: [n_ch][nc] (a few hundred host multiplies per gate)
+void alpha_powers(const uint64_t* alphas, uint32_t n_ch, uint32_t offset, uint32_t nc, uint64_t* out) {
+    for (uint32_t k = 0; k < n_ch; k++) {
+        const uint64_t al = gl::canon(alphas[k]);
+        uint64_t cur = gl::h_pow(al, offset);
+        for (uint32_t i = 0; i < nc; i++) { out[(size_t)k * nc + i] = cur; cur = gl::h_mul(cur, al); }
+    }
+}
+
+void launch_gate_quotient(gl_ctx* c, const gates::QuotientArgs& a) {
+    const uint32_t grid = (uint32_t)((a.n_rows + 127) / 128);
+    const size_t smem = (size_t)a.n_challenges * a.n_constraints * 8;
+    switch (a.n_challenges) {
+        case 1: gates::gate_quotient_kernel<1><<<grid, 128, smem, c->stream>>>(a); break;
+        case 2: gates::gate_quotient_kernel<2><<<grid, 128, smem, c->stream>>>(a); break;
+        case 3: gates::gate_quotient_kernel<3><<<grid, 128, smem, c->stream>>>(a); break;
+        default: gates::gate_quotient_kernel<4><<<grid, 128, smem, c->stream>>>(a); break;
+    }
+    CUDA_CHECK(cudaGetLastError());
 }
 }  // namespace
 
 int gl_gate_num_wires(int kind, uint32_t param) { return gate_wires(kind, param); }
 int gl_gate_num_constraints(int kind, uint32_t param) { return gate_constraints(kind, param); }
+int gl_gate_num_constants(int kind, uint32_t param) { return gate_constants(kind, param); }
 
 int gl_gate_eval_rows(gl_ctx* c, int kind, uint32_t param, const uint64_t* rows, uint64_t n_rows, uint64_t* out) {
     GL_API_BEGIN(c)
-    check_gate(kind, param);
+    check_gate_without_constants(kind, param, "gl_gate_eval_rows_with_constants");
     if ((!rows || !out) && n_rows) GL_THROW(GL_ERR_INVALID, "NULL pointer");
-    if (n_rows == 0) return GL_OK;
-    const uint32_t nw = (uint32_t)gate_wires(kind, param), nc = (uint32_t)gate_constraints(kind, param);
-    c->scratch.ensure(n_rows * (nw + nc));
-    uint64_t* d_rows = c->scratch.p;
-    uint64_t* d_out = d_rows + n_rows * nw;
-    CUDA_CHECK(cudaMemcpyAsync(d_rows, rows, n_rows * nw * 8, cudaMemcpyHostToDevice, c->stream));
-    gates::gate_constraints_kernel<<<(uint32_t)((n_rows + 127) / 128), 128, 0, c->stream>>>(kind, param, d_rows, nw, n_rows, nc, d_out);
-    CUDA_CHECK(cudaGetLastError());
-    CUDA_CHECK(cudaMemcpyAsync(out, d_out, n_rows * nc * 8, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    eval_rows(c, kind, param, rows, nullptr, nullptr, n_rows, out);
+    return GL_OK;
+    GL_API_END(c)
+}
+
+int gl_gate_eval_rows_with_constants(gl_ctx* c, int kind, uint32_t param, const uint64_t* rows, const uint64_t* consts,
+                                     const uint64_t public_inputs_hash[4], uint64_t n_rows, uint64_t* out) {
+    GL_API_BEGIN(c)
+    check_gate(kind, param);
+    if (!public_inputs_hash) GL_THROW(GL_ERR_INVALID, "public_inputs_hash is NULL");
+    if ((!rows || !out || (!consts && gate_constants(kind, param) > 0)) && n_rows) GL_THROW(GL_ERR_INVALID, "NULL pointer");
+    eval_rows(c, kind, param, rows, consts, public_inputs_hash, n_rows, out);
     return GL_OK;
     GL_API_END(c)
 }
@@ -2232,7 +2300,7 @@ int gl_quotient_add_gate(gl_ctx* c, gl_handle qh, int kind, uint32_t param, cons
                          gl_handle filter_batch, uint32_t filter_col) {
     GL_API_BEGIN(c)
     Quotient* q = c->quotients.get(qh);
-    check_gate(kind, param);
+    check_gate_without_constants(kind, param, "gl_quotient_add_gates");
     if (!alphas) GL_THROW(GL_ERR_INVALID, "alphas is NULL");
     Tree* t = c->trees.get(q->wires);
     const uint32_t nw = (uint32_t)gate_wires(kind, param), nc = (uint32_t)gate_constraints(kind, param);
@@ -2245,28 +2313,84 @@ int gl_quotient_add_gate(gl_ctx* c, gl_handle qh, int kind, uint32_t param, cons
         Tree* f = c->trees.get(filter_batch);
         if (f->n_leaves != q->n_rows) GL_THROW(GL_ERR_INVALID, "filter batch has %llu rows, the wires batch %llu", (unsigned long long)f->n_leaves, (unsigned long long)q->n_rows);
         if (filter_col >= f->leaf_len) GL_THROW(GL_ERR_INVALID, "filter column %u out of range", filter_col);
-        a.filter = f->leaves.p; a.filter_pitch = f->pitch; a.filter_col = filter_col;
+        a.filter = f->leaves.p; a.filter_pitch = f->pitch; a.filter_col = filter_col; a.filter_mode = gates::FILTER_COLUMN;
     }
-    // alpha_k^(offset + i): a few hundred host multiplies per call
+    c->aux_ms = 0;
+    if (nc == 0) return GL_OK;   // NoopGate
     std::vector<uint64_t> pw((size_t)q->n_challenges * nc);
-    for (uint32_t k = 0; k < q->n_challenges; k++) {
-        const uint64_t al = gl::canon(alphas[k]);
-        uint64_t cur = gl::h_pow(al, constraint_offset);
-        for (uint32_t i = 0; i < nc; i++) { pw[(size_t)k * nc + i] = cur; cur = gl::h_mul(cur, al); }
-    }
+    alpha_powers(alphas, q->n_challenges, constraint_offset, nc, pw.data());
     CUDA_CHECK(cudaMemcpyAsync(q->powers.p, pw.data(), pw.size() * 8, cudaMemcpyHostToDevice, c->stream));
-    const uint32_t grid = (uint32_t)((q->n_rows + 127) / 128);
-    const size_t smem = pw.size() * 8;
     CUDA_CHECK(cudaEventRecord(c->ev[0], c->stream));
-    switch (q->n_challenges) {
-        case 1: gates::gate_quotient_kernel<1><<<grid, 128, smem, c->stream>>>(a); break;
-        case 2: gates::gate_quotient_kernel<2><<<grid, 128, smem, c->stream>>>(a); break;
-        case 3: gates::gate_quotient_kernel<3><<<grid, 128, smem, c->stream>>>(a); break;
-        default: gates::gate_quotient_kernel<4><<<grid, 128, smem, c->stream>>>(a); break;
-    }
-    CUDA_CHECK(cudaGetLastError());
+    launch_gate_quotient(c, a);
     CUDA_CHECK(cudaEventRecord(c->ev[1], c->stream));
     CUDA_CHECK(cudaStreamSynchronize(c->stream));   // pw is a host vector of this call
+    CUDA_CHECK(cudaEventElapsedTime(&c->aux_ms, c->ev[0], c->ev[1]));
+    return GL_OK;
+    GL_API_END(c)
+}
+
+int gl_quotient_add_gates(gl_ctx* c, gl_handle qh, const int* kinds, const uint32_t* params, uint32_t n_gates, const uint32_t* selector_indices,
+                          const uint32_t* groups, uint32_t num_selectors, uint32_t num_lookup_selectors, gl_handle constants_sigmas,
+                          uint32_t num_constants, const uint64_t public_inputs_hash[4], const uint64_t* alphas, uint32_t constraint_offset) {
+    GL_API_BEGIN(c)
+    Quotient* q = c->quotients.get(qh);
+    if (!kinds || !params || !selector_indices || !groups || !public_inputs_hash || !alphas) GL_THROW(GL_ERR_INVALID, "NULL pointer");
+    if (n_gates == 0) GL_THROW(GL_ERR_INVALID, "No gates?");
+    Tree* tw = c->trees.get(q->wires);
+    Tree* tc = c->trees.get(constants_sigmas);
+    if (tc->n_leaves != tw->n_leaves || tc->degree_log != tw->degree_log || tc->rate_bits != tw->rate_bits)
+        GL_THROW(GL_ERR_INVALID, "Polynomial degrees inconsistent (the constants/sigmas batch must share the wires batch's rows, degree and rate_bits)");
+    if (num_constants > tc->leaf_len) GL_THROW(GL_ERR_INVALID, "num_constants %u exceeds the constants/sigmas batch's %u columns", num_constants, tc->leaf_len);
+    const uint32_t const_col0 = num_selectors + num_lookup_selectors;
+    // every gate is checked before the first launch: a refused call leaves the accumulator as it was
+    uint32_t max_nc = 0;
+    for (uint32_t i = 0; i < n_gates; i++) {
+        check_gate(kinds[i], params[i]);
+        const uint32_t nw = (uint32_t)gate_wires(kinds[i], params[i]), nc = (uint32_t)gate_constraints(kinds[i], params[i]);
+        const uint32_t s = selector_indices[i];
+        if (s >= num_selectors) GL_THROW(GL_ERR_INVALID, "gate %u: selector index %u >= num_selectors %u", i, s, num_selectors);
+        if (groups[2 * s] > groups[2 * s + 1] || groups[2 * s + 1] > n_gates)
+            GL_THROW(GL_ERR_INVALID, "selector group %u = [%u, %u) is not a range of the %u gates", s, groups[2 * s], groups[2 * s + 1], n_gates);
+        if (i < groups[2 * s] || i >= groups[2 * s + 1])
+            GL_THROW(GL_ERR_INVALID, "gate %u is outside its selector group %u = [%u, %u)", i, s, groups[2 * s], groups[2 * s + 1]);
+        if (const_col0 + (uint32_t)gate_constants(kinds[i], params[i]) > num_constants)
+            GL_THROW(GL_ERR_INVALID, "gate %u: %u selector columns + %u gate constants exceed num_constants %u", i, const_col0,
+                     (uint32_t)gate_constants(kinds[i], params[i]), num_constants);
+        if (tw->leaf_len < nw) GL_THROW(GL_ERR_INVALID, "gate %u: the wires batch has %u columns, the gate needs %u", i, tw->leaf_len, nw);
+        if (nc > (uint32_t)gates::MAX_CONSTRAINTS) GL_THROW(GL_ERR_UNSUPPORTED, "gate %u: too many constraints", i);
+        max_nc = std::max(max_nc, nc);
+    }
+    const uint32_t n_ch = q->n_challenges;
+    c->aux_ms = 0;
+    if (max_nc == 0) return GL_OK;   // only NoopGates
+    // every gate's constraints start at alpha^offset (evaluate_gate_constraints_base_batch sums them into one constraint vector)
+    std::vector<uint64_t> pw((size_t)n_ch * max_nc);
+    alpha_powers(alphas, n_ch, constraint_offset, max_nc, pw.data());
+    gates::QuotientArgs a{};
+    a.rows = tw->leaves.p; a.pitch = tw->pitch; a.n_rows = q->n_rows; a.acc = q->acc.p; a.n_challenges = n_ch;
+    a.filter = tc->leaves.p; a.filter_pitch = tc->pitch; a.filter_mode = gates::FILTER_SELECTOR;
+    a.many_selectors = num_selectors > 1; a.const_col0 = const_col0;
+    for (int j = 0; j < 4; j++) a.pi.w[j] = gl::canon(public_inputs_hash[j]);
+    // one [n_ch][nc] table per gate (the kernel reads its table with row stride nc), uploaded in one copy
+    std::vector<uint64_t> host;
+    std::vector<size_t> table_at(n_gates);
+    for (uint32_t i = 0; i < n_gates; i++) {
+        const uint32_t nc = (uint32_t)gate_constraints(kinds[i], params[i]);
+        table_at[i] = host.size();
+        for (uint32_t k = 0; k < n_ch; k++) host.insert(host.end(), pw.begin() + (size_t)k * max_nc, pw.begin() + (size_t)k * max_nc + nc);
+    }
+    c->scratch.ensure(host.size());
+    CUDA_CHECK(cudaMemcpyAsync(c->scratch.p, host.data(), host.size() * 8, cudaMemcpyHostToDevice, c->stream));
+    CUDA_CHECK(cudaEventRecord(c->ev[0], c->stream));
+    for (uint32_t i = 0; i < n_gates; i++) {
+        const uint32_t nc = (uint32_t)gate_constraints(kinds[i], params[i]), s = selector_indices[i];
+        if (nc == 0) continue;   // NoopGate
+        a.kind = (uint32_t)kinds[i]; a.param = params[i]; a.n_constraints = nc; a.powers = c->scratch.p + table_at[i];
+        a.gate_index = i; a.filter_col = s; a.group_start = groups[2 * s]; a.group_end = groups[2 * s + 1];
+        launch_gate_quotient(c, a);
+    }
+    CUDA_CHECK(cudaEventRecord(c->ev[1], c->stream));
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));   // `host` is a vector of this call
     CUDA_CHECK(cudaEventElapsedTime(&c->aux_ms, c->ev[0], c->ev[1]));
     return GL_OK;
     GL_API_END(c)

@@ -467,6 +467,19 @@ impl Drop for Openings<'_> {
     }
 }
 
+/// `gates/selectors.rs · SelectorsInfo`: gate i is filtered by selector column `selector_indices[i]`, whose gate range is
+/// `groups[selector_indices[i]]`
+pub struct SelectorsInfo {
+    pub selector_indices: Vec<usize>,
+    pub groups: Vec<std::ops::Range<usize>>,
+}
+
+impl SelectorsInfo {
+    pub fn num_selectors(&self) -> usize {
+        self.groups.len()
+    }
+}
+
 /// Pinned host memory for outputs that must be materialised on the host (INTEGRATION.md "Host memory for copy-back")
 /// accumulator of `sum_i alpha_k^(offset + i) * constraint_i` over every LDE row of a wires commit (`gl_quotient_*`)
 pub struct Quotient<'c> {
@@ -480,6 +493,25 @@ impl<'c> Quotient<'c> {
         assert_eq!(alphas.len(), self.num_challenges, "one alpha per challenge");
         let (fb, fc) = filter.map(|(t, c)| (t.handle, c as u32)).unwrap_or((0, 0));
         self.ctx.check(unsafe { ffi::gl_quotient_add_gate(self.ctx.raw, self.handle, kind as c_int, param, alphas.as_ptr(), constraint_offset as u32, fb, fc) })
+    }
+
+    /// `plonk/vanishing_poly.rs · evaluate_gate_constraints_base_batch` over the LDE rows: `gates[i] = (kind, param)` of
+    /// `CommonCircuitData::gates`, `selectors_info` its `SelectorsInfo`; each gate's constraints times `compute_filter` of its selector
+    /// column in `constants_sigmas` (commit #0), constants read from the columns after the selectors
+    #[allow(clippy::too_many_arguments)]
+    pub fn add_gates(&mut self, gates: &[(i32, u32)], selectors_info: &SelectorsInfo, num_lookup_selectors: usize, constants_sigmas: &DeviceTree<'c>,
+                     num_constants: usize, public_inputs_hash: &[u64; 4], alphas: &[u64], constraint_offset: usize) -> Result<(), Error> {
+        assert_eq!(alphas.len(), self.num_challenges, "one alpha per challenge");
+        assert_eq!(selectors_info.selector_indices.len(), gates.len(), "one selector index per gate");
+        let kinds: Vec<c_int> = gates.iter().map(|g| g.0 as c_int).collect();
+        let params: Vec<u32> = gates.iter().map(|g| g.1).collect();
+        let sel: Vec<u32> = selectors_info.selector_indices.iter().map(|&i| i as u32).collect();
+        let groups: Vec<u32> = selectors_info.groups.iter().flat_map(|r| [r.start as u32, r.end as u32]).collect();
+        self.ctx.check(unsafe {
+            ffi::gl_quotient_add_gates(self.ctx.raw, self.handle, kinds.as_ptr(), params.as_ptr(), gates.len() as u32, sel.as_ptr(), groups.as_ptr(),
+                                       selectors_info.num_selectors() as u32, num_lookup_selectors as u32, constants_sigmas.handle,
+                                       num_constants as u32, public_inputs_hash.as_ptr(), alphas.as_ptr(), constraint_offset as u32)
+        })
     }
 
     /// the permutation-argument terms of `eval_vanishing_poly_base_batch` (`vanishing_terms[0 .. n_ch * (1 + n_chunks))`)
