@@ -184,14 +184,24 @@ int gl_fri_read(gl_ctx* ctx, gl_handle fri, uint64_t* out_coeffs_ext, uint64_t* 
  *   GL_GATE_PUBLIC_INPUT    PublicInputGate                    param 0                                  4 wires, 4 constraints, 0 constants
  *   GL_GATE_ARITHMETIC      ArithmeticGate (base)              param = num_ops (1..33; 20 at 80 routed)  4*n wires, n constraints, 2 constants
  *   GL_GATE_BASE_SUM        BaseSumGate<B>                     param = num_limbs | B << 8 (B 2..16)      1+n wires, 1+n constraints, 0 constants
+ * and three more base-field gates of plonky2 @ 3de92d9 (gates/{poseidon,exponentiation,random_access}.rs; restated, parity unpinned):
+ *   GL_GATE_POSEIDON        PoseidonGate                       param 0                                  135 wires, 123 constraints, 0 constants
+ *                           (Poseidon2Gate's wire layout; the permutation is the leaf hash's plonky2 Poseidon)
+ *   GL_GATE_EXPONENTIATION  ExponentiationGate                 param = num_power_bits (1..66; 66 at 135 wires / 80 routed)
+ *                                                              2+2n wires, n+1 constraints, 0 constants
+ *   GL_GATE_RANDOM_ACCESS   RandomAccessGate                   param = bits | num_copies << 8 | num_extra_constants << 16
+ *                           (bits 1..6, v = 2^bits, (2+v+bits)*num_copies + num_extra_constants <= 135 wires)
+ *                                                              (bits+2)*num_copies + num_extra_constants constraints, num_extra_constants constants
+ * Kind 14 is not assigned: it stays an unknown kind, as it was before these three gates existed.
  * gl_quotient_add_gate:  acc[k][row] += filter(row) * sum_i alphas[k]^(constraint_offset + i) * constraint_i(wires(row)),  k < n_challenges
  * (alphas are BASE-field challenges, as upstream; filter(row) = column filter_col of the batch filter_batch at the same row, or 1 when
  * filter_batch == 0).  gl_quotient_read: [n_challenges][R] words, row order = the leaves' (bit-reversed).
  * gl_gate_eval_rows and gl_quotient_add_gate refuse the gates that read gate constants or the public-inputs hash (CONSTANT, ARITHMETIC,
- * PUBLIC_INPUT): those go through gl_gate_eval_rows_with_constants and gl_quotient_add_gates.                                             */
+ * PUBLIC_INPUT, and RANDOM_ACCESS with extra constants): those go through gl_gate_eval_rows_with_constants and gl_quotient_add_gates. */
 enum { GL_GATE_POSEIDON2 = 0, GL_GATE_U32_ARITHMETIC = 1, GL_GATE_U32_ADD_MANY = 2, GL_GATE_U32_SUBTRACTION = 3, GL_GATE_U32_RANGE_CHECK = 4,
        GL_GATE_U32_INTERLEAVE = 5, GL_GATE_UNINTERLEAVE_TO_U32 = 6, GL_GATE_UNINTERLEAVE_TO_B32 = 7, GL_GATE_COMPARISON = 8, GL_GATE_NOOP = 9,
-       GL_GATE_CONSTANT = 10, GL_GATE_PUBLIC_INPUT = 11, GL_GATE_ARITHMETIC = 12, GL_GATE_BASE_SUM = 13 };
+       GL_GATE_CONSTANT = 10, GL_GATE_PUBLIC_INPUT = 11, GL_GATE_ARITHMETIC = 12, GL_GATE_BASE_SUM = 13, GL_GATE_POSEIDON = 15,
+       GL_GATE_EXPONENTIATION = 16, GL_GATE_RANDOM_ACCESS = 17 };
 int gl_gate_num_wires(int kind, uint32_t param);
 int gl_gate_num_constraints(int kind, uint32_t param);
 /* Gate::num_constants: the gate constants a gate reads (-1 for a bad kind or parameter) */
@@ -232,12 +242,15 @@ int gl_quotient_read(gl_ctx* ctx, gl_handle quotient, uint64_t* out);
  * out_batch: the committed batch (coefficients, leaves, digests resident), as from gl_commit.  Restated from upstream (parity unpinned).  */
 int gl_quotient_commit(gl_ctx* ctx, gl_handle quotient, uint32_t cap_height, uint64_t* out_cap, gl_handle* out_batch);
 int gl_quotient_end(gl_ctx* ctx, gl_handle quotient);
-/* CUDA-event milliseconds of the last gl_quotient_add_gate / gl_poseidon2_gate_witness kernel on this context (gl_quotient_add_gates:
+/* CUDA-event milliseconds of the last gl_quotient_add_gate / gl_poseidon2_gate_witness / gl_poseidon_gate_witness kernel on this context (gl_quotient_add_gates:
  * from its first launch to its last; 0 when it launched nothing) */
 int gl_ctx_aux_ms(gl_ctx* ctx, float* out_ms);
 /* witness generation for Poseidon2Gate rows (poseidon2_gate.rs:447-523 · Poseidon2Generator::run_once): inputs [n][13] = the 12 state
  * inputs + the swap flag of each row -> out_rows [n][135], every wire of the row (deltas, S-box inputs of all rounds, outputs)        */
 int gl_poseidon2_gate_witness(gl_ctx* ctx, const uint64_t* inputs, uint64_t n, uint64_t* out_rows);
+/* witness generation for plonky2's PoseidonGate rows (gates/poseidon.rs · PoseidonGenerator::run_once; restated, parity unpinned): the
+ * same shape as gl_poseidon2_gate_witness — inputs [n][13] -> out_rows [n][135], every wire written, canonical; swap applied when it is 1 */
+int gl_poseidon_gate_witness(gl_ctx* ctx, const uint64_t* inputs, uint64_t n, uint64_t* out_rows);
 
 /* ---- permutation argument: partial products and Z (SURVEY §8f rank 4) --------------------------------------------------------
  * plonky2 plonk/prover.rs · all_wires_permutation_partial_products (+ the "Z first" reordering prove() applies before committing):

@@ -734,7 +734,8 @@ struct OpeningSet {
 
 /* ------------------------------------------------------------------------------------------------ quotient / permutation / witness */
 /* SURVEY §8(f) ranks 3-4.  Gate kinds are include/gl_commit.h's GL_GATE_* (the reference's own gates: Poseidon2Gate and the eight
- * u32 / b32 gates under /root/reference/src/common/u32/gates/). */
+ * u32 / b32 gates under /root/reference/src/common/u32/gates/; plonky2's Noop, Constant, PublicInput, Arithmetic, BaseSum, Poseidon,
+ * Exponentiation and RandomAccess gates). */
 
 /* Gate::eval_unfiltered_base_batch on host rows: rows = n x num_wires words -> n x num_constraints constraint values */
 inline std::vector<F> evaluate_gate_constraints(int kind, uint32_t param, const std::vector<F>& rows, Context* ctx = nullptr) {
@@ -828,6 +829,16 @@ inline std::vector<F> poseidon2_gate_witness(const std::vector<F>& inputs, Conte
     const size_t n = inputs.size() / 13;
     std::vector<F> out(n * 135);
     c.check(gl_poseidon2_gate_witness(c.raw(), inputs.data(), n, out.data()));
+    return out;
+}
+
+/* plonky2 gates/poseidon.rs · PoseidonGenerator::run_once for n PoseidonGate rows: inputs n x 13 -> n x 135 */
+inline std::vector<F> poseidon_gate_witness(const std::vector<F>& inputs, Context* ctx = nullptr) {
+    Context& c = ctx_or_default(ctx);
+    if (inputs.size() % 13) throw Panic("poseidon_gate_witness: inputs must be n * 13 words (12 state inputs + swap)");
+    const size_t n = inputs.size() / 13;
+    std::vector<F> out(n * 135);
+    c.check(gl_poseidon_gate_witness(c.raw(), inputs.data(), n, out.data()));
     return out;
 }
 

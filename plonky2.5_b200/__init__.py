@@ -13,6 +13,7 @@ from .api import (GATE_COMPARISON, GATE_POSEIDON2, GATE_U32_ADD_MANY, GATE_U32_A
                   GATE_U32_SUBTRACTION, GATE_UNINTERLEAVE_TO_B32, GATE_UNINTERLEAVE_TO_U32, Quotient, evaluate_gate_constraints, gate_shape,
                   partial_products_and_zs, poseidon2_gate_witness)
 from .api import GATE_ARITHMETIC, GATE_BASE_SUM, GATE_CONSTANT, GATE_NOOP, GATE_PUBLIC_INPUT, SelectorsInfo  # noqa: F401
+from .api import GATE_EXPONENTIATION, GATE_POSEIDON, GATE_RANDOM_ACCESS, poseidon_gate_witness, random_access_params  # noqa: F401
 from .build import build  # noqa: F401
 
 __all__ = ["Challenger", "Context", "FriBatchInfo", "FriOpeningBatch", "FriOpenings", "FriParams", "FriProofHead", "GlError", "MerkleCap",

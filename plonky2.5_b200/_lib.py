@@ -78,6 +78,7 @@ SIGNATURES = {
     "gl_quotient_end": (c_int, [c_void_p, c_uint64]),
     "gl_ctx_aux_ms": (c_int, [c_void_p, POINTER(c_float)]),
     "gl_poseidon2_gate_witness": (c_int, [c_void_p, c_void_p, c_uint64, c_void_p]),
+    "gl_poseidon_gate_witness": (c_int, [c_void_p, c_void_p, c_uint64, c_void_p]),
     "gl_partial_products": (c_int, [c_void_p, POINTER(c_void_p), POINTER(c_void_p), c_uint32, c_uint32, c_void_p, c_void_p, c_void_p, c_uint32,
                                     c_uint32, c_void_p]),
     "gl_fri_pow": (c_int, [c_void_p, c_void_p, c_void_p, c_uint32, c_uint32, POINTER(c_uint64)]),

@@ -608,6 +608,17 @@ GATE_POSEIDON2, GATE_U32_ARITHMETIC, GATE_U32_ADD_MANY, GATE_U32_SUBTRACTION, GA
 GATE_U32_INTERLEAVE, GATE_UNINTERLEAVE_TO_U32, GATE_UNINTERLEAVE_TO_B32, GATE_COMPARISON = 5, 6, 7, 8
 # plonky2's core gates: NoopGate, ConstantGate { num_consts }, PublicInputGate, ArithmeticGate { num_ops }, BaseSumGate<B> (num_limbs | B << 8)
 GATE_NOOP, GATE_CONSTANT, GATE_PUBLIC_INPUT, GATE_ARITHMETIC, GATE_BASE_SUM = 9, 10, 11, 12, 13
+# PoseidonGate (param 0), ExponentiationGate { num_power_bits }, RandomAccessGate (bits | num_copies << 8 | num_extra_constants << 16)
+GATE_POSEIDON, GATE_EXPONENTIATION, GATE_RANDOM_ACCESS = 15, 16, 17
+
+
+def random_access_params(bits: int, num_wires: int = 135, num_routed: int = 80, num_constants: int = 2) -> int:
+    """plonky2 gates/random_access.rs · RandomAccessGate::new_from_config as a GATE_RANDOM_ACCESS param: as many copies as the routed
+    and total wires allow, and the routed wires left over (at most num_constants) as extra constants"""
+    v = 1 << bits
+    copies = min(num_routed // (2 + v), num_wires // (2 + v + bits))
+    extras = min(num_routed - (2 + v) * copies, num_constants)
+    return bits | copies << 8 | extras << 16
 
 
 def gate_shape(kind: int, param: int = 0) -> Tuple[int, int]:
@@ -746,6 +757,18 @@ class Quotient:
             self.free()
         except Exception:
             pass
+
+
+def poseidon_gate_witness(inputs, ctx: Optional[Context] = None) -> np.ndarray:
+    """plonky2 gates/poseidon.rs · PoseidonGenerator::run_once for a batch of PoseidonGate rows: inputs [n][13] = 12 state inputs + swap
+    flag -> [n][135] wires (the shape of poseidon2_gate_witness)"""
+    ctx = ctx or default_context()
+    x = np.ascontiguousarray(inputs, dtype=np.uint64)
+    if x.ndim != 2 or x.shape[1] != 13:
+        raise ValueError("inputs must be [n][13]")
+    out = np.zeros((x.shape[0], 135), dtype=np.uint64)
+    _check(ctx, ctx.lib.gl_poseidon_gate_witness(ctx.handle, _ptr(x), x.shape[0], _ptr(out)))
+    return out
 
 
 def partial_products_and_zs(wire_cols, sigma_cols, k_is, betas, gammas, degree: int, ctx: Optional[Context] = None) -> np.ndarray:

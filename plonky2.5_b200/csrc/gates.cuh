@@ -12,6 +12,7 @@
 #pragma once
 #include "gl_field.cuh"
 #include "poseidon2_constants.cuh"
+#include "poseidon_constants.cuh"
 
 namespace gates {
 
@@ -309,10 +310,140 @@ __device__ __forceinline__ void base_sum_gate(Wires&& w, Emit&& emit, uint32_t p
     }
 }
 
+// ---- three more base-field gates of plonky2 @ 3de92d9 (gates/{poseidon,exponentiation,random_access}.rs · eval_unfiltered, same
+// constraint order).  Upstream source is not in this tree: restated, parity unpinned (tests/plonky2_std_gates_oracle.py restates them too).
+
+// plonky2 Poseidon::mds_layer: out[r] = sum_i CIRC[i] s[(i + r) % 12] + DIAG[r] s[r] (hash/poseidon_goldilocks.rs MDS_MATRIX_CIRC /
+// MDS_MATRIX_DIAG, DIAG = 8 at r = 0 only).  The coefficients are small (sum 264 < 2^9), so the 32-bit halves of the canonical inputs
+// are accumulated apart (each sum < 2^41, one IMAD.WIDE.U32 per term) and every lane is reduced once.
+__device__ __forceinline__ void poseidon_mds(uint64_t (&s)[P2_WIDTH]) {
+    constexpr uint32_t CIRC[P2_WIDTH] = {17, 15, 41, 16, 2, 28, 13, 13, 39, 18, 34, 20};
+    uint32_t lo[P2_WIDTH], hi[P2_WIDTH];
+#pragma unroll
+    for (int i = 0; i < P2_WIDTH; i++) { lo[i] = (uint32_t)s[i]; hi[i] = (uint32_t)(s[i] >> 32); }
+#pragma unroll
+    for (int r = 0; r < P2_WIDTH; r++) {
+        uint64_t L = 0, H = 0;
+#pragma unroll
+        for (int i = 0; i < P2_WIDTH; i++) {
+            const uint32_t c = CIRC[i] + (r == 0 && i == 0 ? 8 : 0);
+            L += (uint64_t)lo[(i + r) % P2_WIDTH] * c;
+            H += (uint64_t)hi[(i + r) % P2_WIDTH] * c;
+        }
+        const uint64_t x = L + (H << 32);                               // L + H 2^32 < 2^74 as (H >> 32 + carry : x)
+        s[r] = gl::canon(gl::reduce128(x, (H >> 32) + (x < L)));
+    }
+}
+
+// plonky2 Poseidon::poseidon in the naive form (full_rounds / partial_rounds_naive, ALL_ROUND_CONSTANTS) from the state after the swap.
+// `at(wire, v)` gets every S-box input PoseidonGate stores (the wire that holds it, the value computed from the state) and returns the
+// value the S-box takes: the constraint stream emits v - wire and continues from the wire, the witness generator writes v.  The
+// upstream gate writes the partial rounds in the "fast" form; it yields the same lane-0 S-box inputs, so the same constraints
+// (DESIGN.md §3.4).
+template <class At>
+__device__ __forceinline__ void poseidon_rounds(uint64_t (&s)[P2_WIDTH], At&& at) {
+#pragma unroll 1
+    for (int r = 0; r < 4; r++) {
+#pragma unroll
+        for (int i = 0; i < P2_WIDTH; i++) {
+            uint64_t v = gl::add(s[i], POSEIDON_RC[P2_WIDTH * r + i]);
+            if (r != 0) v = at(P2_START_RF_BEGIN + P2_WIDTH * (r - 1) + i, v);
+            s[i] = sbox7(v);
+        }
+        poseidon_mds(s);
+    }
+#pragma unroll 1
+    for (int r = 0; r < P2_RP; r++) {
+#pragma unroll
+        for (int i = 0; i < P2_WIDTH; i++) s[i] = gl::add(s[i], POSEIDON_RC[P2_WIDTH * (4 + r) + i]);
+        s[0] = sbox7(at(P2_START_PARTIAL + r, s[0]));
+        poseidon_mds(s);
+    }
+#pragma unroll 1
+    for (int r = 0; r < 4; r++) {
+#pragma unroll
+        for (int i = 0; i < P2_WIDTH; i++)
+            s[i] = sbox7(at(P2_START_RF_END + P2_WIDTH * r + i, gl::add(s[i], POSEIDON_RC[P2_WIDTH * (26 + r) + i])));
+        poseidon_mds(s);
+    }
+}
+
+// PoseidonGate (gates/poseidon.rs): Poseidon2Gate's wire layout and constraint order — swap binary, 4 deltas, the S-box inputs of full
+// rounds 1..3, of the 22 partial rounds and of the 4 second-half full rounds, then the 12 outputs (123 constraints, degree 7)
+template <class Wires, class Emit>
+__device__ __forceinline__ void poseidon_gate(Wires&& w, Emit&& emit) {
+    const uint64_t swap = w(P2_WIRE_SWAP);
+    emit(gl::mulc(swap, gl::sub(swap, 1)));
+    uint64_t s[P2_WIDTH];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const uint64_t lhs = w(i), rhs = w(i + 4), d = w(P2_START_DELTA + i);
+        emit(gl::sub(gl::mulc(swap, gl::sub(rhs, lhs)), d));
+        s[i] = gl::add(lhs, d);
+        s[i + 4] = gl::sub(rhs, d);
+    }
+#pragma unroll
+    for (int i = 8; i < P2_WIDTH; i++) s[i] = w(i);
+    poseidon_rounds(s, [&](int wire, uint64_t v) {
+        const uint64_t in = w(wire);
+        emit(gl::sub(v, in));
+        return in;
+    });
+#pragma unroll
+    for (int i = 0; i < P2_WIDTH; i++) emit(gl::sub(s[i], w(P2_WIDTH + i)));
+}
+
+// ExponentiationGate (gates/exponentiation.rs): param = num_power_bits n; wires base 0, bits 1..n (little-endian), output 1+n,
+// intermediates 2+n..1+2n.  For i < n, with prev = 1 (i = 0) or intermediate[i-1]^2 and b = bits[n-1-i]:
+// prev (b base + 1 - b) - intermediate[i]; then output - intermediate[n-1]
+template <class Wires, class Emit>
+__device__ __forceinline__ void exponentiation_gate(Wires&& w, Emit&& emit, uint32_t n) {
+    const uint64_t base = w(0);
+    uint64_t prev = 1;
+#pragma unroll 1
+    for (uint32_t i = 0; i < n; i++) {
+        const uint64_t b = w(n - i), inter = w(2 + n + i);
+        emit(gl::sub(gl::mulc(prev, gl::add(gl::mulc(b, base), gl::sub(1, b))), inter));
+        prev = gl::canon(gl::sqr(inter));
+    }
+    emit(gl::sub(w(1 + n), w(1 + 2 * n)));
+}
+
+// RandomAccessGate (gates/random_access.rs): param = bits | num_copies << 8 | num_extra_constants << 16, v = 2^bits.  Copy c: index at
+// (2+v)c, claimed element (2+v)c+1, list (2+v)c+2+i; extra constant i at (2+v) num_copies + i; bit i of copy c at num_routed + c bits + i.
+// Per copy: b(b-1) per bit, sum b_i 2^i - index, folded - claimed; then k(i) - extra_i.  The pairwise fold x + b(y - x) over the bits in
+// order is the multilinear sum_i x_i prod_j (bit j of i ? b_j : 1 - b_j), evaluated term by term (exact field identity, no list buffer).
+template <class Wires, class Consts, class Emit>
+__device__ __forceinline__ void random_access_gate(Wires&& w, Consts&& k, Emit&& emit, uint32_t param) {
+    const uint32_t bits = param & 0xFF, copies = (param >> 8) & 0xFF, extras = param >> 16, v = 1u << bits;
+    const uint32_t extra0 = (2 + v) * copies, routed = extra0 + extras;
+    for (uint32_t c = 0; c < copies; c++) {
+        const uint32_t b0 = routed + c * bits, l0 = (2 + v) * c;
+        uint64_t idx = 0;
+        for (uint32_t j = 0; j < bits; j++) emit(range2(w(b0 + j)));
+        for (int j = (int)bits - 1; j >= 0; j--) idx = gl::add(dbl(idx), w(b0 + j));
+        emit(gl::sub(idx, w(l0)));
+        uint64_t folded = 0;
+#pragma unroll 1
+        for (uint32_t i = 0; i < v; i++) {
+            uint64_t t = w(l0 + 2 + i);
+            for (uint32_t j = 0; j < bits; j++) {
+                const uint64_t b = w(b0 + j);
+                t = gl::mulc(t, (i >> j) & 1 ? b : gl::sub(1, b));
+            }
+            folded = gl::add(folded, t);
+        }
+        emit(gl::sub(folded, w(l0 + 1)));
+    }
+    for (uint32_t i = 0; i < extras; i++) emit(gl::sub(k(i), w(extra0 + i)));
+}
+
 enum { GATE_POSEIDON2 = 0, GATE_U32_ARITHMETIC = 1, GATE_U32_ADD_MANY = 2, GATE_U32_SUBTRACTION = 3, GATE_U32_RANGE_CHECK = 4,
        GATE_U32_INTERLEAVE = 5, GATE_UNINTERLEAVE_TO_U32 = 6, GATE_UNINTERLEAVE_TO_B32 = 7, GATE_COMPARISON = 8, GATE_NOOP = 9,
-       GATE_CONSTANT = 10, GATE_PUBLIC_INPUT = 11, GATE_ARITHMETIC = 12, GATE_BASE_SUM = 13 };
+       GATE_CONSTANT = 10, GATE_PUBLIC_INPUT = 11, GATE_ARITHMETIC = 12, GATE_BASE_SUM = 13, GATE_POSEIDON = 15, GATE_EXPONENTIATION = 16,
+       GATE_RANDOM_ACCESS = 17 };
 
+// every kind but GATE_POSEIDON, which has kernel instances of its own (inlined here it would raise the register count of every gate)
 template <class Wires, class Consts, class Emit>
 __device__ __forceinline__ void eval_gate(int kind, uint32_t param, Wires&& w, Consts&& k, const uint64_t (&pi)[4], Emit&& emit) {
     switch (kind) {
@@ -328,6 +459,8 @@ __device__ __forceinline__ void eval_gate(int kind, uint32_t param, Wires&& w, C
         case GATE_PUBLIC_INPUT: public_input_gate(w, pi, emit); break;
         case GATE_ARITHMETIC: arithmetic_gate(w, k, emit, param); break;
         case GATE_BASE_SUM: base_sum_gate(w, emit, param); break;
+        case GATE_EXPONENTIATION: exponentiation_gate(w, emit, param); break;
+        case GATE_RANDOM_ACCESS: random_access_gate(w, k, emit, param); break;
         case GATE_NOOP: break;
         default: comparison_gate(w, emit, param); break;
     }
@@ -355,8 +488,10 @@ __global__ void gate_constraints_kernel(int kind, uint32_t param, const uint64_t
     const uint64_t* c = consts + row * n_consts;
     uint64_t* o = out + row * n_constraints;
     uint32_t k = 0;
-    eval_gate(kind, param, [&](int i) { return gl::canon(__ldg(r + i)); }, [&](int i) { return gl::canon(__ldg(c + i)); }, pi.w,
-              [&](uint64_t v) { o[k++] = v; });
+    auto wires = [&](int i) { return gl::canon(__ldg(r + i)); };
+    auto emit = [&](uint64_t v) { o[k++] = v; };
+    if (kind == GATE_POSEIDON) poseidon_gate(wires, emit);
+    else eval_gate(kind, param, wires, [&](int i) { return gl::canon(__ldg(c + i)); }, pi.w, emit);
 }
 
 enum { FILTER_NONE = 0, FILTER_COLUMN = 1, FILTER_SELECTOR = 2 };
@@ -375,8 +510,8 @@ struct QuotientArgs {
     PiHash pi;
 };
 
-// acc[k][row] += filter(row) * sum_i powers[k][i] * constraint_i(row)
-template <int NCH>
+// acc[k][row] += filter(row) * sum_i powers[k][i] * constraint_i(row); POSEIDON: the instance of GATE_POSEIDON, else every other kind
+template <int NCH, bool POSEIDON = false>
 __global__ void __launch_bounds__(128) gate_quotient_kernel(const QuotientArgs a) {
     extern __shared__ uint64_t pw[];   // [NCH][n_constraints]
     for (uint32_t i = threadIdx.x; i < NCH * a.n_constraints; i += blockDim.x) pw[i] = a.powers[i];
@@ -388,13 +523,17 @@ __global__ void __launch_bounds__(128) gate_quotient_kernel(const QuotientArgs a
 #pragma unroll
     for (int k = 0; k < NCH; k++) acc[k] = 0;
     uint32_t i = 0;
-    eval_gate((int)a.kind, a.param, [&](int j) { return gl::canon(__ldg(r + j)); },
-              [&](int j) { return gl::canon(__ldg(a.filter + row * a.filter_pitch + a.const_col0 + j)); }, a.pi.w,
-              [&](uint64_t v) {
+    auto wires = [&](int j) { return gl::canon(__ldg(r + j)); };
+    auto emit = [&](uint64_t v) {
 #pragma unroll
-                  for (int k = 0; k < NCH; k++) acc[k] = gl::add(acc[k], gl::mulc(v, pw[k * a.n_constraints + i]));
-                  i++;
-              });
+        for (int k = 0; k < NCH; k++) acc[k] = gl::add(acc[k], gl::mulc(v, pw[k * a.n_constraints + i]));
+        i++;
+    };
+    if constexpr (POSEIDON)
+        poseidon_gate(wires, emit);
+    else
+        eval_gate((int)a.kind, a.param, wires, [&](int j) { return gl::canon(__ldg(a.filter + row * a.filter_pitch + a.const_col0 + j)); },
+                  a.pi.w, emit);
     uint64_t f = 1;
     if (a.filter_mode != FILTER_NONE) {
         f = gl::canon(__ldg(a.filter + row * a.filter_pitch + a.filter_col));
@@ -471,6 +610,30 @@ __global__ void poseidon2_witness_kernel(const uint64_t* __restrict__ in, uint64
         }
         matmul_external(s);
     }
+#pragma unroll
+    for (int i = 0; i < P2_WIDTH; i++) w[P2_WIDTH + i] = s[i];
+}
+
+// PoseidonGenerator::run_once (gates/poseidon.rs) for a batch of rows, poseidon2_witness_kernel's shape: in[n][13] -> out[n][out_pitch]
+__global__ void poseidon_witness_kernel(const uint64_t* __restrict__ in, uint64_t n, uint64_t* __restrict__ out, uint32_t out_pitch) {
+    const uint64_t row = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= n) return;
+    const uint64_t* x = in + row * 13;
+    uint64_t* w = out + row * out_pitch;
+    uint64_t s[P2_WIDTH];
+#pragma unroll
+    for (int i = 0; i < P2_WIDTH; i++) { s[i] = gl::canon(x[i]); w[i] = s[i]; }
+    const uint64_t swap = gl::canon(x[12]);
+    w[P2_WIRE_SWAP] = swap;
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        w[P2_START_DELTA + i] = gl::mulc(swap, gl::sub(s[i + 4], s[i]));
+        if (swap == 1) { const uint64_t t = s[i]; s[i] = s[i + 4]; s[i + 4] = t; }   // `if swap_value == F::ONE { state.swap(i, 4 + i) }`
+    }
+    poseidon_rounds(s, [&](int wire, uint64_t v) {
+        w[wire] = v;
+        return v;
+    });
 #pragma unroll
     for (int i = 0; i < P2_WIDTH; i++) w[P2_WIDTH + i] = s[i];
 }

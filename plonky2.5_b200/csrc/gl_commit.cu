@@ -2172,6 +2172,14 @@ int gate_wires(int kind, uint32_t param) {
         case GL_GATE_PUBLIC_INPUT: return param == 0 ? 4 : -1;
         case GL_GATE_ARITHMETIC: return param >= 1 && param <= 33 ? (int)(4 * param) : -1;
         case GL_GATE_BASE_SUM: return lo >= 1 && 1 + lo <= 135 && hi >= 2 && hi <= 16 ? (int)(1 + lo) : -1;
+        case GL_GATE_POSEIDON: return param == 0 ? gates::P2_NUM_WIRES : -1;
+        case GL_GATE_EXPONENTIATION: return param >= 1 && param <= 66 ? (int)(2 + 2 * param) : -1;
+        case GL_GATE_RANDOM_ACCESS: {   // bits | num_copies << 8 | num_extra_constants << 16
+            const uint32_t copies = hi & 0xFF, extras = param >> 16;
+            if (lo < 1 || lo > 6 || copies < 1) return -1;
+            const uint32_t nw = ((2u + (1u << lo)) + lo) * copies + extras;
+            return nw <= 135 ? (int)nw : -1;
+        }
         default: return -1;
     }
 }
@@ -2192,6 +2200,9 @@ int gate_constraints(int kind, uint32_t param) {
         case GL_GATE_CONSTANT: return (int)param;
         case GL_GATE_PUBLIC_INPUT: return 4;
         case GL_GATE_ARITHMETIC: return (int)param;
+        case GL_GATE_POSEIDON: return gates::P2_NUM_CONSTRAINTS;
+        case GL_GATE_EXPONENTIATION: return (int)(param + 1);
+        case GL_GATE_RANDOM_ACCESS: return (int)((lo + 2) * (hi & 0xFF) + (param >> 16));
         default: return (int)(1 + lo);   // GL_GATE_BASE_SUM
     }
 }
@@ -2200,11 +2211,13 @@ int gate_constants(int kind, uint32_t param) {
     switch (kind) {
         case GL_GATE_CONSTANT: return (int)param;
         case GL_GATE_ARITHMETIC: return 2;
+        case GL_GATE_RANDOM_ACCESS: return (int)(param >> 16);
         default: return 0;
     }
 }
 void check_gate(int kind, uint32_t param) {
-    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_BASE_SUM) GL_THROW(GL_ERR_INVALID, "unknown gate kind %d", kind);
+    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_RANDOM_ACCESS || (kind > GL_GATE_BASE_SUM && kind < GL_GATE_POSEIDON))
+        GL_THROW(GL_ERR_INVALID, "unknown gate kind %d", kind);
     if (gate_wires(kind, param) < 0) GL_THROW(GL_ERR_INVALID, "gate kind %d: parameter %u out of range (see include/gl_commit.h)", kind, param);
 }
 // the entry points without gate constants / public-inputs hash refuse the gates that read them
@@ -2244,15 +2257,33 @@ void alpha_powers(const uint64_t* alphas, uint32_t n_ch, uint32_t offset, uint32
 }
 
 void launch_gate_quotient(gl_ctx* c, const gates::QuotientArgs& a) {
+    // PoseidonGate has its own instances: the shared switch keeps the registers (and CTAs per SM) it has without it
+    static void (*const kernels[2][4])(gates::QuotientArgs) = {
+        {gates::gate_quotient_kernel<1>, gates::gate_quotient_kernel<2>, gates::gate_quotient_kernel<3>, gates::gate_quotient_kernel<4>},
+        {gates::gate_quotient_kernel<1, true>, gates::gate_quotient_kernel<2, true>, gates::gate_quotient_kernel<3, true>,
+         gates::gate_quotient_kernel<4, true>}};
     const uint32_t grid = (uint32_t)((a.n_rows + 127) / 128);
     const size_t smem = (size_t)a.n_challenges * a.n_constraints * 8;
-    switch (a.n_challenges) {
-        case 1: gates::gate_quotient_kernel<1><<<grid, 128, smem, c->stream>>>(a); break;
-        case 2: gates::gate_quotient_kernel<2><<<grid, 128, smem, c->stream>>>(a); break;
-        case 3: gates::gate_quotient_kernel<3><<<grid, 128, smem, c->stream>>>(a); break;
-        default: gates::gate_quotient_kernel<4><<<grid, 128, smem, c->stream>>>(a); break;
-    }
+    kernels[a.kind == GL_GATE_POSEIDON][std::min(a.n_challenges, 4u) - 1]<<<grid, 128, smem, c->stream>>>(a);
     CUDA_CHECK(cudaGetLastError());
+}
+
+// gl_poseidon2_gate_witness / gl_poseidon_gate_witness: inputs [n][13] -> out_rows [n][135], kernel time in aux_ms
+void gate_witness(gl_ctx* c, const uint64_t* inputs, uint64_t n, uint64_t* out_rows,
+                  void (*kernel)(const uint64_t*, uint64_t, uint64_t*, uint32_t)) {
+    if ((!inputs || !out_rows) && n) GL_THROW(GL_ERR_INVALID, "NULL pointer");
+    if (n == 0) return;
+    c->scratch.ensure(n * (13 + gates::P2_NUM_WIRES));
+    uint64_t* d_in = c->scratch.p;
+    uint64_t* d_out = d_in + n * 13;
+    CUDA_CHECK(cudaMemcpyAsync(d_in, inputs, n * 13 * 8, cudaMemcpyHostToDevice, c->stream));
+    CUDA_CHECK(cudaEventRecord(c->ev[0], c->stream));
+    kernel<<<(uint32_t)((n + 127) / 128), 128, 0, c->stream>>>(d_in, n, d_out, gates::P2_NUM_WIRES);
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaEventRecord(c->ev[1], c->stream));
+    CUDA_CHECK(cudaMemcpyAsync(out_rows, d_out, n * gates::P2_NUM_WIRES * 8, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    CUDA_CHECK(cudaEventElapsedTime(&c->aux_ms, c->ev[0], c->ev[1]));
 }
 }  // namespace
 
@@ -2519,19 +2550,14 @@ int gl_ctx_aux_ms(gl_ctx* c, float* out_ms) {
 
 int gl_poseidon2_gate_witness(gl_ctx* c, const uint64_t* inputs, uint64_t n, uint64_t* out_rows) {
     GL_API_BEGIN(c)
-    if ((!inputs || !out_rows) && n) GL_THROW(GL_ERR_INVALID, "NULL pointer");
-    if (n == 0) return GL_OK;
-    c->scratch.ensure(n * (13 + gates::P2_NUM_WIRES));
-    uint64_t* d_in = c->scratch.p;
-    uint64_t* d_out = d_in + n * 13;
-    CUDA_CHECK(cudaMemcpyAsync(d_in, inputs, n * 13 * 8, cudaMemcpyHostToDevice, c->stream));
-    CUDA_CHECK(cudaEventRecord(c->ev[0], c->stream));
-    gates::poseidon2_witness_kernel<<<(uint32_t)((n + 127) / 128), 128, 0, c->stream>>>(d_in, n, d_out, gates::P2_NUM_WIRES);
-    CUDA_CHECK(cudaGetLastError());
-    CUDA_CHECK(cudaEventRecord(c->ev[1], c->stream));
-    CUDA_CHECK(cudaMemcpyAsync(out_rows, d_out, n * gates::P2_NUM_WIRES * 8, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_CHECK(cudaStreamSynchronize(c->stream));
-    CUDA_CHECK(cudaEventElapsedTime(&c->aux_ms, c->ev[0], c->ev[1]));
+    gate_witness(c, inputs, n, out_rows, gates::poseidon2_witness_kernel);
+    return GL_OK;
+    GL_API_END(c)
+}
+
+int gl_poseidon_gate_witness(gl_ctx* c, const uint64_t* inputs, uint64_t n, uint64_t* out_rows) {
+    GL_API_BEGIN(c)
+    gate_witness(c, inputs, n, out_rows, gates::poseidon_witness_kernel);
     return GL_OK;
     GL_API_END(c)
 }

@@ -245,6 +245,18 @@ impl Context {
         Ok(out)
     }
 
+    /// plonky2 `gates/poseidon.rs · PoseidonGenerator::run_once` for `inputs.len() / 13` PoseidonGate rows (12 state inputs + swap flag
+    /// each) -> 135 wires per row
+    pub fn poseidon_gate_witness(&self, inputs: &[u64]) -> Result<Vec<u64>, Error> {
+        if inputs.len() % 13 != 0 {
+            return Err(Error::Invalid("inputs must be n * 13 words".into()));
+        }
+        let n = inputs.len() / 13;
+        let mut out = vec![0u64; n * 135];
+        self.check(unsafe { ffi::gl_poseidon_gate_witness(self.raw, inputs.as_ptr(), n as u64, out.as_mut_ptr()) })?;
+        Ok(out)
+    }
+
     pub fn openings_begin(&self, log_n: usize) -> Result<Openings<'_>, Error> {
         let mut h: ffi::gl_handle = 0;
         self.check(unsafe { ffi::gl_openings_begin(self.raw, log_n as u32, &mut h) })?;
