@@ -192,16 +192,27 @@ int gl_fri_read(gl_ctx* ctx, gl_handle fri, uint64_t* out_coeffs_ext, uint64_t* 
  *   GL_GATE_RANDOM_ACCESS   RandomAccessGate                   param = bits | num_copies << 8 | num_extra_constants << 16
  *                           (bits 1..6, v = 2^bits, (2+v+bits)*num_copies + num_extra_constants <= 135 wires)
  *                                                              (bits+2)*num_copies + num_extra_constants constraints, num_extra_constants constants
- * Kind 14 is not assigned: it stays an unknown kind, as it was before these three gates existed.
+ * and plonky2's extension-field gates, D = 2 (plonky2 @ 3de92d9 gates/{arithmetic_extension,multiplication_extension,reducing_extension}.rs;
+ * restated, parity unpinned).  An extension value is two consecutive wires [a0, a1] in F_p[X]/(X^2 - 7); each extension constraint is two
+ * base constraints, component 0 first:
+ *   GL_GATE_ARITHMETIC_EXTENSION  ArithmeticExtensionGate   param = num_ops (1..16; 10 = new_from_config at 80 routed)
+ *                                                           8n wires, 2n constraints, 2 constants (degree 3)
+ *   GL_GATE_MUL_EXTENSION         MulExtensionGate          param = num_ops (1..22; 13 = new_from_config at 80 routed)
+ *                                                           6n wires, 2n constraints, 1 constant (degree 3)
+ *   GL_GATE_REDUCING_EXTENSION    ReducingExtensionGate     param = num_coeffs (1..32; 32 = max_coeffs_len(135, 80))
+ *                                                           4 + 4n wires, 2n constraints, 0 constants (degree 2)
+ * Kinds 14 and 18 are not assigned: they stay unknown kinds, as they were in earlier releases.
  * gl_quotient_add_gate:  acc[k][row] += filter(row) * sum_i alphas[k]^(constraint_offset + i) * constraint_i(wires(row)),  k < n_challenges
  * (alphas are BASE-field challenges, as upstream; filter(row) = column filter_col of the batch filter_batch at the same row, or 1 when
  * filter_batch == 0).  gl_quotient_read: [n_challenges][R] words, row order = the leaves' (bit-reversed).
  * gl_gate_eval_rows and gl_quotient_add_gate refuse the gates that read gate constants or the public-inputs hash (CONSTANT, ARITHMETIC,
- * PUBLIC_INPUT, and RANDOM_ACCESS with extra constants): those go through gl_gate_eval_rows_with_constants and gl_quotient_add_gates. */
+ * PUBLIC_INPUT, RANDOM_ACCESS with extra constants, ARITHMETIC_EXTENSION and MUL_EXTENSION): those go through
+ * gl_gate_eval_rows_with_constants and gl_quotient_add_gates. */
 enum { GL_GATE_POSEIDON2 = 0, GL_GATE_U32_ARITHMETIC = 1, GL_GATE_U32_ADD_MANY = 2, GL_GATE_U32_SUBTRACTION = 3, GL_GATE_U32_RANGE_CHECK = 4,
        GL_GATE_U32_INTERLEAVE = 5, GL_GATE_UNINTERLEAVE_TO_U32 = 6, GL_GATE_UNINTERLEAVE_TO_B32 = 7, GL_GATE_COMPARISON = 8, GL_GATE_NOOP = 9,
        GL_GATE_CONSTANT = 10, GL_GATE_PUBLIC_INPUT = 11, GL_GATE_ARITHMETIC = 12, GL_GATE_BASE_SUM = 13, GL_GATE_POSEIDON = 15,
-       GL_GATE_EXPONENTIATION = 16, GL_GATE_RANDOM_ACCESS = 17 };
+       GL_GATE_EXPONENTIATION = 16, GL_GATE_RANDOM_ACCESS = 17, GL_GATE_ARITHMETIC_EXTENSION = 19, GL_GATE_MUL_EXTENSION = 20,
+       GL_GATE_REDUCING_EXTENSION = 21 };
 int gl_gate_num_wires(int kind, uint32_t param);
 int gl_gate_num_constraints(int kind, uint32_t param);
 /* Gate::num_constants: the gate constants a gate reads (-1 for a bad kind or parameter) */

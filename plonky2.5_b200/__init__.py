@@ -14,6 +14,7 @@ from .api import (GATE_COMPARISON, GATE_POSEIDON2, GATE_U32_ADD_MANY, GATE_U32_A
                   partial_products_and_zs, poseidon2_gate_witness)
 from .api import GATE_ARITHMETIC, GATE_BASE_SUM, GATE_CONSTANT, GATE_NOOP, GATE_PUBLIC_INPUT, SelectorsInfo  # noqa: F401
 from .api import GATE_EXPONENTIATION, GATE_POSEIDON, GATE_RANDOM_ACCESS, poseidon_gate_witness, random_access_params  # noqa: F401
+from .api import GATE_ARITHMETIC_EXTENSION, GATE_MUL_EXTENSION, GATE_REDUCING_EXTENSION  # noqa: F401
 from .build import build  # noqa: F401
 
 __all__ = ["Challenger", "Context", "FriBatchInfo", "FriOpeningBatch", "FriOpenings", "FriParams", "FriProofHead", "GlError", "MerkleCap",

@@ -610,6 +610,9 @@ GATE_U32_INTERLEAVE, GATE_UNINTERLEAVE_TO_U32, GATE_UNINTERLEAVE_TO_B32, GATE_CO
 GATE_NOOP, GATE_CONSTANT, GATE_PUBLIC_INPUT, GATE_ARITHMETIC, GATE_BASE_SUM = 9, 10, 11, 12, 13
 # PoseidonGate (param 0), ExponentiationGate { num_power_bits }, RandomAccessGate (bits | num_copies << 8 | num_extra_constants << 16)
 GATE_POSEIDON, GATE_EXPONENTIATION, GATE_RANDOM_ACCESS = 15, 16, 17
+# plonky2's extension-field gates (D = 2): ArithmeticExtensionGate { num_ops } (1..16; new_from_config: 10 at 80 routed wires),
+# MulExtensionGate { num_ops } (1..22; new_from_config: 13), ReducingExtensionGate { num_coeffs } (1..32; max_coeffs_len(135, 80) = 32)
+GATE_ARITHMETIC_EXTENSION, GATE_MUL_EXTENSION, GATE_REDUCING_EXTENSION = 19, 20, 21
 
 
 def random_access_params(bits: int, num_wires: int = 135, num_routed: int = 80, num_constants: int = 2) -> int:

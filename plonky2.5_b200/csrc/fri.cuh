@@ -10,17 +10,6 @@
 
 namespace fri {
 
-struct Ext { uint64_t a0, a1; };
-
-__device__ __forceinline__ Ext ext_mul(Ext a, Ext b) {   // canonical in/out
-    uint64_t m00 = gl::mulc(a.a0, b.a0), m11 = gl::mulc(a.a1, b.a1);
-    uint64_t m01 = gl::mulc(a.a0, b.a1), m10 = gl::mulc(a.a1, b.a0);
-    Ext r;
-    r.a0 = gl::add(m00, gl::mulc(m11, 7));
-    r.a1 = gl::add(m01, m10);
-    return r;
-}
-
 // dst[i] = canon(src[bitrev_bits(i)]) for extension elements (16 B each)
 __global__ void bitrev_gather_ext_kernel(const ulonglong2* __restrict__ src, ulonglong2* __restrict__ dst, uint32_t bits) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -39,11 +28,11 @@ __global__ void fold_kernel(const ulonglong2* __restrict__ in, ulonglong2* __res
                             uint32_t arity, uint64_t beta0, uint64_t beta1) {
     uint32_t m = blockIdx.x * blockDim.x + threadIdx.x;
     if (m >= n_out) return;
-    Ext beta = {beta0, beta1};
-    Ext acc = {0, 0};
+    gl::Ext beta = {beta0, beta1};
+    gl::Ext acc = {0, 0};
     for (uint32_t t = arity; t-- > 0;) {
         ulonglong2 c = in[(size_t)arity * m + t];
-        acc = ext_mul(acc, beta);
+        acc = gl::ext_mul(acc, beta);
         acc.a0 = gl::add(acc.a0, c.x);
         acc.a1 = gl::add(acc.a1, c.y);
     }

@@ -438,10 +438,56 @@ __device__ __forceinline__ void random_access_gate(Wires&& w, Consts&& k, Emit&&
     for (uint32_t i = 0; i < extras; i++) emit(gl::sub(k(i), w(extra0 + i)));
 }
 
+// ---- plonky2's extension-field gates (plonky2 @ 3de92d9 gates/{arithmetic_extension,multiplication_extension,reducing_extension}.rs ·
+// eval_unfiltered, D = 2; restated, parity unpinned, tests/plonky2_ext_gates_oracle.py restates them too).  An extension value is the two
+// wires [a0, a1]; every extension constraint is emitted as to_basefield_array(), component 0 first, so it is two base constraints.
+template <class Wires>
+__device__ __forceinline__ gl::Ext ext_wire(uint32_t i, Wires&& w) { return {w(i), w(i + 1)}; }
+template <class Emit>
+__device__ __forceinline__ void emit_ext_sub(gl::Ext a, gl::Ext b, Emit&& emit) {
+    emit(gl::sub(a.a0, b.a0));
+    emit(gl::sub(a.a1, b.a1));
+}
+
+// ArithmeticExtensionGate: param = num_ops; op i at wires 8i + [m0, m1, addend, output]: output - ((m0 m1) k(0) + addend k(1))
+template <class Wires, class Consts, class Emit>
+__device__ __forceinline__ void arithmetic_extension_gate(Wires&& w, Consts&& k, Emit&& emit, uint32_t num_ops) {
+    const uint64_t c0 = k(0), c1 = k(1);
+#pragma unroll 1
+    for (uint32_t i = 0; i < num_ops; i++) {
+        const gl::Ext p = gl::ext_mul(ext_wire(8 * i, w), ext_wire(8 * i + 2, w)), a = ext_wire(8 * i + 4, w);
+        const gl::Ext computed = {gl::add(gl::mulc(p.a0, c0), gl::mulc(a.a0, c1)), gl::add(gl::mulc(p.a1, c0), gl::mulc(a.a1, c1))};
+        emit_ext_sub(ext_wire(8 * i + 6, w), computed, emit);
+    }
+}
+// MulExtensionGate: param = num_ops; op i at wires 6i + [m0, m1, output]: output - (m0 m1) k(0)
+template <class Wires, class Consts, class Emit>
+__device__ __forceinline__ void mul_extension_gate(Wires&& w, Consts&& k, Emit&& emit, uint32_t num_ops) {
+    const uint64_t c0 = k(0);
+#pragma unroll 1
+    for (uint32_t i = 0; i < num_ops; i++) {
+        const gl::Ext p = gl::ext_mul(ext_wire(6 * i, w), ext_wire(6 * i + 2, w));
+        emit_ext_sub(ext_wire(6 * i + 4, w), {gl::mulc(p.a0, c0), gl::mulc(p.a1, c0)}, emit);
+    }
+}
+// ReducingExtensionGate: param = num_coeffs n; output 0, alpha 2, old_acc 4, coefficient i at 6 + 2i, accumulator i at 6 + 2n + 2i for
+// i < n - 1 and accumulator n - 1 is the output.  From acc = old_acc: acc alpha + coeff_i - acc_i, then acc = acc_i (the wire)
+template <class Wires, class Emit>
+__device__ __forceinline__ void reducing_extension_gate(Wires&& w, Emit&& emit, uint32_t n) {
+    const gl::Ext alpha = ext_wire(2, w);
+    gl::Ext acc = ext_wire(4, w);
+#pragma unroll 1
+    for (uint32_t i = 0; i < n; i++) {
+        const gl::Ext acc_i = ext_wire(i + 1 < n ? 6 + 2 * n + 2 * i : 0, w);
+        emit_ext_sub(gl::ext_add(gl::ext_mul(acc, alpha), ext_wire(6 + 2 * i, w)), acc_i, emit);
+        acc = acc_i;
+    }
+}
+
 enum { GATE_POSEIDON2 = 0, GATE_U32_ARITHMETIC = 1, GATE_U32_ADD_MANY = 2, GATE_U32_SUBTRACTION = 3, GATE_U32_RANGE_CHECK = 4,
        GATE_U32_INTERLEAVE = 5, GATE_UNINTERLEAVE_TO_U32 = 6, GATE_UNINTERLEAVE_TO_B32 = 7, GATE_COMPARISON = 8, GATE_NOOP = 9,
        GATE_CONSTANT = 10, GATE_PUBLIC_INPUT = 11, GATE_ARITHMETIC = 12, GATE_BASE_SUM = 13, GATE_POSEIDON = 15, GATE_EXPONENTIATION = 16,
-       GATE_RANDOM_ACCESS = 17 };
+       GATE_RANDOM_ACCESS = 17, GATE_ARITHMETIC_EXTENSION = 19, GATE_MUL_EXTENSION = 20, GATE_REDUCING_EXTENSION = 21 };
 
 // every kind but GATE_POSEIDON, which has kernel instances of its own (inlined here it would raise the register count of every gate)
 template <class Wires, class Consts, class Emit>
@@ -461,6 +507,9 @@ __device__ __forceinline__ void eval_gate(int kind, uint32_t param, Wires&& w, C
         case GATE_BASE_SUM: base_sum_gate(w, emit, param); break;
         case GATE_EXPONENTIATION: exponentiation_gate(w, emit, param); break;
         case GATE_RANDOM_ACCESS: random_access_gate(w, k, emit, param); break;
+        case GATE_ARITHMETIC_EXTENSION: arithmetic_extension_gate(w, k, emit, param); break;
+        case GATE_MUL_EXTENSION: mul_extension_gate(w, k, emit, param); break;
+        case GATE_REDUCING_EXTENSION: reducing_extension_gate(w, emit, param); break;
         case GATE_NOOP: break;
         default: comparison_gate(w, emit, param); break;
     }

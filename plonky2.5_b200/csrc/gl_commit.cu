@@ -2180,6 +2180,9 @@ int gate_wires(int kind, uint32_t param) {
             const uint32_t nw = ((2u + (1u << lo)) + lo) * copies + extras;
             return nw <= 135 ? (int)nw : -1;
         }
+        case GL_GATE_ARITHMETIC_EXTENSION: return param >= 1 && param <= 16 ? (int)(8 * param) : -1;
+        case GL_GATE_MUL_EXTENSION: return param >= 1 && param <= 22 ? (int)(6 * param) : -1;
+        case GL_GATE_REDUCING_EXTENSION: return param >= 1 && param <= 32 ? (int)(4 + 4 * param) : -1;
         default: return -1;
     }
 }
@@ -2203,6 +2206,9 @@ int gate_constraints(int kind, uint32_t param) {
         case GL_GATE_POSEIDON: return gates::P2_NUM_CONSTRAINTS;
         case GL_GATE_EXPONENTIATION: return (int)(param + 1);
         case GL_GATE_RANDOM_ACCESS: return (int)((lo + 2) * (hi & 0xFF) + (param >> 16));
+        case GL_GATE_ARITHMETIC_EXTENSION:
+        case GL_GATE_MUL_EXTENSION:
+        case GL_GATE_REDUCING_EXTENSION: return (int)(2 * param);
         default: return (int)(1 + lo);   // GL_GATE_BASE_SUM
     }
 }
@@ -2210,13 +2216,16 @@ int gate_constants(int kind, uint32_t param) {
     if (gate_wires(kind, param) < 0) return -1;
     switch (kind) {
         case GL_GATE_CONSTANT: return (int)param;
-        case GL_GATE_ARITHMETIC: return 2;
+        case GL_GATE_ARITHMETIC:
+        case GL_GATE_ARITHMETIC_EXTENSION: return 2;
+        case GL_GATE_MUL_EXTENSION: return 1;
         case GL_GATE_RANDOM_ACCESS: return (int)(param >> 16);
         default: return 0;
     }
 }
 void check_gate(int kind, uint32_t param) {
-    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_RANDOM_ACCESS || (kind > GL_GATE_BASE_SUM && kind < GL_GATE_POSEIDON))
+    // kinds 14 and 18 are not assigned: earlier releases refused them as unknown kinds, and they still are
+    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_REDUCING_EXTENSION || kind == 14 || kind == 18)
         GL_THROW(GL_ERR_INVALID, "unknown gate kind %d", kind);
     if (gate_wires(kind, param) < 0) GL_THROW(GL_ERR_INVALID, "gate kind %d: parameter %u out of range (see include/gl_commit.h)", kind, param);
 }

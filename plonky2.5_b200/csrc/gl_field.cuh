@@ -161,6 +161,19 @@ __device__ __forceinline__ uint64_t sub_any(uint64_t a, uint64_t b) {
         "}" : "=&r"(l), "=&r"(h) : "r"((uint32_t)a), "r"((uint32_t)(a >> 32)), "r"((uint32_t)b), "r"((uint32_t)(b >> 32)));
     return ((uint64_t)h << 32) | l;
 }
+// The quadratic extension F_p[X]/(X^2 - 7) (plonky2 field/src/extension/quadratic.rs; W = 7 as /root/reference/src/p3/extension.rs:147-151):
+// an element is [a0, a1] = a0 + a1 X.  The one device F_p^2 product: FRI folding, openings and the extension gates use it.
+struct Ext { uint64_t a0, a1; };
+__device__ __forceinline__ Ext ext_mul(Ext a, Ext b) {   // canonical in/out
+    uint64_t m00 = mulc(a.a0, b.a0), m11 = mulc(a.a1, b.a1);
+    uint64_t m01 = mulc(a.a0, b.a1), m10 = mulc(a.a1, b.a0);
+    Ext r;
+    r.a0 = add(m00, mulc(m11, 7));
+    r.a1 = add(m01, m10);
+    return r;
+}
+__device__ __forceinline__ Ext ext_add(Ext a, Ext b) { return {add(a.a0, b.a0), add(a.a1, b.a1)}; }
+
 // x * 2^24 and x * 2^48 (any -> any): the 8th and 4th roots of unity of plonky2's root choice are powers of two
 // (w_8 = 2^120 = -2^24, w_4 = 2^48, w_8^3 = 2^168 = -2^72), so the radix-8 butterflies need shifts, not multiplies.
 __device__ __forceinline__ uint64_t mul_2_24(uint64_t x) {

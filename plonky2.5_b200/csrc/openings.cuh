@@ -32,43 +32,41 @@ __global__ void reduce_polys_base_kernel(const PolyRef* __restrict__ polys, cons
     out[k] = make_ulonglong2(a0, a1);
 }
 
-__device__ __forceinline__ fri::Ext ext_add(fri::Ext a, fri::Ext b) { return {gl::add(a.a0, b.a0), gl::add(a.a1, b.a1)}; }
-
 // In place: f (n extension coefficients) -> q with q[k] = f[k+1] + z*q[k+1], q[n-1] = 0  (synthetic division by X - z).
 // One CTA; thread t owns the chunk [t*L, (t+1)*L): (1) Horner value of its chunk, (2) a serial right-to-left carry over
 // the <= 1024 chunk values by thread 0, (3) the chunk's quotient coefficients from its carry-in.
 __global__ void divide_by_linear_kernel(ulonglong2* __restrict__ f, uint32_t n, uint64_t z0, uint64_t z1) {
-    __shared__ fri::Ext chunk_val[1024];
-    __shared__ fri::Ext carry_in[1024];
+    __shared__ gl::Ext chunk_val[1024];
+    __shared__ gl::Ext carry_in[1024];
     const uint32_t T = blockDim.x, t = threadIdx.x, L = n / T;   // n, T powers of two, T <= n
-    const fri::Ext z = {z0, z1};
+    const gl::Ext z = {z0, z1};
     // (1) h_t = sum_{i in chunk} f[i] z^(i - t*L)
-    fri::Ext h = {0, 0};
+    gl::Ext h = {0, 0};
     for (uint32_t i = L; i-- > 0;) {
         const ulonglong2 c = f[(size_t)t * L + i];
-        h = fri::ext_mul(h, z);
-        h = ext_add(h, {c.x, c.y});
+        h = gl::ext_mul(h, z);
+        h = gl::ext_add(h, {c.x, c.y});
     }
     chunk_val[t] = h;
     __syncthreads();
     // (2) carry_in[t] = sum_{i >= (t+1)L} f[i] z^(i - (t+1)L)  (= q[(t+1)L - 1], the quotient coefficient just left of chunk t+1)
     if (t == 0) {
-        fri::Ext zL = {1, 0};
-        for (uint32_t i = 0; i < L; i++) zL = fri::ext_mul(zL, z);
-        fri::Ext acc = {0, 0};
+        gl::Ext zL = {1, 0};
+        for (uint32_t i = 0; i < L; i++) zL = gl::ext_mul(zL, z);
+        gl::Ext acc = {0, 0};
         for (uint32_t u = T; u-- > 0;) {
             carry_in[u] = acc;
-            acc = ext_add(fri::ext_mul(acc, zL), chunk_val[u]);
+            acc = gl::ext_add(gl::ext_mul(acc, zL), chunk_val[u]);
         }
     }
     __syncthreads();
     // (3) q[k] = f[k+1] + z*q[k+1] inside the chunk, starting from q[(t+1)L - 1] = carry_in[t]
-    fri::Ext q = carry_in[t];
+    gl::Ext q = carry_in[t];
     for (uint32_t i = L; i-- > 0;) {
         const size_t k = (size_t)t * L + i;
         const ulonglong2 c = f[k];                      // f[k] is needed for q[k-1]; read before overwriting
         f[k] = make_ulonglong2(q.a0, q.a1);
-        q = ext_add(fri::ext_mul(q, z), {c.x, c.y});
+        q = gl::ext_add(gl::ext_mul(q, z), {c.x, c.y});
     }
 }
 
@@ -77,7 +75,7 @@ __global__ void shift_add_kernel(ulonglong2* __restrict__ fin, const ulonglong2*
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
     const ulonglong2 a = fin[k], b = q[k];
-    fri::Ext r = fri::ext_mul({a.x, a.y}, {s0, s1});
+    gl::Ext r = gl::ext_mul({a.x, a.y}, {s0, s1});
     fin[k] = make_ulonglong2(gl::add(r.a0, b.x), gl::add(r.a1, b.y));
 }
 
@@ -97,10 +95,10 @@ constexpr uint32_t EVAL_BATCH = 8;       // coefficient loads a thread issues be
 
 struct EvalPoints { uint64_t z2k[2][32][2]; };   // z_p^(2^b), canonical
 
-__device__ __forceinline__ fri::Ext ext_pow_table(const uint64_t (*z2k)[2], uint64_t e) {
-    fri::Ext r = {1, 0};
+__device__ __forceinline__ gl::Ext ext_pow_table(const uint64_t (*z2k)[2], uint64_t e) {
+    gl::Ext r = {1, 0};
     for (uint32_t b = 0; e; b++, e >>= 1)
-        if (e & 1) r = fri::ext_mul(r, {z2k[b][0], z2k[b][1]});
+        if (e & 1) r = gl::ext_mul(r, {z2k[b][0], z2k[b][1]});
     return r;
 }
 
@@ -108,13 +106,13 @@ template <int NP>
 __global__ void __launch_bounds__(EVAL_THREADS) batch_eval_partial_kernel(const uint64_t* __restrict__ coeffs, uint32_t pitch,
                                                                           uint32_t leaf_len, uint32_t wc, uint32_t lanes, uint32_t sub_rows,
                                                                           uint32_t subs, const EvalPoints pts, ulonglong2* __restrict__ partial) {
-    __shared__ fri::Ext pw[NP][EVAL_SUB];
-    __shared__ fri::Ext red[NP][EVAL_THREADS];
+    __shared__ gl::Ext pw[NP][EVAL_SUB];
+    __shared__ gl::Ext red[NP][EVAL_THREADS];
     const uint32_t t = threadIdx.x, lane = t / wc, cl = t - lane * wc, col = blockIdx.y * wc + cl;
     const bool live = lane < lanes && col < leaf_len;
     const uint32_t log_sub = 31 - __clz(sub_rows);
     const uint64_t row0 = (uint64_t)blockIdx.x * subs * sub_rows;
-    fri::Ext acc[NP];
+    gl::Ext acc[NP];
 #pragma unroll
     for (int p = 0; p < NP; p++) acc[p] = {0, 0};
     for (uint32_t s = 0; s < subs; s++) {
@@ -124,7 +122,7 @@ __global__ void __launch_bounds__(EVAL_THREADS) batch_eval_partial_kernel(const 
 #pragma unroll
             for (int p = 0; p < NP; p++)
                 pw[p][i] = s == 0 ? ext_pow_table(pts.z2k[p], r0 + i)
-                                  : fri::ext_mul(pw[p][i], {pts.z2k[p][log_sub][0], pts.z2k[p][log_sub][1]});
+                                  : gl::ext_mul(pw[p][i], {pts.z2k[p][log_sub][0], pts.z2k[p][log_sub][1]});
         }
         __syncthreads();
         if (live) {
@@ -142,7 +140,7 @@ __global__ void __launch_bounds__(EVAL_THREADS) batch_eval_partial_kernel(const 
                     if (r < sub_rows) {
 #pragma unroll
                         for (int p = 0; p < NP; p++) {
-                            const fri::Ext w = pw[p][r];
+                            const gl::Ext w = pw[p][r];
                             acc[p].a0 = gl::add(acc[p].a0, gl::mulc(v[u], w.a0));
                             acc[p].a1 = gl::add(acc[p].a1, gl::mulc(v[u], w.a1));
                         }
@@ -157,8 +155,8 @@ __global__ void __launch_bounds__(EVAL_THREADS) batch_eval_partial_kernel(const 
     if (lane == 0 && col < leaf_len) {
 #pragma unroll
         for (int p = 0; p < NP; p++) {
-            fri::Ext sum = red[p][cl];
-            for (uint32_t l = 1; l < lanes; l++) sum = ext_add(sum, red[p][l * wc + cl]);
+            gl::Ext sum = red[p][cl];
+            for (uint32_t l = 1; l < lanes; l++) sum = gl::ext_add(sum, red[p][l * wc + cl]);
             partial[((size_t)blockIdx.x * NP + p) * leaf_len + col] = make_ulonglong2(sum.a0, sum.a1);
         }
     }
@@ -166,18 +164,18 @@ __global__ void __launch_bounds__(EVAL_THREADS) batch_eval_partial_kernel(const 
 
 // out[i] = sum_x partial[x][i], i < n_out (= n_points * leaf_len).  Block (32, 32): threadIdx.x walks i (coalesced), threadIdx.y walks x.
 __global__ void batch_eval_reduce_kernel(const ulonglong2* __restrict__ partial, uint32_t n_parts, uint32_t n_out, ulonglong2* __restrict__ out) {
-    __shared__ fri::Ext red[32][33];
+    __shared__ gl::Ext red[32][33];
     const uint32_t i = blockIdx.x * 32 + threadIdx.x;
-    fri::Ext sum = {0, 0};
+    gl::Ext sum = {0, 0};
     if (i < n_out)
         for (uint32_t x = threadIdx.y; x < n_parts; x += 32) {
             const ulonglong2 v = partial[(size_t)x * n_out + i];
-            sum = ext_add(sum, {v.x, v.y});
+            sum = gl::ext_add(sum, {v.x, v.y});
         }
     red[threadIdx.y][threadIdx.x] = sum;
     __syncthreads();
     if (threadIdx.y == 0 && i < n_out) {
-        for (uint32_t y = 1; y < 32; y++) sum = ext_add(sum, red[y][threadIdx.x]);
+        for (uint32_t y = 1; y < 32; y++) sum = gl::ext_add(sum, red[y][threadIdx.x]);
         out[i] = make_ulonglong2(sum.a0, sum.a1);
     }
 }

@@ -1,13 +1,16 @@
-"""Device time of plonky2's PoseidonGate, ExponentiationGate(66) and RandomAccessGate(bits 4, 4 copies, 2 extra constants) in
-gl_quotient_add_gates at the wrapper shape, and of the PoseidonGate witness generator; prints one JSON line (and writes it to --out).
+"""Device time of plonky2's PoseidonGate, ExponentiationGate(66), RandomAccessGate(bits 4, 4 copies, 2 extra constants) and of the
+extension-field gates ArithmeticExtensionGate(10), MulExtensionGate(13) and ReducingExtensionGate(32) in gl_quotient_add_gates at the
+wrapper shape, and of the PoseidonGate witness generator; prints one JSON line (and writes it to --out).
 
     python tools/plonky2_gates_bench.py [--repeats 20] [--warmup 3] [--out FILE]
 
 Shape (as tools/quotient_gates_bench.py): N = 2^16, rate_bits 3 (R = 2^19 LDE rows), a 135-column wires commit, a constants/sigmas commit
-with 3 selectors, 2 gate constants and 80 sigmas, 2 challenges.  Gate list [Poseidon] [Poseidon2] [Exponentiation(66), RandomAccess] in
-3 selector groups.
+with 4 selectors, 2 gate constants and 80 sigmas, 2 challenges.  Gate list [Poseidon] [Poseidon2] [Exponentiation(66), RandomAccess]
+[ArithmeticExtension(10), Arithmetic(20), MulExtension(13), ReducingExtension(32)] in 4 selector groups.
   per_gate_ms         one add_gates call with every other gate replaced by NoopGate: one launch, median over the repeats.  PoseidonGate
-                      and Poseidon2Gate (same wires, same constraint count) are run alternately in the same process.
+                      and Poseidon2Gate (same wires, same constraint count) are run alternately in the same process, and so are
+                      ArithmeticExtensionGate(10) and ArithmeticGate(20) (both 80 routed wires and 20 constraints: the pair shows
+                      what the extension product costs).
   witness_ms          gl_poseidon_gate_witness and gl_poseidon2_gate_witness for 2^16 rows, alternately (kernel time, CUDA events).
   parity              the accumulator of each gate's first timed launch equals the oracle's eval_filtered (reduced with the two alphas)
                       at 64 sampled LDE rows, and the timed PoseidonGate witness rows' outputs equal Context.poseidon_permute of the
@@ -29,16 +32,18 @@ for p in (ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "oracle"), os.pa
 
 import plonky25_b200 as g  # noqa: E402
 import gates_oracle as go  # noqa: E402
-import plonky2_std_gates_oracle as pgo  # noqa: E402
+import plonky2_ext_gates_oracle as pgo  # noqa: E402
 from oracle_c import splitmix_columns  # noqa: E402
 from quotient_gates_bench import gpu_info  # noqa: E402
 
 P = g.api.P
 LOG_N, RATE_BITS, N_CH, WITNESS_ROWS = 16, 3, 2, 1 << 16
 GATES = [("poseidon", g.GATE_POSEIDON, 0), ("poseidon2", g.GATE_POSEIDON2, 0), ("exponentiation_66", g.GATE_EXPONENTIATION, 66),
-         ("random_access_4x4_2", g.GATE_RANDOM_ACCESS, g.random_access_params(4))]
-GROUPS = [(0, 1), (1, 2), (2, 4)]
-SELECTORS = [0, 1, 2, 2]
+         ("random_access_4x4_2", g.GATE_RANDOM_ACCESS, g.random_access_params(4)),
+         ("arithmetic_extension_10", g.GATE_ARITHMETIC_EXTENSION, 10), ("arithmetic_20", g.GATE_ARITHMETIC, 20),
+         ("mul_extension_13", g.GATE_MUL_EXTENSION, 13), ("reducing_extension_32", g.GATE_REDUCING_EXTENSION, 32)]
+GROUPS = [(0, 1), (1, 2), (2, 4), (4, 8)]
+SELECTORS = [0, 1, 2, 2, 3, 3, 3, 3]
 NUM_CONSTANTS = len(GROUPS) + 2
 
 
@@ -100,7 +105,7 @@ def main():
         witness(g.poseidon_gate_witness); witness(g.poseidon2_gate_witness)
     t_wit = {"poseidon": [], "poseidon2": []}
     for _ in range(args.repeats):
-        for i, (name, _, _) in enumerate(GATES):      # Poseidon and Poseidon2 alternate within every repeat
+        for i, (name, _, _) in enumerate(GATES):      # Poseidon / Poseidon2 and ArithmeticExtension / Arithmetic alternate in every repeat
             t_gate[name].append(q.add_gates(only[i], info, cs, NUM_CONSTANTS, pi, alphas))
         rows_p, ms = witness(g.poseidon_gate_witness)
         t_wit["poseidon"].append(ms)
@@ -116,6 +121,7 @@ def main():
     out = {"tool": "plonky2_gates_bench", **gpu_info(), "log_n": LOG_N, "rate_bits": RATE_BITS, "lde_rows": R, "wires_cols": 135,
            "constants_sigmas_cols": NUM_CONSTANTS + 80, "n_challenges": N_CH, "groups": GROUPS, "repeats": args.repeats,
            "per_gate": per_gate, "poseidon_over_poseidon2": round(per_gate["poseidon"]["ms"] / per_gate["poseidon2"]["ms"], 3),
+           "arithmetic_extension_over_arithmetic": round(per_gate["arithmetic_extension_10"]["ms"] / per_gate["arithmetic_20"]["ms"], 3),
            "witness_rows": WITNESS_ROWS, "witness_ms": {k: med(v) for k, v in t_wit.items()}, "parity_rows": len(rows), "parity": bool(parity)}
     line = json.dumps(out)
     print(line)
