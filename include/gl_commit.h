@@ -201,7 +201,15 @@ int gl_fri_read(gl_ctx* ctx, gl_handle fri, uint64_t* out_coeffs_ext, uint64_t* 
  *                                                           6n wires, 2n constraints, 1 constant (degree 3)
  *   GL_GATE_REDUCING_EXTENSION    ReducingExtensionGate     param = num_coeffs (1..32; 32 = max_coeffs_len(135, 80))
  *                                                           4 + 4n wires, 2n constraints, 0 constants (degree 2)
- * Kinds 14 and 18 are not assigned: they stay unknown kinds, as they were in earlier releases.
+ * and the three other gates plonky2's recursive verifier circuit registers (plonky2 @ 3de92d9 gates/{coset_interpolation,reducing,
+ * poseidon_mds}.rs; restated, parity unpinned; D = 2, extension constraints as above; none reads gate constants):
+ *   GL_GATE_COSET_INTERPOLATION   CosetInterpolationGate    param = subgroup_bits | degree << 8 (bits 1..5, 2 <= degree <= n = 2^bits;
+ *                                                           with_max_degree(4, 8) = 4 | 6 << 8), k = (n - 2) / (degree - 1):
+ *                                                           7 + 2n + 4k wires (<= 135), 4 + 4k constraints, 0 constants (degree `degree`)
+ *   GL_GATE_REDUCING              ReducingGate              param = num_coeffs (1..43; 43 = max_coeffs_len(135, 80)), base coefficients
+ *                                                           4 + 3n wires, 2n constraints, 0 constants (degree 2)
+ *   GL_GATE_POSEIDON_MDS          PoseidonMdsGate           param 0: 48 wires, 24 constraints, 0 constants (degree 1)
+ * Kinds 14, 18 and 22 are not assigned: they stay unknown kinds, as they were in earlier releases.
  * gl_quotient_add_gate:  acc[k][row] += filter(row) * sum_i alphas[k]^(constraint_offset + i) * constraint_i(wires(row)),  k < n_challenges
  * (alphas are BASE-field challenges, as upstream; filter(row) = column filter_col of the batch filter_batch at the same row, or 1 when
  * filter_batch == 0).  gl_quotient_read: [n_challenges][R] words, row order = the leaves' (bit-reversed).
@@ -212,7 +220,7 @@ enum { GL_GATE_POSEIDON2 = 0, GL_GATE_U32_ARITHMETIC = 1, GL_GATE_U32_ADD_MANY =
        GL_GATE_U32_INTERLEAVE = 5, GL_GATE_UNINTERLEAVE_TO_U32 = 6, GL_GATE_UNINTERLEAVE_TO_B32 = 7, GL_GATE_COMPARISON = 8, GL_GATE_NOOP = 9,
        GL_GATE_CONSTANT = 10, GL_GATE_PUBLIC_INPUT = 11, GL_GATE_ARITHMETIC = 12, GL_GATE_BASE_SUM = 13, GL_GATE_POSEIDON = 15,
        GL_GATE_EXPONENTIATION = 16, GL_GATE_RANDOM_ACCESS = 17, GL_GATE_ARITHMETIC_EXTENSION = 19, GL_GATE_MUL_EXTENSION = 20,
-       GL_GATE_REDUCING_EXTENSION = 21 };
+       GL_GATE_REDUCING_EXTENSION = 21, GL_GATE_COSET_INTERPOLATION = 23, GL_GATE_REDUCING = 24, GL_GATE_POSEIDON_MDS = 25 };
 int gl_gate_num_wires(int kind, uint32_t param);
 int gl_gate_num_constraints(int kind, uint32_t param);
 /* Gate::num_constants: the gate constants a gate reads (-1 for a bad kind or parameter) */

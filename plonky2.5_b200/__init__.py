@@ -15,6 +15,7 @@ from .api import (GATE_COMPARISON, GATE_POSEIDON2, GATE_U32_ADD_MANY, GATE_U32_A
 from .api import GATE_ARITHMETIC, GATE_BASE_SUM, GATE_CONSTANT, GATE_NOOP, GATE_PUBLIC_INPUT, SelectorsInfo  # noqa: F401
 from .api import GATE_EXPONENTIATION, GATE_POSEIDON, GATE_RANDOM_ACCESS, poseidon_gate_witness, random_access_params  # noqa: F401
 from .api import GATE_ARITHMETIC_EXTENSION, GATE_MUL_EXTENSION, GATE_REDUCING_EXTENSION  # noqa: F401
+from .api import GATE_COSET_INTERPOLATION, GATE_POSEIDON_MDS, GATE_REDUCING, coset_interpolation_params  # noqa: F401
 from .build import build  # noqa: F401
 
 __all__ = ["Challenger", "Context", "FriBatchInfo", "FriOpeningBatch", "FriOpenings", "FriParams", "FriProofHead", "GlError", "MerkleCap",

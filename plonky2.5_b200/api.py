@@ -613,6 +613,19 @@ GATE_POSEIDON, GATE_EXPONENTIATION, GATE_RANDOM_ACCESS = 15, 16, 17
 # plonky2's extension-field gates (D = 2): ArithmeticExtensionGate { num_ops } (1..16; new_from_config: 10 at 80 routed wires),
 # MulExtensionGate { num_ops } (1..22; new_from_config: 13), ReducingExtensionGate { num_coeffs } (1..32; max_coeffs_len(135, 80) = 32)
 GATE_ARITHMETIC_EXTENSION, GATE_MUL_EXTENSION, GATE_REDUCING_EXTENSION = 19, 20, 21
+# the other gates of plonky2's recursive verifier circuit: CosetInterpolationGate (subgroup_bits | degree << 8, see
+# coset_interpolation_params), ReducingGate { num_coeffs } (base coefficients; 1..43, max_coeffs_len(135, 80) = 43), PoseidonMdsGate (param 0)
+GATE_COSET_INTERPOLATION, GATE_REDUCING, GATE_POSEIDON_MDS = 23, 24, 25
+
+
+def coset_interpolation_params(subgroup_bits: int, max_degree: int = 8) -> int:
+    """plonky2 gates/coset_interpolation.rs · CosetInterpolationGate::with_max_degree as a GATE_COSET_INTERPOLATION param: the fewest
+    intermediate values k = (n - 2) / (max_degree - 1) for n = 2^subgroup_bits points, then the smallest degree that still covers them"""
+    if subgroup_bits < 1 or max_degree < 2:
+        raise ValueError(f"subgroup_bits {subgroup_bits} / max_degree {max_degree}: need subgroup_bits >= 1 and max_degree >= 2")
+    n = 1 << subgroup_bits
+    k = (n - 2) // (max_degree - 1)
+    return subgroup_bits | ((n - 2) // (k + 1) + 2) << 8
 
 
 def random_access_params(bits: int, num_wires: int = 135, num_routed: int = 80, num_constants: int = 2) -> int:

@@ -313,11 +313,20 @@ __device__ __forceinline__ void base_sum_gate(Wires&& w, Emit&& emit, uint32_t p
 // ---- three more base-field gates of plonky2 @ 3de92d9 (gates/{poseidon,exponentiation,random_access}.rs · eval_unfiltered, same
 // constraint order).  Upstream source is not in this tree: restated, parity unpinned (tests/plonky2_std_gates_oracle.py restates them too).
 
+// coefficient i of output row r of plonky2's Poseidon MDS matrix: CIRC[i] + DIAG[r] at i = 0
+__device__ __forceinline__ constexpr uint32_t mds_coeff(uint32_t i, uint32_t r) {
+    constexpr uint32_t CIRC[P2_WIDTH] = {17, 15, 41, 16, 2, 28, 13, 13, 39, 18, 34, 20};
+    return CIRC[i] + (r == 0 && i == 0 ? 8 : 0);
+}
+// L + H 2^32 < 2^74 as (H >> 32 + carry : x), reduced once
+__device__ __forceinline__ uint64_t reduce_halves(uint64_t L, uint64_t H) {
+    const uint64_t x = L + (H << 32);
+    return gl::canon(gl::reduce128(x, (H >> 32) + (x < L)));
+}
 // plonky2 Poseidon::mds_layer: out[r] = sum_i CIRC[i] s[(i + r) % 12] + DIAG[r] s[r] (hash/poseidon_goldilocks.rs MDS_MATRIX_CIRC /
 // MDS_MATRIX_DIAG, DIAG = 8 at r = 0 only).  The coefficients are small (sum 264 < 2^9), so the 32-bit halves of the canonical inputs
 // are accumulated apart (each sum < 2^41, one IMAD.WIDE.U32 per term) and every lane is reduced once.
 __device__ __forceinline__ void poseidon_mds(uint64_t (&s)[P2_WIDTH]) {
-    constexpr uint32_t CIRC[P2_WIDTH] = {17, 15, 41, 16, 2, 28, 13, 13, 39, 18, 34, 20};
     uint32_t lo[P2_WIDTH], hi[P2_WIDTH];
 #pragma unroll
     for (int i = 0; i < P2_WIDTH; i++) { lo[i] = (uint32_t)s[i]; hi[i] = (uint32_t)(s[i] >> 32); }
@@ -326,12 +335,11 @@ __device__ __forceinline__ void poseidon_mds(uint64_t (&s)[P2_WIDTH]) {
         uint64_t L = 0, H = 0;
 #pragma unroll
         for (int i = 0; i < P2_WIDTH; i++) {
-            const uint32_t c = CIRC[i] + (r == 0 && i == 0 ? 8 : 0);
+            const uint32_t c = mds_coeff(i, r);
             L += (uint64_t)lo[(i + r) % P2_WIDTH] * c;
             H += (uint64_t)hi[(i + r) % P2_WIDTH] * c;
         }
-        const uint64_t x = L + (H << 32);                               // L + H 2^32 < 2^74 as (H >> 32 + carry : x)
-        s[r] = gl::canon(gl::reduce128(x, (H >> 32) + (x < L)));
+        s[r] = reduce_halves(L, H);
     }
 }
 
@@ -470,24 +478,93 @@ __device__ __forceinline__ void mul_extension_gate(Wires&& w, Consts&& k, Emit&&
         emit_ext_sub(ext_wire(6 * i + 4, w), {gl::mulc(p.a0, c0), gl::mulc(p.a1, c0)}, emit);
     }
 }
-// ReducingExtensionGate: param = num_coeffs n; output 0, alpha 2, old_acc 4, coefficient i at 6 + 2i, accumulator i at 6 + 2n + 2i for
-// i < n - 1 and accumulator n - 1 is the output.  From acc = old_acc: acc alpha + coeff_i - acc_i, then acc = acc_i (the wire)
-template <class Wires, class Emit>
-__device__ __forceinline__ void reducing_extension_gate(Wires&& w, Emit&& emit, uint32_t n) {
+// ReducingExtensionGate (D = 2) and ReducingGate (D = 1, base-field coefficients): param = num_coeffs n; output 0, alpha 2, old_acc 4,
+// coefficient i at 6 + D i, accumulator i at 6 + D n + 2i for i < n - 1 and accumulator n - 1 is the output.  From acc = old_acc:
+// acc alpha + coeff_i - acc_i, then acc = acc_i (the wire)
+template <int D, class Wires, class Emit>
+__device__ __forceinline__ void reducing_gate(Wires&& w, Emit&& emit, uint32_t n) {
     const gl::Ext alpha = ext_wire(2, w);
     gl::Ext acc = ext_wire(4, w);
 #pragma unroll 1
     for (uint32_t i = 0; i < n; i++) {
-        const gl::Ext acc_i = ext_wire(i + 1 < n ? 6 + 2 * n + 2 * i : 0, w);
-        emit_ext_sub(gl::ext_add(gl::ext_mul(acc, alpha), ext_wire(6 + 2 * i, w)), acc_i, emit);
+        const gl::Ext acc_i = ext_wire(i + 1 < n ? 6 + D * n + 2 * i : 0, w);
+        gl::Ext next = gl::ext_mul(acc, alpha);
+        if constexpr (D == 2) next = gl::ext_add(next, ext_wire(6 + 2 * i, w));
+        else next.a0 = gl::add(next.a0, w(6 + i));
+        emit_ext_sub(next, acc_i, emit);
         acc = acc_i;
     }
+}
+
+// ---- the gates plonky2's recursive verifier adds (plonky2 @ 3de92d9 gates/{poseidon_mds,coset_interpolation}.rs · eval_unfiltered, D = 2;
+// restated, parity unpinned, tests/plonky2_recursion_gates_oracle.py restates them too; ReducingGate is reducing_gate<1> above).
+
+// PoseidonMdsGate: ext input i at wires 2i, ext output i at 24 + 2i (i < 12).  Per output row i, component by component:
+// out_i - (sum_j CIRC[j] in_{(i+j) % 12} + DIAG[i] in_i), the constants as base scalars (poseidon_mds's matrix and its 32-bit-halves
+// accumulation).  One row at a time from the wire reader, so no 12-wide state is held (24 constraints, degree 1)
+template <class Wires, class Emit>
+__device__ __forceinline__ void poseidon_mds_gate(Wires&& w, Emit&& emit) {
+#pragma unroll 1
+    for (uint32_t i = 0; i < P2_WIDTH; i++) {
+        uint64_t L0 = 0, H0 = 0, L1 = 0, H1 = 0;
+#pragma unroll
+        for (uint32_t j = 0; j < P2_WIDTH; j++) {
+            const uint32_t c = mds_coeff(j, i), at = 2 * ((i + j) % P2_WIDTH);
+            const uint64_t x0 = w(at), x1 = w(at + 1);
+            L0 += (uint64_t)(uint32_t)x0 * c; H0 += (x0 >> 32) * c;
+            L1 += (uint64_t)(uint32_t)x1 * c; H1 += (x1 >> 32) * c;
+        }
+        emit(gl::sub(w(24 + 2 * i), reduce_halves(L0, H0)));
+        emit(gl::sub(w(25 + 2 * i), reduce_halves(L1, H1)));
+    }
+}
+
+// the 2^bits-th root of unity of plonky2's choice (primitive_root_of_unity), bits 0..5
+__constant__ uint64_t COSET_INTERPOLATION_ROOTS[6] = {1ULL, 0xFFFFFFFF00000000ULL, 0x1000000000000ULL, 0xFFFFFFFEFF000001ULL,
+                                                      0xEFFFFFFF00000001ULL, 0x3FFFFFFFC000ULL};
+
+// CosetInterpolationGate: param = subgroup_bits | degree << 8, n = 2^subgroup_bits, k = (n - 2) / (degree - 1) intermediates.  Wires:
+// shift 0 (base), value i at 1 + 2i (i < n), evaluation point 1 + 2n, evaluation value 3 + 2n; with s = 5 + 2n, intermediate eval i at
+// s + 2i, intermediate prod i at s + 2(k + i), shifted evaluation point s + 4k.  Constraints: evaluation_point - shifted_point shift; then
+// partial_interpolate over domain[0, degree) from (eval, prod) = (0, 1), and for each i < k: int_eval_i - eval, int_prod_i - prod, continuing
+// from those two wires over domain[1 + (degree - 1)(i + 1), min(that + degree - 1, n)); last evaluation_value - eval.  One step, with
+// t = z' - x_j: eval <- eval t + (v_j w_j) prod, prod <- prod t.  The domain is the subgroup, so the barycentric weight of x_j = omega^j is
+// w_j = x_j / n exactly; the chunks are consecutive, so x_j is stepped by omega and no table is read
+template <class Wires, class Emit>
+__device__ __forceinline__ void coset_interpolation_gate(Wires&& w, Emit&& emit, uint32_t param) {
+    const uint32_t bits = param & 0xFF, degree = param >> 8, n = 1u << bits, k = (n - 2) / (degree - 1), s = 5 + 2 * n;
+    const uint64_t shift = w(0), omega = COSET_INTERPOLATION_ROOTS[bits], n_inv = gl::P - ((gl::P - 1) >> bits);
+    const gl::Ext z = ext_wire(s + 4 * k, w);
+    const gl::Ext point = ext_wire(1 + 2 * n, w);
+    emit(gl::sub(point.a0, gl::mulc(z.a0, shift)));
+    emit(gl::sub(point.a1, gl::mulc(z.a1, shift)));
+    gl::Ext eval = {0, 0}, prod = {1, 0};
+    uint64_t x = 1;
+    uint32_t next = degree, inter = 0;   // the domain index that ends the current chunk, the intermediate pair it is checked against
+#pragma unroll 1
+    for (uint32_t j = 0; j < n; j++) {
+        if (j == next) {
+            const gl::Ext ie = ext_wire(s + 2 * inter, w), ip = ext_wire(s + 2 * (k + inter), w);
+            emit_ext_sub(ie, eval, emit);
+            emit_ext_sub(ip, prod, emit);
+            eval = ie; prod = ip;
+            next += degree - 1; inter++;
+        }
+        const gl::Ext t = {gl::sub(z.a0, x), z.a1};
+        const uint64_t wj = gl::mulc(x, n_inv);
+        const gl::Ext vw = {gl::mulc(w(1 + 2 * j), wj), gl::mulc(w(2 + 2 * j), wj)};
+        eval = gl::ext_add(gl::ext_mul(eval, t), gl::ext_mul(vw, prod));
+        prod = gl::ext_mul(prod, t);
+        x = gl::mulc(x, omega);
+    }
+    emit_ext_sub(ext_wire(3 + 2 * n, w), eval, emit);
 }
 
 enum { GATE_POSEIDON2 = 0, GATE_U32_ARITHMETIC = 1, GATE_U32_ADD_MANY = 2, GATE_U32_SUBTRACTION = 3, GATE_U32_RANGE_CHECK = 4,
        GATE_U32_INTERLEAVE = 5, GATE_UNINTERLEAVE_TO_U32 = 6, GATE_UNINTERLEAVE_TO_B32 = 7, GATE_COMPARISON = 8, GATE_NOOP = 9,
        GATE_CONSTANT = 10, GATE_PUBLIC_INPUT = 11, GATE_ARITHMETIC = 12, GATE_BASE_SUM = 13, GATE_POSEIDON = 15, GATE_EXPONENTIATION = 16,
-       GATE_RANDOM_ACCESS = 17, GATE_ARITHMETIC_EXTENSION = 19, GATE_MUL_EXTENSION = 20, GATE_REDUCING_EXTENSION = 21 };
+       GATE_RANDOM_ACCESS = 17, GATE_ARITHMETIC_EXTENSION = 19, GATE_MUL_EXTENSION = 20, GATE_REDUCING_EXTENSION = 21,
+       GATE_COSET_INTERPOLATION = 23, GATE_REDUCING = 24, GATE_POSEIDON_MDS = 25 };
 
 // every kind but GATE_POSEIDON, which has kernel instances of its own (inlined here it would raise the register count of every gate)
 template <class Wires, class Consts, class Emit>
@@ -509,7 +586,10 @@ __device__ __forceinline__ void eval_gate(int kind, uint32_t param, Wires&& w, C
         case GATE_RANDOM_ACCESS: random_access_gate(w, k, emit, param); break;
         case GATE_ARITHMETIC_EXTENSION: arithmetic_extension_gate(w, k, emit, param); break;
         case GATE_MUL_EXTENSION: mul_extension_gate(w, k, emit, param); break;
-        case GATE_REDUCING_EXTENSION: reducing_extension_gate(w, emit, param); break;
+        case GATE_REDUCING_EXTENSION: reducing_gate<2>(w, emit, param); break;
+        case GATE_COSET_INTERPOLATION: coset_interpolation_gate(w, emit, param); break;
+        case GATE_REDUCING: reducing_gate<1>(w, emit, param); break;
+        case GATE_POSEIDON_MDS: poseidon_mds_gate(w, emit); break;
         case GATE_NOOP: break;
         default: comparison_gate(w, emit, param); break;
     }

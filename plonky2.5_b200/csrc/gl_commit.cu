@@ -2183,6 +2183,13 @@ int gate_wires(int kind, uint32_t param) {
         case GL_GATE_ARITHMETIC_EXTENSION: return param >= 1 && param <= 16 ? (int)(8 * param) : -1;
         case GL_GATE_MUL_EXTENSION: return param >= 1 && param <= 22 ? (int)(6 * param) : -1;
         case GL_GATE_REDUCING_EXTENSION: return param >= 1 && param <= 32 ? (int)(4 + 4 * param) : -1;
+        case GL_GATE_COSET_INTERPOLATION: {   // subgroup_bits | degree << 8
+            if (lo < 1 || lo > 5 || hi < 2 || hi > (1u << lo)) return -1;
+            const uint32_t n = 1u << lo, nw = 7 + 2 * n + 4 * ((n - 2) / (hi - 1));
+            return nw <= 135 ? (int)nw : -1;
+        }
+        case GL_GATE_REDUCING: return param >= 1 && param <= 43 ? (int)(4 + 3 * param) : -1;
+        case GL_GATE_POSEIDON_MDS: return param == 0 ? 48 : -1;
         default: return -1;
     }
 }
@@ -2208,7 +2215,10 @@ int gate_constraints(int kind, uint32_t param) {
         case GL_GATE_RANDOM_ACCESS: return (int)((lo + 2) * (hi & 0xFF) + (param >> 16));
         case GL_GATE_ARITHMETIC_EXTENSION:
         case GL_GATE_MUL_EXTENSION:
-        case GL_GATE_REDUCING_EXTENSION: return (int)(2 * param);
+        case GL_GATE_REDUCING_EXTENSION:
+        case GL_GATE_REDUCING: return (int)(2 * param);
+        case GL_GATE_COSET_INTERPOLATION: return (int)(4 + 4 * (((1u << lo) - 2) / (hi - 1)));
+        case GL_GATE_POSEIDON_MDS: return 24;
         default: return (int)(1 + lo);   // GL_GATE_BASE_SUM
     }
 }
@@ -2224,8 +2234,8 @@ int gate_constants(int kind, uint32_t param) {
     }
 }
 void check_gate(int kind, uint32_t param) {
-    // kinds 14 and 18 are not assigned: earlier releases refused them as unknown kinds, and they still are
-    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_REDUCING_EXTENSION || kind == 14 || kind == 18)
+    // kinds 14, 18 and 22 are not assigned: earlier releases refused them as unknown kinds, and they still are
+    if (kind < GL_GATE_POSEIDON2 || kind > GL_GATE_POSEIDON_MDS || kind == 14 || kind == 18 || kind == 22)
         GL_THROW(GL_ERR_INVALID, "unknown gate kind %d", kind);
     if (gate_wires(kind, param) < 0) GL_THROW(GL_ERR_INVALID, "gate kind %d: parameter %u out of range (see include/gl_commit.h)", kind, param);
 }

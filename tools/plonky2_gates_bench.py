@@ -1,12 +1,14 @@
 """Device time of plonky2's PoseidonGate, ExponentiationGate(66), RandomAccessGate(bits 4, 4 copies, 2 extra constants) and of the
-extension-field gates ArithmeticExtensionGate(10), MulExtensionGate(13) and ReducingExtensionGate(32) in gl_quotient_add_gates at the
-wrapper shape, and of the PoseidonGate witness generator; prints one JSON line (and writes it to --out).
+extension-field gates ArithmeticExtensionGate(10), MulExtensionGate(13) and ReducingExtensionGate(32), and of the recursive verifier's
+CosetInterpolationGate(4, 6), ReducingGate(43) and PoseidonMdsGate in gl_quotient_add_gates at the wrapper shape, and of the PoseidonGate
+witness generator; prints one JSON line (and writes it to --out).
 
     python tools/plonky2_gates_bench.py [--repeats 20] [--warmup 3] [--out FILE]
 
 Shape (as tools/quotient_gates_bench.py): N = 2^16, rate_bits 3 (R = 2^19 LDE rows), a 135-column wires commit, a constants/sigmas commit
-with 4 selectors, 2 gate constants and 80 sigmas, 2 challenges.  Gate list [Poseidon] [Poseidon2] [Exponentiation(66), RandomAccess]
-[ArithmeticExtension(10), Arithmetic(20), MulExtension(13), ReducingExtension(32)] in 4 selector groups.
+with 5 selectors, 2 gate constants and 80 sigmas, 2 challenges.  Gate list [Poseidon] [Poseidon2] [Exponentiation(66), RandomAccess]
+[ArithmeticExtension(10), Arithmetic(20), MulExtension(13), ReducingExtension(32)] [CosetInterpolation(4, 6), Reducing(43), PoseidonMds]
+in 5 selector groups.
   per_gate_ms         one add_gates call with every other gate replaced by NoopGate: one launch, median over the repeats.  PoseidonGate
                       and Poseidon2Gate (same wires, same constraint count) are run alternately in the same process, and so are
                       ArithmeticExtensionGate(10) and ArithmeticGate(20) (both 80 routed wires and 20 constraints: the pair shows
@@ -32,7 +34,7 @@ for p in (ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "oracle"), os.pa
 
 import plonky25_b200 as g  # noqa: E402
 import gates_oracle as go  # noqa: E402
-import plonky2_ext_gates_oracle as pgo  # noqa: E402
+import plonky2_recursion_gates_oracle as pgo  # noqa: E402
 from oracle_c import splitmix_columns  # noqa: E402
 from quotient_gates_bench import gpu_info  # noqa: E402
 
@@ -41,9 +43,11 @@ LOG_N, RATE_BITS, N_CH, WITNESS_ROWS = 16, 3, 2, 1 << 16
 GATES = [("poseidon", g.GATE_POSEIDON, 0), ("poseidon2", g.GATE_POSEIDON2, 0), ("exponentiation_66", g.GATE_EXPONENTIATION, 66),
          ("random_access_4x4_2", g.GATE_RANDOM_ACCESS, g.random_access_params(4)),
          ("arithmetic_extension_10", g.GATE_ARITHMETIC_EXTENSION, 10), ("arithmetic_20", g.GATE_ARITHMETIC, 20),
-         ("mul_extension_13", g.GATE_MUL_EXTENSION, 13), ("reducing_extension_32", g.GATE_REDUCING_EXTENSION, 32)]
-GROUPS = [(0, 1), (1, 2), (2, 4), (4, 8)]
-SELECTORS = [0, 1, 2, 2, 3, 3, 3, 3]
+         ("mul_extension_13", g.GATE_MUL_EXTENSION, 13), ("reducing_extension_32", g.GATE_REDUCING_EXTENSION, 32),
+         ("coset_interpolation_4_6", g.GATE_COSET_INTERPOLATION, g.coset_interpolation_params(4)), ("reducing_43", g.GATE_REDUCING, 43),
+         ("poseidon_mds", g.GATE_POSEIDON_MDS, 0)]
+GROUPS = [(0, 1), (1, 2), (2, 4), (4, 8), (8, 11)]
+SELECTORS = [0, 1, 2, 2, 3, 3, 3, 3, 4, 4, 4]
 NUM_CONSTANTS = len(GROUPS) + 2
 
 
