@@ -339,6 +339,8 @@ int gl_lde_scatter(gl_ctx* ctx, const uint64_t* const* cols, uint32_t n_cols, ui
  * gl_dev_lde_own_cosets: peer_coeffs[q] = rank q's coefficient block (own buffer for q == self, CUDA-IPC mapping otherwise), with
  * pitches[q], col_counts[q], col_offsets[q]; d_stage[q] = local staging for rank q's block (ignored for q == self);
  * leaf blocks [self*2^rate_bits/n_peers, (self+1)*2^rate_bits/n_peers) are written to d_leaves [rows_per_rank][leaf_pitch].
+ * pitches[q] and col_offsets[q] must be multiples of 4, and so must leaf_pitch (GL_ERR_INVALID otherwise): a block is stored in whole
+ * groups of 4 or 8 columns, so columns [col_offsets[q] + col_counts[q], round_up(col_counts[q], 4 or 8)) of every leaf row are written too.
  * The caller synchronises the ranks between the two calls (every block complete) — see plonky2.5_b200/sharded.py.                   */
 int gl_dev_intt(gl_ctx* ctx, const uint64_t* d_cols, uint64_t col_stride, uint32_t n_cols, uint32_t log_n, int input_is_coeffs,
                 uint64_t* d_out_coeffs, uint32_t coeff_pitch);

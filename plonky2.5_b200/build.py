@@ -50,9 +50,10 @@ def build(force: bool = False, verbose: bool = False) -> str:
         print(" ".join(cmd), file=sys.stderr)
     env = dict(os.environ)
     env.pop("CC", None); env.pop("CXX", None)   # the image's CC wrapper is not a valid nvcc host compiler choice
+    stamp = source_hash()                        # of the bytes nvcc reads: a source edited while it compiles must not look built
     subprocess.run(cmd, check=True, env=env)
     with open(STAMP, "w") as f:
-        f.write(source_hash())
+        f.write(stamp)
     return LIB
 
 

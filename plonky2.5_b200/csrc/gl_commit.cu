@@ -1142,6 +1142,9 @@ int gl_dev_lde_own_cosets(gl_ctx* c, uint64_t* const* peer_coeffs, uint64_t* con
     if (n_peers == 0 || (n_peers & (n_peers - 1)) || n_peers > (uint32_t)ntt::MAX_PEERS || self >= n_peers) GL_THROW(GL_ERR_INVALID, "bad peer count / rank");
     if (n_peers > (1u << rate_bits)) GL_THROW(GL_ERR_INVALID, "coset sharding needs n_peers <= 2^rate_bits");
     if (log_n + rate_bits > 31) GL_THROW(GL_ERR_UNSUPPORTED, "log_n + rate_bits > 31");
+    // every block is stored in whole column groups (round_up(col_counts[q], G) columns, G = 4 or 8, at an offset that is a multiple
+    // of 4): only a pitch of whole 4-column groups keeps a block's padding columns inside its own row
+    if (leaf_pitch % 4) GL_THROW(GL_ERR_INVALID, "leaf_pitch must be a multiple of 4");
     const uint64_t N = 1ULL << log_n;
     const uint32_t blocks_per_rank = (1u << rate_bits) / n_peers, first_block = self * blocks_per_rank;
     for (uint32_t q = 0; q < n_peers; q++) {
