@@ -2536,7 +2536,8 @@ int gl_quotient_commit(gl_ctx* c, gl_handle qh, uint32_t cap_height, uint64_t* o
     uint64_t cur = gN;
     for (uint32_t j = 0; j < (1u << r); j++) { zh[j] = gl::h_inv(cur - 1); cur = gl::h_mul(cur, wr);   /* cur is a non-zero canonical element; Z_H != 0 on the coset */ }
     DevBuf vals, coeffs, tab, cols;
-    vals.ensure(R * pitch); coeffs.ensure(R * pitch); tab.ensure(R + 8); cols.ensure((uint64_t)n_ch * R);
+    // tab: shift^-j for j < R, then the 2^r Z_H inverses
+    vals.ensure(R * pitch); coeffs.ensure(R * pitch); tab.ensure(R + zh.size()); cols.ensure((uint64_t)n_ch * R);
     uint64_t* d_zh = tab.p + R;
     CUDA_CHECK(cudaMemcpyAsync(d_zh, zh.data(), zh.size() * 8, cudaMemcpyHostToDevice, c->stream));
     gates::quotient_gather_kernel<<<(uint32_t)((R + 255) / 256), 256, 0, c->stream>>>(q->acc.p, vals.p, pitch, n_ch, bits, r, d_zh);
